@@ -25,6 +25,8 @@ top-k / candidate scores are combined with an NCCL all-gather and a max all-redu
                rank 0 at N = 1 only
 
 `--impl reference` times that CPU implementation alone (no GPU work at all), --steps / --warmup honoured.
+`--dump-outputs DIR` writes what each timed GPU path returned in its last step (predictions and scores of every search
+leg, the fingerprints) as DIR/<name>.npy, float32 / float64, under 64 MB in all.
 """
 from __future__ import annotations
 
@@ -53,6 +55,7 @@ FLOPS_PER_SEGMENT = 607_199_232  # model/arch.py (conv + div-enc)
 LOGMEL_BYTES_PER_SEGMENT = 64_768    # SURVEY 8(d): 32,000 B of samples in + 32,768 B of log-mel out
 CPU_FIT = [(250_000, 200), (1_000_000, 200), (4_000_000, 40)]      # (database rows, test ids) of the CPU baseline fit
 REF_STEP_ROWS, REF_STEP_IDS = 1_000_000, 24                          # one step of the --impl reference arm
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peaks():
@@ -290,6 +293,16 @@ def build_sharded_index(ctx, torch, sidx, n_dummy, dev):
     del buf
 
 
+def dump_outputs(outputs, out_dir):
+    """--dump-outputs: each array as out_dir/<name>.npy.  The inputs are seeded, so two builds run with the same
+    arguments can be compared output for output."""
+    assert sum(a.nbytes for a in outputs.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def time_steps(torch, dev, fn, steps, warmup, barrier):
     for _ in range(warmup):
         fn()
@@ -392,6 +405,9 @@ def run_gpu(args):
     launches0 = ctx.launches
     ms_res = max_over_ranks(time_steps(torch, dev, step_resident, args.steps, 0, barrier))
     clocks = sampler.stop()
+    # what each timed path returned in its last step, for --dump-outputs (ids as float64: exact below 2**53)
+    outputs = {"search_pred_ids": result["pid"].cpu().numpy().astype(np.float64),
+               "search_pred_scores": result["psc"].cpu().numpy()}
     launches = ctx.launches - launches0
     scan_ms, n_scans = sidx.index.profile_scans(False)
     stats = sidx.index.last_search_stats()
@@ -463,8 +479,9 @@ def run_gpu(args):
         l0 = ctx.launches
         ms_fp = max_over_ranks(time_steps(torch, dev, fp_resident, args.steps, args.warmup, barrier))
         fp_launches = (ctx.launches - l0) // (args.steps + args.warmup)
+        outputs["fingerprints"] = emb_dev.cpu().numpy()
         ms_fp_e2e = max_over_ranks(time_steps(torch, dev, fp_e2e, args.steps, 3, barrier))
-        ms_mel = max_over_ranks(time_steps(torch, dev, logmel_only, max(args.steps, 10), 3, barrier))
+        ms_mel = max_over_ranks(time_steps(torch, dev, logmel_only, args.steps, 3, barrier))
         segs = FP_SEGS_PER_STEP * world
         tfl = segs / (ms_fp * 1e-3) * FLOPS_PER_SEGMENT / 1e12 / world
         mel_gbs = FP_SEGS_PER_STEP * LOGMEL_BYTES_PER_SEGMENT / (ms_mel * 1e-3) / 1e9
@@ -505,6 +522,8 @@ def run_gpu(args):
 
         ms_mini = time_steps(torch, dev, mini_step, args.steps, args.warmup, barrier)
         mp = result["mini"][0].cpu().numpy()
+        outputs["mini_1M_pred_ids"] = mp.astype(np.float64)
+        outputs["mini_1M_pred_scores"] = result["mini"][1].cpu().numpy()
         mini = {"db_rows": 1_000_000 + N_DB, "value": n_queries / (ms_mini * 1e-3), "unit": "queries/s",
                 "ms_per_step": ms_mini,
                 "top1_hit_rate": [float(100.0 * np.mean(mp[:, si, 0] == test_ids + 1_000_000)) for si in range(len(SEQ_LENS))]}
@@ -512,7 +531,7 @@ def run_gpu(args):
 
     # ---- IVF-PQ (SURVEY 8 a6, BASELINE configs[4]): the approximate index the reference builds for index_type "ivfpq"
     # (nlist 256, M 64, 8 bit, nprobe 40), host API incl. H2D / D2H
-    def ivfpq_leg(rows_dummy, keep=False):
+    def ivfpq_leg(rows_dummy, name, keep=False):
         """Index build (k-means on a 1-in-N sample of the dummy rows, encoding of every row) and the timed
         evaluation job through the host API; the database is generated chunk by chunk on the device."""
         from nafp_b200.eval.utils.get_index import IVFPQ, Index
@@ -546,6 +565,8 @@ def run_gpu(args):
         ms_ivf = time_steps(torch, dev, ivf_step, args.steps, args.warmup, barrier)
         st = iidx.last_search_stats()
         ip = result["ivf"][0]
+        outputs[f"{name}_pred_ids"] = ip.astype(np.float64)
+        outputs[f"{name}_pred_scores"] = result["ivf"][1]
         n_run = args.steps + args.warmup             # the statistics cover the warm-up steps too
         tiles = st["reranked"] / n_run               # (for an IVF-PQ index: 128 x 128 tiles of the list-major scan)
         out = {"index": "IVFPQ nlist 256, M 64, 8 bit, nprobe 40", "db_rows": rows_dummy + N_DB,
@@ -613,7 +634,7 @@ def run_gpu(args):
         def lut_step():
             lidx.search_dev(qd.data_ptr(), nq, K_PROBE, Dd.data_ptr(), Id.data_ptr())
 
-        ms = time_steps(torch, dev, lut_step, max(3, args.steps // 4), 3, barrier)
+        ms = time_steps(torch, dev, lut_step, args.steps, 3, barrier)
         Dl, Il = iidx.search(qd.cpu().numpy(), K_PROBE)
         probed_rows = 40.0 / 256.0 * (rows + N_DB)
         return {"kernel": "ivfpq_scan_kernel (shared-memory LUT ADC scan, one CTA per (query row, probed list))",
@@ -626,11 +647,11 @@ def run_gpu(args):
     ivf = None
     if world == 1 and not args.no_mini and not args.no_ivfpq and n_dummy >= 1_000_000:
         if args.no_cpu:
-            ivf, iidx_keep, train_rows = ivfpq_leg(1_000_000, keep=True)
+            ivf, iidx_keep, train_rows = ivfpq_leg(1_000_000, "ivfpq_1M", keep=True)
             ivf["lut_kernel"] = ivfpq_lut_leg(iidx_keep)
             del iidx_keep
         else:
-            ivf, iidx_keep, train_rows = ivfpq_leg(1_000_000, keep=True)
+            ivf, iidx_keep, train_rows = ivfpq_leg(1_000_000, "ivfpq_1M", keep=True)
             ivf["lut_kernel"] = ivfpq_lut_leg(iidx_keep)
             del iidx_keep
             orc = ivfpq_oracle_hit_rates(train_rows, 1_000_000)
@@ -646,7 +667,7 @@ def run_gpu(args):
     # local), same all-gather + merge + max all-reduce
     ivf_full = None
     if world == 1 and not args.no_ivfpq_full and n_dummy > 1_000_000:
-        ivf_full = ivfpq_leg(n_dummy)
+        ivf_full = ivfpq_leg(n_dummy, "ivfpq_full")
     if world > 1 and not args.no_ivfpq_full:
         from nafp_b200.eval.utils.get_index import IVFPQ
         t_ivf = time.time()
@@ -664,6 +685,8 @@ def run_gpu(args):
 
         ms_sivf = max_over_ranks(time_steps(torch, dev, sivf_step, args.steps, args.warmup, barrier))
         sp = result["sivf"][0].cpu().numpy()
+        outputs["ivfpq_full_pred_ids"] = sp.astype(np.float64)
+        outputs["ivfpq_full_pred_scores"] = result["sivf"][1].cpu().numpy()
         ivf_full = {"index": "IVFPQ nlist 256, M 64, 8 bit, nprobe 40, row-sharded", "db_rows": n_total,
                     "value": n_queries / (ms_sivf * 1e-3), "unit": "queries/s", "ms_per_step": ms_sivf, "train_s": t_train,
                     "add_s": t_add, "through": "device-resident queries (seq_match_dev), NCCL all-gather + max all-reduce",
@@ -703,6 +726,8 @@ def run_gpu(args):
                 "search_stats_per_step": {k: v / args.steps for k, v in stats.items()},
                 "fingerprint": fp, "mini_1M": mini, "ivfpq_1M": ivf, "ivfpq_full": ivf_full, "config0": cfg0,
                 "db_build_s": t_build}
+        if args.dump_outputs:
+            dump_outputs(outputs, args.dump_outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -800,7 +825,11 @@ def main():
     ap.add_argument("--no-ivfpq-full", action="store_true", help="skip IVF-PQ on the full-size database (BASELINE configs[4])")
     ap.add_argument("--no-config0", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what each timed path returned in its last step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
     args.warmup = max(args.warmup, 3)              # timing rule: at least three warm-up steps
     if args.impl == "reference":
         return run_reference(args)
