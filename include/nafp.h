@@ -195,11 +195,12 @@ int nafp_index_last_search_stats(nafp_index* idx, int64_t* out8);
  * previous call (at most 8192 launches are recorded between calls). */
 int nafp_index_profile_scans(nafp_index* idx, int enable, double* total_ms, int64_t* n_scans);
 
-/* developer probe of the last flat scan pass (256 entries each): fallback flags, shared
- * thresholds, survivors per query row */
-int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags256, float* thr256, int32_t* total256);
-/* developer probe: per-CTA survivor counts [grid][256] and the tile index at which each CTA first
- * saw a shared threshold per query [grid][256] (-1 = never); the first call arms the probe */
+/* developer probe of the last flat scan pass (512 entries each, one per query row of a pass): fallback flags,
+ * shared thresholds, survivors per query row */
+int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags512, float* thr512, int32_t* total512);
+/* developer probe: per-CTA survivor counts [grid][512] (0 where a CTA does not hold the query row) and the tile index
+ * at which each CTA first saw a shared threshold per query row [grid][512] (-1 = never; entries 504..511 are in-kernel
+ * timestamps when the pass has <= 504 rows); the first call arms the probe */
 int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_out, int32_t* grid_out);
 
 /* ------------------------------------------------------------------ sequence matcher

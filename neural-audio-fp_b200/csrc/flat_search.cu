@@ -5,9 +5,12 @@
 // eval/eval_faiss.py:147-148,211).  Ranking score  s(q,x) = q.x - 0.5|x|^2  (argmax s == argmin
 // |q-x|^2), distance reported as |q|^2 - 2 s.
 //
-// One scan pass handles up to 256 query rows against the whole database:
+// One scan pass handles up to 512 query rows against the whole database:
 //   flat_prep_kernel    fp32 queries -> bf16 A-operand tile, |q|^2, pass state reset
-//   flat_scan_kernel    persistent, one CTA per SM, 256-row DB tiles handed out by a global counter:
+//   flat_scan_kernel    persistent, one CTA per SM, launched as clusters of two CTAs: the CTA of cluster rank r scores
+//                       pass rows [r h, r h + h), h = 128 or 256.  256-row DB tiles are handed out to the pairs by a
+//                       global counter; rank 0 loads each tile ONCE and TMA multicast writes it into both CTAs' rings
+//                       (half the HBM bytes per score of one CTA per tile).  Per CTA:
 //                       TMA (SWIZZLE_128B) -> smem ring of K blocks -> tcgen05.mma (M = 128
 //                       queries, N = 256 DB rows, K = 128, bf16, fp32 accumulators double-buffered in
 //                       TMEM) -> epilogue threads own one query each: a 3-input max over the tile's
@@ -15,10 +18,10 @@
 //                       which a lane fires gets the exact  q.x - 0.5|x|^2 > T  test in straight-line
 //                       code and its hits' row ids join the CTA's pool.
 //                       T is a per-query threshold that all CTAs share through L2 (the kg-th largest
-//                       of the per-CTA running maxima -- a valid lower bound on the kg-th best
-//                       score, maintained by one reducer warp per CTA, lock-free); every CTA first scans
-//                       eight "warm" tiles max-only (re-visited at the end) so that the thresholds are
-//                       tight before the first candidate is appended.
+//                       of the running maxima per (pair, accumulator column half) -- disjoint row sets, so a
+//                       valid lower bound on the kg-th best score -- maintained by one reducer warp per CTA,
+//                       lock-free); every pair first scans eight "warm" tiles max-only (re-visited at the end)
+//                       so that the thresholds are tight before the first candidate is appended.
 //   flat_select_kernel  per query: gather survivors, exact fp32 re-score, sort, and PROVE the
 //                       top-k: every dropped row has bf16 score <= T, hence exact score <= T + eps
 //                       with eps = (2u+u^2)|q|max|x| (u = 2^-8); if the k-th exact score is not
@@ -28,6 +31,7 @@
 #include <climits>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <vector>
 
 #include "index.h"
@@ -113,17 +117,18 @@ constexpr int EPI_PARTS = EPI_WARPS / 4;          // the 4 warps of a TMEM lane 
 constexpr int PART_COLS = SCAN_TILE / EPI_PARTS;  // 64 DB rows (accumulator columns) per warp per unit
 constexpr int SLOT_BYTES = SCAN_TILE * 128;                // 32 KB: one 64-column K block of a 256-row tile
 constexpr int BOX_BYTES = TILE_ROWS * 128;                 // 16 KB per TMA box (128 rows)
-constexpr int Q_KB_BYTES = NQ_MAX * 128;                   // 32 KB: one K block of the query operand
+constexpr int Q_KB_BYTES = NQ_CTA * 128;                   // 32 KB: one K block of the query operand
 constexpr int Q_BYTES_MAX = 2 * Q_KB_BYTES;                // 64 KB
 constexpr int H_RING = 4;                               // tiles of 0.5|x|^2 kept in shared memory
-constexpr int WARM_TILES = 8;                           // tiles every CTA scans max-only before it uses thresholds
-constexpr int SCAN_SMEM = Q_BYTES_MAX + RING_SLOTS * SLOT_BYTES + H_RING * SCAN_TILE * 4 + 2 * NQ_MAX * 4 + 256 + 1024;
+constexpr int WARM_TILES = 8;                           // tiles every pair scans max-only before it uses thresholds
+constexpr int SCAN_SMEM = Q_BYTES_MAX + RING_SLOTS * SLOT_BYTES + H_RING * SCAN_TILE * 4 + 3 * NQ_CTA * 4 + 256 + 1024;
+constexpr uint16_t PAIR_MASK = 0b11, RANK0_MASK = 0b01;       // multicast targets: both CTAs of the pair / rank 0
 constexpr int NEG_INF_ORD = static_cast<int>(0x807FFFFFu);  // f2ord(-inf)
 static_assert(PART_COLS == 64, "epilogue reads two 32-column chunks per unit");
 
 struct ScanBars {
     uint64_t full[RING_SLOTS];
-    uint64_t empty[RING_SLOTS];
+    uint64_t empty[RING_SLOTS];    // only rank 0's is used: both CTAs' MMA warps release a slot there
     uint64_t tfull[2];
     uint64_t tempty[2];
     uint64_t qfull;
@@ -208,27 +213,34 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     uint8_t* q_s = smem;                                   // [kb 2][256 query rows][128 B]
     uint8_t* b_s = smem + Q_BYTES_MAX;                     // [slot][256 DB rows][128 B]
     float* h_s = reinterpret_cast<float*>(b_s + RING_SLOTS * SLOT_BYTES);     // [H_RING][256] 0.5|x|^2 of the tile's rows
-    int* lmax_s = reinterpret_cast<int*>(h_s + H_RING * SCAN_TILE);
-    int* cnt_s = lmax_s + NQ_MAX;
-    ScanBars* bars = reinterpret_cast<ScanBars*>(cnt_s + NQ_MAX);
+    int* lmax_s = reinterpret_cast<int*>(h_s + H_RING * SCAN_TILE);          // [column half 2][NQ_CTA]
+    int* cnt_s = lmax_s + 2 * NQ_CTA;                                         // [NQ_CTA]
+    ScanBars* bars = reinterpret_cast<ScanBars*>(cnt_s + NQ_CTA);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
+    // Clusters of two CTAs (cluster rank = cta & 1).  Both CTAs of a pair score the same DB tiles, each against its own
+    // n_half x 128 query rows: rank 0's producer draws the tiles and multicasts each one into both CTAs' shared
+    // memory, so a tile crosses HBM once per pair.  G CTAs, C = G / 2 pairs.  The maxima that build the thresholds
+    // come from G sources, one per (pair, accumulator column half): disjoint row sets.
     const int G = gridDim.x;
     const int cta = blockIdx.x;
-    // Work items of a CTA: `warm` tiles cta, cta + G, ... scanned max-only (their exact maxima seed the shared
+    const int rank = cta & 1, clu = cta >> 1, C = G >> 1;
+    const int qrow0 = rank * n_half * 128;                 // this CTA's first row of the pass
+    // Work items of a pair: `warm` tiles clu, clu + C, ... scanned max-only (their exact maxima seed the shared
     // thresholds, which are ready -- no wait -- when the last of them is done; a row scanned at tile t survives
     // with probability ~ kg / (rows seen so far), so the first tiles of a pass would otherwise append, and pay
     // for, half of all survivors), then tiles handed out by a global counter (SMs do not all stream at the same
     // rate: with a static split the slowest CTA finished 35 % after the fastest), then the warm tiles again
-    // (with thresholds), then the end marker.  The TMA producer draws the tiles and tells the MMA issuer and
-    // the epilogue through bars->tile_of.
+    // (with thresholds), then the end marker.  Rank 0's TMA producer draws the tiles and tells the MMA issuers and
+    // the epilogues of both CTAs through bars->tile_of.
     // bits 8..11 of the tune word override the number of warm tiles (A/B measurements)
     const int warm_cap = ((tune >> 8) & 15) ? ((tune >> 8) & 15) : WARM_TILES;
-    const int warm = (tune & 2) ? 1 : max(1, min(warm_cap, n_tiles / G));
+    const int warm = (tune & 2) ? 1 : max(1, min(warm_cap, n_tiles / C));
 
-    for (int i = threadIdx.x; i < NQ_MAX; i += blockDim.x) {
+    for (int i = threadIdx.x; i < NQ_CTA; i += blockDim.x) {
         lmax_s[i] = INT_MIN;
+        lmax_s[NQ_CTA + i] = INT_MIN;
         cnt_s[i] = 0;
     }
     if (threadIdx.x == 0) {
@@ -236,7 +248,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         tma_prefetch_desc(&tmap_db);
         for (int s = 0; s < RING_SLOTS; ++s) {
             mbar_init(&bars->full[s], 1);
-            mbar_init(&bars->empty[s], 1);
+            mbar_init(&bars->empty[s], 2);
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(&bars->tfull[a], 1);
@@ -251,7 +263,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         tmem_relinquish();
     }
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();                // the peer's barriers are initialised before the first remote arrive / commit
     tc_fence_after();
     const uint32_t tmem_base = __shfl_sync(0xffffffffu, bars->tmem_base, 0);     // provably warp-uniform
 
@@ -262,16 +274,26 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             mbar_arrive_expect_tx(&bars->qfull, 2u * q_rows * 128u);
             for (int kb = 0; kb < 2; ++kb)
                 for (int r0 = 0; r0 < q_rows; r0 += 32)
-                    tma_load_2d(q_s + kb * Q_KB_BYTES + r0 * 128, &tmap_q, &bars->qfull, kb * 64, r0);
-            int tile = cta;
+                    tma_load_2d(q_s + kb * Q_KB_BYTES + r0 * 128, &tmap_q, &bars->qfull, kb * 64, qrow0 + r0);
+        }
+        if (lane == 0 && rank == 0) {
+            // Rank 0 delivers every item to both CTAs.  Its empty[s] completes when both MMA warps have released the
+            // slot.  It arms the peer's full[s] remotely; the tile id reaches the peer's tile_of by st.async, which
+            // completes on the peer's full[s0], so the id becomes visible there together with the slot's data.
+            const uint32_t peer_full0 = map_shared_rank(&bars->full[0], 1);       // the peer's full[s]: + 8 s
+            const uint32_t peer_tile_of0 = map_shared_rank(&bars->tile_of[0], 1);
+            int tile = clu;
             int revisit = -1;                                   // >= 0: index of the warm tile being revisited
-            int nxt = warm * G + atomicAdd(tile_counter, 1);    // drawn one item ahead: the round trip hides behind the loads
-            for (int i = 0;; ++i) {
+            int nxt = warm * C + atomicAdd(tile_counter, 1);    // drawn one item ahead: the round trip hides behind the loads
+            int i = 0;
+            for (;; ++i) {
                 const int kc0 = 2 * i;
                 const uint32_t ph = (kc0 / RING_SLOTS) & 1;
                 const int s0 = kc0 % RING_SLOTS;
                 mbar_wait_parked(&bars->empty[s0], ph ^ 1);
-                bars->tile_of[i & 7] = tile;                      // released to the consumers by the arrive below
+                bars->tile_of[i & 7] = tile;                      // released to this CTA's consumers by the arrive below
+                mbar_arrive_expect_tx_remote(peer_full0 + 8 * s0, (tile < 0 ? 0 : SLOT_BYTES + SCAN_TILE * 4) + 4);
+                st_async_remote(peer_tile_of0 + 4 * (i & 7), tile, peer_full0 + 8 * s0);
                 if (tile < 0) {
                     mbar_arrive(&bars->full[s0]);
                     break;
@@ -279,33 +301,43 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
 #pragma unroll
                 for (int kb = 0; kb < 2; ++kb) {
                     const int s = s0 + kb;
-                    if (kb == 1) mbar_wait_parked(&bars->empty[s], ph ^ 1);
+                    if (kb == 1) {
+                        mbar_wait_parked(&bars->empty[s], ph ^ 1);
+                        mbar_arrive_expect_tx_remote(peer_full0 + 8 * s, SLOT_BYTES);
+                    }
                     mbar_arrive_expect_tx(&bars->full[s], SLOT_BYTES + (kb == 0 ? SCAN_TILE * 4 : 0));
                     // the tile's 0.5|x|^2 travel with its first K block.  Ring of 4: entry i is rewritten for
-                    // item i+4, whose load is issued after item i+2's MMAs, which start after item i's epilogue
+                    // item i+4, whose load is issued after item i+2's MMAs (in both CTAs), which start after item i's
+                    // epilogue
                     if (kb == 0)
-                        bulk_load_1d(h_s + (i % H_RING) * SCAN_TILE, hn + static_cast<int64_t>(tile) * SCAN_TILE, SCAN_TILE * 4,
-                                     &bars->full[s]);
+                        bulk_load_1d_multicast(h_s + (i % H_RING) * SCAN_TILE, hn + static_cast<int64_t>(tile) * SCAN_TILE,
+                                               SCAN_TILE * 4, &bars->full[s], PAIR_MASK);
                     uint8_t* dst = b_s + s * SLOT_BYTES;
-                    tma_load_2d(dst, &tmap_db, &bars->full[s], kb * 64, tile * SCAN_TILE);
-                    tma_load_2d(dst + BOX_BYTES, &tmap_db, &bars->full[s], kb * 64, tile * SCAN_TILE + TILE_ROWS);
+                    tma_load_2d_multicast(dst, &tmap_db, &bars->full[s], kb * 64, tile * SCAN_TILE, PAIR_MASK);
+                    tma_load_2d_multicast(dst + BOX_BYTES, &tmap_db, &bars->full[s], kb * 64, tile * SCAN_TILE + TILE_ROWS,
+                                          PAIR_MASK);
                 }
                 if (i + 1 < warm) {
-                    tile = cta + (i + 1) * G;
+                    tile = clu + (i + 1) * C;
                 } else if (revisit < 0 && nxt < n_tiles) {
                     tile = nxt;
-                    nxt = warm * G + atomicAdd(tile_counter, 1);
+                    nxt = warm * C + atomicAdd(tile_counter, 1);
                 } else {
                     ++revisit;
-                    tile = revisit < warm ? cta + revisit * G : -1;
+                    tile = revisit < warm ? clu + revisit * C : -1;
                 }
             }
+            // The peer's MMA warp commits into this CTA's empty barriers: wait for its last commits (the K blocks
+            // 2i-3 .. 2i-1 of the last items) before this CTA may leave.  K block kc of a slot is the (kc / 4)-th use.
+            for (int kc = 2 * i + 1; kc < 2 * i + RING_SLOTS; ++kc)
+                mbar_wait_parked(&bars->empty[kc % RING_SLOTS], ((kc / RING_SLOTS) & 1) ^ 1);
         }
         __syncwarp();
     } else if (warp == MMA_WARP) {
         // ------------------------------------------------------------ MMA issuer
         // unit = (tile, 128-query half): D[query][db row] in accumulator (unit & 1).  The second K block's
-        // slot is released as soon as the last unit's MMAs on it are issued, the first one's four MMAs earlier.
+        // slot is released as soon as the last unit's MMAs on it are issued, the first one's four MMAs earlier; a slot is
+        // released on rank 0's empty barrier, which counts both CTAs of the pair.
         // The whole warp runs the loop (uniform control flow keeps descriptors and counters in uniform
         // registers); one elected lane issues.
         const bool leader = elect_one();
@@ -324,7 +356,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 const bool last = hq == n_half - 1;
                 mbar_wait_parked(&bars->tempty[acc], aph ^ 1);
                 if (hq == 0) {
-                    mbar_wait_parked(&bars->full[s0], ph);
+                    mbar_wait_parked_cluster(&bars->full[s0], ph);       // completed from rank 0 (tile id, data)
                     if (smem_ld_volatile(&bars->tile_of[i & 7]) < 0) {      // end marker: wake the epilogue and stop
                         if (leader) tc_commit(&bars->tfull[acc]);
                         __syncwarp();
@@ -341,16 +373,16 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 if (leader) {
 #pragma unroll
                     for (int j = 0; j < 4; ++j) tc_mma_f16(d_tmem, a_kb0 + 2 * j, b_kb0 + 2 * j, idesc, j != 0 ? 1u : 0u);
-                    if (last) tc_commit(&bars->empty[s0]);
+                    if (last) tc_commit_multicast(&bars->empty[s0], RANK0_MASK);
                 }
                 if (hq == 0) {
-                    mbar_wait_parked(&bars->full[s1], ph);
+                    mbar_wait_parked_cluster(&bars->full[s1], ph);
                     tc_fence_after();
                 }
                 if (leader) {
 #pragma unroll
                     for (int j = 0; j < 4; ++j) tc_mma_f16(d_tmem, a_kb1 + 2 * j, b_kb1 + 2 * j, idesc, 1u);
-                    if (last) tc_commit(&bars->empty[s1]);
+                    if (last) tc_commit_multicast(&bars->empty[s1], RANK0_MASK);
                     tc_commit(&bars->tfull[acc]);
                 }
                 __syncwarp();
@@ -360,11 +392,15 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     } else if (warp < EPI_WARPS) {
         // ------------------------------------------------------------ epilogue (EPI_WARPS warps)
         // Warp e reads TMEM lane quadrant (warp & 3) -- 32 queries per half -- and the 64 accumulator
-        // columns (DB rows) [64 part, 64 part + 64) of every unit.
+        // columns (DB rows) [64 part, 64 part + 64) of every unit: column half part >> 1.  Query rows are local
+        // (0 .. n_half * 128 - 1, pass row qrow0 + local row).
         const int qd = warp & 3;
         const int e = warp;               // 0..EPI_WARPS-1
         const int part = e >> 2;          // 0..EPI_PARTS-1
-        constexpr int QPW = NQ_MAX / EPI_WARPS;      // queries whose maxima this warp publishes
+        constexpr int QPW = NQ_CTA / EPI_WARPS;      // queries whose maxima (both column halves) this warp publishes
+        static_assert(2 * QPW == 32, "one lane per (query, column half) when maxima are published");
+        const int q_rows = n_half * 128;
+        int* lmax_part = lmax_s + (part >> 1) * NQ_CTA;
         const float NEG_INF = -INFINITY;
         int pub = INT_MIN;
         int thr_ord[2] = {NEG_INF_ORD, NEG_INF_ORD};
@@ -372,16 +408,16 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         bool active[2];
 #pragma unroll
         for (int hq = 0; hq < 2; ++hq) {
-            active[hq] = hq < n_half && (hq * 128 + qd * 32 + lane) < nq;
+            active[hq] = hq < n_half && qrow0 + (hq * 128 + qd * 32 + lane) < nq;
             t_exact[hq] = active[hq] ? NEG_INF : INFINITY;      // padding queries never fire
             t_pre[hq] = t_exact[hq];
         }
-        uint64_t* my_pool = pool + static_cast<int64_t>(cta) * NQ_MAX * POOL_CAP;
+        uint64_t* my_pool = pool + static_cast<int64_t>(cta) * NQ_CTA * POOL_CAP;
         const uint32_t ns32 = static_cast<uint32_t>(n_search);
         // shared thresholds of this thread's queries -> registers; true when all of the warp's are known
         auto load_thresholds = [&](int (&tg)[2]) {
 #pragma unroll
-            for (int hq = 0; hq < 2; ++hq) tg[hq] = active[hq] ? ld_relaxed(&Tg[hq * 128 + qd * 32 + lane]) : INT_MIN;
+            for (int hq = 0; hq < 2; ++hq) tg[hq] = active[hq] ? ld_relaxed(&Tg[qrow0 + hq * 128 + qd * 32 + lane]) : INT_MIN;
         };
         auto apply_thresholds = [&](const int (&tg)[2], int i) -> bool {
             bool valid = true;
@@ -390,7 +426,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 if (active[hq]) {
                     if (tg[hq] > thr_ord[hq]) {
                         if (dbg_first && part == 0 && thr_ord[hq] == NEG_INF_ORD)
-                            dbg_first[cta * NQ_MAX + hq * 128 + qd * 32 + lane] = i;
+                            dbg_first[cta * NQ_MAX + qrow0 + hq * 128 + qd * 32 + lane] = i;
                         thr_ord[hq] = tg[hq];
                         const float t = ord2f(tg[hq]);
                         t_exact[hq] = t;
@@ -401,41 +437,42 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             }
             return __all_sync(0xffffffffu, valid);
         };
-        // publish this CTA's running maxima: warp e owns queries [QPW e, QPW e + QPW)
+        // publish this CTA's running maxima: warp e owns local queries [QPW e, QPW e + QPW), lane / QPW is the column
+        // half, and source (pair, column half) is column 2 clu + half of Mx
         auto publish_maxima = [&]() {
-            const int q = e * QPW + lane;
-            if (lane < QPW && q < nq) {
-                const int m = smem_ld_volatile(&lmax_s[q]);
+            const int ql = e * QPW + (lane % QPW), half = lane / QPW;
+            if (ql < q_rows && qrow0 + ql < nq) {
+                const int m = smem_ld_volatile(&lmax_s[half * NQ_CTA + ql]);
                 if (m > pub) {
-                    st_relaxed(&Mx[q * G + cta], m);
+                    st_relaxed(&Mx[(qrow0 + ql) * G + 2 * clu + half], m);
                     pub = m;
                 }
             }
         };
-        // developer probe (nq <= 248): ns since kernel start at which tile 0 / the threshold wait / the scan ended
-        const bool probe = dbg_first != nullptr && threadIdx.x == 0 && nq <= 248;
+        // developer probe (nq <= NQ_MAX - 8): ns since kernel start at which tile 0 / the threshold wait / the scan ended
+        const bool probe = dbg_first != nullptr && threadIdx.x == 0 && nq <= NQ_MAX - 8;
         unsigned long long t_start = 0;
         if (probe) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_start));
         auto stamp = [&](int slot) {
             if (probe) {
                 unsigned long long t;
                 asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-                dbg_first[cta * NQ_MAX + 248 + slot] = static_cast<int>(t - t_start);
+                dbg_first[cta * NQ_MAX + NQ_MAX - 8 + slot] = static_cast<int>(t - t_start);
             }
         };
         const uint32_t tlane = tmem_base + (static_cast<uint32_t>(qd * 32) << 16) + part * PART_COLS;
         uint32_t uc = 0;
 
-        // ---- items 0 .. warm-1 (tiles cta, cta + G, ...) are scanned "max-only": their exact scores feed the
+        // ---- items 0 .. warm-1 (tiles clu, clu + C, ...) are scanned "max-only": their exact scores feed the
         // running maxima from which the shared thresholds are built; they come back, with thresholds, as the
         // last items.
         for (int w = 0; w < warm; ++w) {
-            const uint32_t row0 = static_cast<uint32_t>(cta + w * G) * SCAN_TILE + part * PART_COLS;
+            const uint32_t row0 = static_cast<uint32_t>(clu + w * C) * SCAN_TILE + part * PART_COLS;
             const float* h_part = h_s + (w % H_RING) * SCAN_TILE + part * PART_COLS;
             // rows of (numerically) equal norm, all searchable -- fingerprints are unit vectors --: the best score of a
             // chunk is its maximum minus the common 0.5|x|^2 (FMNMX3 chain).  Otherwise (reconstructions of an
             // IVF-PQ index, raw vectors, halo / padding rows): exact, column by column.
-            bool edge = (static_cast<uint32_t>(cta + w * G) + 1u) * SCAN_TILE > ns32 || (tune & 4);
+            bool edge = (static_cast<uint32_t>(clu + w * C) + 1u) * SCAN_TILE > ns32 || (tune & 4);
             float hx = 0.f;
             for (int hq = 0; hq < n_half; ++hq, ++uc) {
                 const int acc = uc & 1;
@@ -472,7 +509,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                             if (j < nvalid) munit = fmaxf(munit, __uint_as_float(v[j]) - hc[j]);
                     }
                 }
-                if (hq == 0 ? active[0] : active[1]) smem_red_max(&lmax_s[hq * 128 + qd * 32 + lane], f2ord(munit));
+                if (hq == 0 ? active[0] : active[1]) smem_red_max(&lmax_part[hq * 128 + qd * 32 + lane], f2ord(munit));
                 tc_fence_before();
                 __syncwarp();
                 mbar_arrive_lane0(&bars->tempty[acc], lane);
@@ -550,10 +587,10 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                         const float te = hq == 0 ? t_exact[0] : t_exact[1];
                         const uint32_t rbase = row0 + c * 32;
                         if (!edge)
-                            scan_chunk_hits<false>(v, h_part + c * 32, te, 32, rbase, &cnt_s[q], &lmax_s[q], my_pool + q * POOL_CAP);
+                            scan_chunk_hits<false>(v, h_part + c * 32, te, 32, rbase, &cnt_s[q], &lmax_part[q], my_pool + q * POOL_CAP);
                         else
                             scan_chunk_hits<true>(v, h_part + c * 32, te, static_cast<int>(min(ns32 - min(ns32, rbase), 32u)), rbase,
-                                                  &cnt_s[q], &lmax_s[q], my_pool + q * POOL_CAP);
+                                                  &cnt_s[q], &lmax_part[q], my_pool + q * POOL_CAP);
                         __syncwarp();
                     }
                 }
@@ -576,18 +613,19 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         // all epilogue warps are done appending before counts are published
         asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
         {
-            const int q = e * QPW + lane;
-            if (lane < QPW && q < nq) {
-                const int c = cnt_s[q];
-                cnt[cta * NQ_MAX + q] = min(c, POOL_CAP);
-                if (c > POOL_CAP) flags[q] = 1;      // pool overflow -> exact fallback answers this query
+            const int ql = e * QPW + lane;
+            if (lane < QPW && ql < q_rows && qrow0 + ql < nq) {
+                const int c = cnt_s[ql];
+                cnt[cta * NQ_CTA + ql] = min(c, POOL_CAP);
+                if (c > POOL_CAP) flags[qrow0 + ql] = 1;      // pool overflow -> exact fallback answers this query
             }
         }
         if (lane == 0) smem_atom_inc(&bars->done);
     } else {
         // ------------------------------------------------------------ threshold reducer (last warp)
-        // For the queries assigned to this CTA: T = kg-th largest of the per-CTA maxima.  At least kg
-        // distinct rows score >= T, so dropping rows that score <= T can never lose a top-kg row.
+        // For the queries assigned to this CTA: T = kg-th largest of the G maxima (one per pair and accumulator column
+        // half, over disjoint row sets).  At least kg distinct rows score >= T, so dropping rows that score <= T can
+        // never lose a top-kg row.
         // The thresholds converge within the first few dozen tiles; afterwards the select runs rarely so
         // that this warp stops competing for its sub-partition's issue slots.
         uint32_t round = 0;
@@ -624,7 +662,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     }
 
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();                // no remote arrive, commit or multicast targets a CTA that has left
     if (warp == MMA_WARP) tmem_dealloc(tmem_base, 512);
 }
 
@@ -661,10 +699,12 @@ __device__ void bitonic_sort_desc(uint64_t* keys, int n) {
 
 struct SelBatch {
     int np[SEL_SLOTS];       // query rows of the pass held in every slot
+    int h[SEL_SLOTS];        // query rows per CTA of that pass: row q is local row q % h of the CTAs of rank q / h
     int grid_alloc;          // CTA dimension the pool / cnt arrays were allocated with
 };
 
-// grid (NQ_MAX, slots): block (q, slot) answers row q of the scan pass parked in `slot`
+// grid (NQ_MAX, slots): block (q, slot) answers row q of the scan pass parked in `slot`; its survivors are in the pools
+// of the grid_scan / 2 CTAs 2 c + rank that held it
 __global__ void __launch_bounds__(256)
 flat_select_kernel(SelBatch batch, int k, int grid_scan, int64_t n_rows, const float* __restrict__ q32,
                    const float* __restrict__ qn2, const float* __restrict__ x32, const float* __restrict__ hn,
@@ -683,8 +723,8 @@ flat_select_kernel(SelBatch batch, int k, int grid_scan, int64_t n_rows, const f
     q32 += static_cast<int64_t>(slot) * NQ_MAX * D128;
     qn2 += slot * NQ_MAX;
     Tg += slot * NQ_MAX;
-    pool += static_cast<int64_t>(slot) * batch.grid_alloc * NQ_MAX * POOL_CAP;
-    cnt += static_cast<int64_t>(slot) * batch.grid_alloc * NQ_MAX;
+    pool += static_cast<int64_t>(slot) * batch.grid_alloc * NQ_CTA * POOL_CAP;
+    cnt += static_cast<int64_t>(slot) * batch.grid_alloc * NQ_CTA;
     flags += slot * NQ_MAX;
     gidx += slot * NQ_MAX;
     const int64_t g = gidx[q];
@@ -698,12 +738,14 @@ flat_select_kernel(SelBatch batch, int k, int grid_scan, int64_t n_rows, const f
     if (threadIdx.x == 0) total_s = 0;
     __syncthreads();
     bool over = false;
-    for (int g = threadIdx.x; g < grid_scan; g += blockDim.x) {
-        const int c = cnt[g * NQ_MAX + q];
+    const int rank = q / batch.h[slot], ql = q - rank * batch.h[slot];
+    for (int pr = threadIdx.x; pr < grid_scan / 2; pr += blockDim.x) {
+        const int cta = 2 * pr + rank;
+        const int c = cnt[cta * NQ_CTA + ql];
         if (c > 0) {
             const int base = atomicAdd(&total_s, c);
             if (base + c <= SELECT_CAP) {
-                const uint64_t* src = pool + (static_cast<int64_t>(g) * NQ_MAX + q) * POOL_CAP;
+                const uint64_t* src = pool + (static_cast<int64_t>(cta) * NQ_CTA + ql) * POOL_CAP;
                 for (int i = 0; i < c; ++i) keys[base + i] = src[i];
             } else {
                 over = true;
@@ -985,19 +1027,42 @@ int flat_add_dev(nafp_index* idx, const float* x, int64_t n, bool src_is_host) {
     return NAFP_OK;
 }
 
+// flat_scan_kernel runs as clusters of two CTAs
+static cudaLaunchConfig_t scan_launch_config(int grid, cudaStream_t stream, cudaLaunchAttribute (&attr)[1]) {
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(SCAN_THREADS);
+    cfg.dynamicSmemBytes = SCAN_SMEM;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cfg;
+}
+
 static int ensure_scratch(nafp_index* idx) {
     if (idx->scratch_ready) return NAFP_OK;
     nafp_ctx* ctx = idx->ctx;
-    idx->grid = ctx->sm_count;
-    NAFP_REQUIRE(idx->grid <= 160, NAFP_ERR_UNSUPPORTED, "flat scan: %d SMs (reducer handles <= 160)", idx->grid);
+    NAFP_CUDA(cudaFuncSetAttribute(flat_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM));
+    // one CTA per SM (shared memory); the scan runs as many CTA pairs as can be resident at once
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = scan_launch_config(2 * (ctx->sm_count / 2), ctx->stream, attr);
+    int clusters = 0;
+    NAFP_CUDA(cudaOccupancyMaxActiveClusters(&clusters, flat_scan_kernel, &cfg));
+    NAFP_REQUIRE(clusters >= 1, NAFP_ERR_UNSUPPORTED, "flat scan: no CTA pair of the scan kernel fits on this device");
+    idx->grid = 2 * clusters;
+    NAFP_REQUIRE(idx->grid <= 160, NAFP_ERR_UNSUPPORTED, "flat scan: %d CTAs (reducer handles <= 160)", idx->grid);
     const int G = idx->grid;
     NAFP_CUDA(cudaMalloc(&idx->qbf, NQ_MAX * D128 * sizeof(__nv_bfloat16)));
     NAFP_CUDA(cudaMalloc(&idx->q32, SEL_SLOTS * NQ_MAX * D128 * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&idx->qn2, SEL_SLOTS * NQ_MAX * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&idx->Mx, static_cast<size_t>(NQ_MAX) * G * sizeof(int32_t)));
     NAFP_CUDA(cudaMalloc(&idx->Tg, SEL_SLOTS * NQ_MAX * sizeof(int32_t)));
-    NAFP_CUDA(cudaMalloc(&idx->pool, SEL_SLOTS * static_cast<size_t>(G) * NQ_MAX * POOL_CAP * sizeof(uint64_t)));
-    NAFP_CUDA(cudaMalloc(&idx->cnt, SEL_SLOTS * static_cast<size_t>(G) * NQ_MAX * sizeof(int32_t)));
+    NAFP_CUDA(cudaMalloc(&idx->pool, SEL_SLOTS * static_cast<size_t>(G) * NQ_CTA * POOL_CAP * sizeof(uint64_t)));
+    NAFP_CUDA(cudaMalloc(&idx->cnt, SEL_SLOTS * static_cast<size_t>(G) * NQ_CTA * sizeof(int32_t)));
     NAFP_CUDA(cudaMalloc(&idx->flags, SEL_SLOTS * NQ_MAX * sizeof(int32_t)));
     NAFP_CUDA(cudaMalloc(&idx->gidx, SEL_SLOTS * NQ_MAX * sizeof(int64_t)));
     NAFP_CUDA(cudaMalloc(&idx->brute_part, static_cast<size_t>(BRUTE_SLOTS) * BRUTE_CHUNKS * MAX_K * sizeof(uint64_t)));
@@ -1009,7 +1074,6 @@ static int ensure_scratch(nafp_index* idx) {
     const uint32_t box[2] = {64, 32};
     NAFP_TRY(make_tensor_map(&idx->tmap_q, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, idx->qbf, dims, strides, box, nullptr,
                              CU_TENSOR_MAP_SWIZZLE_128B));
-    NAFP_CUDA(cudaFuncSetAttribute(flat_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM));
     idx->scratch_ready = true;
     return NAFP_OK;
 }
@@ -1040,29 +1104,32 @@ static int scan_tune() {
 static int scan_pass(nafp_index* idx, const float* q_dev, const int32_t* src_list, int src_off, int64_t p0, int np, int kg,
                      int grid_scan, int n_tiles, int64_t n_search, int slot) {
     nafp_ctx* ctx = idx->ctx;
-    const int n_half = np > 128 ? 2 : 1;
-    const int nq_pad = n_half * 128;
+    const int n_half = np > NQ_MAX / 2 ? 2 : 1;      // 128-row query blocks per CTA; rank r takes rows [r h, r h + h)
+    const int nq_pad = 2 * n_half * 128;
     const int64_t G = idx->grid;
     float* q32 = idx->q32 + static_cast<int64_t>(slot) * NQ_MAX * D128;
     float* qn2 = idx->qn2 + slot * NQ_MAX;
     int32_t* Tg = idx->Tg + slot * NQ_MAX;
-    uint64_t* pool = idx->pool + static_cast<int64_t>(slot) * G * NQ_MAX * POOL_CAP;
-    int32_t* cnt = idx->cnt + static_cast<int64_t>(slot) * G * NQ_MAX;
+    uint64_t* pool = idx->pool + static_cast<int64_t>(slot) * G * NQ_CTA * POOL_CAP;
+    int32_t* cnt = idx->cnt + static_cast<int64_t>(slot) * G * NQ_CTA;
     int32_t* flags = idx->flags + slot * NQ_MAX;
     int64_t* gidx = idx->gidx + slot * NQ_MAX;
     flat_prep_kernel<<<(nq_pad * 32 + 255) / 256, 256, 0, ctx->stream>>>(q_dev, src_list, src_off, p0, np, nq_pad, grid_scan,
                                                                          idx->qbf, q32, qn2, idx->Mx, Tg, flags, gidx, idx->tile_counter);
     const bool prof = idx->profile && idx->prof_n < PROF_RING;
     if (prof) cudaEventRecord(idx->prof_ev[2 * idx->prof_n], ctx->stream);
-    flat_scan_kernel<<<grid_scan, SCAN_THREADS, SCAN_SMEM, ctx->stream>>>(idx->tmap_q, idx->tmap_db, idx->hn, idx->tile_counter, n_search,
-                                                                          n_tiles, np, n_half, kg, idx->Mx, Tg, pool, cnt, flags,
-                                                                          idx->dbg_first, scan_tune());
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = scan_launch_config(grid_scan, ctx->stream, attr);
+    NAFP_CUDA(cudaLaunchKernelEx(&cfg, flat_scan_kernel, idx->tmap_q, idx->tmap_db, static_cast<const float*>(idx->hn),
+                                 idx->tile_counter, n_search, n_tiles, np, n_half, kg, idx->Mx, Tg, pool, cnt, flags,
+                                 idx->dbg_first, scan_tune()));
     if (prof) {
         cudaEventRecord(idx->prof_ev[2 * idx->prof_n + 1], ctx->stream);
         idx->prof_n++;
     }
     ctx->launches += 2;
     idx->last_slot = slot;
+    idx->last_h = n_half * 128;
     return NAFP_OK;
 }
 
@@ -1094,7 +1161,8 @@ int flat_search_dev(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     const int64_t n_search = (idx->search_rows >= 0 && idx->search_rows < idx->n) ? idx->search_rows : idx->n;
     const int n_tiles = static_cast<int>((n_search + SCAN_TILE - 1) / SCAN_TILE);
     const int kg = k + 28;
-    const int grid_scan = n_tiles < idx->grid ? (n_tiles > 0 ? n_tiles : 1) : idx->grid;
+    // CTA pairs: at most one per tile.  grid_scan is also the number of maxima the thresholds are taken from
+    const int grid_scan = 2 * std::max(1, std::min(n_tiles, idx->grid / 2));
     const bool brute = (n_search < 8192) || (kg > grid_scan) || (k > 64);
     idx->host_rows += nq;
     if (brute) return brute_rounds(idx, q_dev, nullptr, 0, nq, k, n_search, D_dev, I_dev);
@@ -1116,6 +1184,7 @@ int flat_search_dev(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     for (int64_t p0 = 0; p0 < nq; p0 += NQ_MAX) {
         const int np = static_cast<int>(nq - p0 < NQ_MAX ? nq - p0 : NQ_MAX);
         NAFP_TRY(scan_pass(idx, q_dev, nullptr, 0, p0, np, kg, grid_scan, n_tiles, n_search, slot));
+        batch.h[slot] = idx->last_h;
         batch.np[slot++] = np;
         idx->host_passes++;
         if (slot == SEL_SLOTS || p0 + NQ_MAX >= nq) {
@@ -1128,12 +1197,13 @@ int flat_search_dev(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     NAFP_CUDA(cudaMemcpyAsync(h, counts, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
     if (h[0] > 0) {
-        // second chance: a threshold about one spread of the per-CTA maxima lower (~2x the survivors)
+        // second chance: a threshold about one spread of the per-source maxima lower (~2x the survivors)
         const int kg_retry = 2 * kg < grid_scan - 2 ? 2 * kg : (grid_scan - 2 > kg ? grid_scan - 2 : kg);
         slot = 0;
         for (int off = 0; off < h[0]; off += NQ_MAX) {
             const int np = h[0] - off < NQ_MAX ? h[0] - off : NQ_MAX;
             NAFP_TRY(scan_pass(idx, q_dev, list1, off, 0, np, kg_retry, grid_scan, n_tiles, n_search, slot));
+            batch.h[slot] = idx->last_h;
             batch.np[slot++] = np;
             idx->host_passes++;
             if (slot == SEL_SLOTS || off + NQ_MAX >= h[0]) {
@@ -1311,9 +1381,19 @@ int nafp_index_reconstruct_host(nafp_index* idx, int64_t i0, int64_t n, float* o
     return NAFP_OK;
 }
 
-// developer probe: state of the last scan pass (flags, shared thresholds as float, survivors per query)
+// survivor counts of pass row q of the last scan pass: [grid][NQ_MAX], 0 in the CTAs that do not hold row q
+static int last_pass_counts(nafp_index* idx, std::vector<int32_t>& by_row) {
+    const size_t n_cta = static_cast<size_t>(idx->grid) * NQ_CTA;
+    std::vector<int32_t> cnt(n_cta);
+    NAFP_CUDA(cudaMemcpy(cnt.data(), idx->cnt + idx->last_slot * n_cta, n_cta * 4, cudaMemcpyDeviceToHost));
+    by_row.assign(static_cast<size_t>(idx->grid) * NQ_MAX, 0);
+    for (int g = 0; g < idx->grid; ++g)
+        for (int ql = 0; ql < idx->last_h; ++ql) by_row[static_cast<size_t>(g) * NQ_MAX + (g & 1) * idx->last_h + ql] = cnt[g * NQ_CTA + ql];
+    return NAFP_OK;
+}
+
 int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_out, int32_t* grid_out) {
-    // first call allocates the probe buffer; later calls copy cnt[grid][256] / first-threshold tile[grid][256]
+    // first call allocates the probe buffer; later calls copy cnt[grid][NQ_MAX] / first-threshold tile[grid][NQ_MAX]
     NAFP_REQUIRE(idx && idx->scratch_ready, NAFP_ERR_STATE, "debug: search once first");
     nafp_ctx* ctx = idx->ctx;
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1323,7 +1403,11 @@ int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_ou
         NAFP_CUDA(cudaMemset(idx->dbg_first, 0xFF, n * 4));
     }
     if (grid_out) *grid_out = idx->grid;
-    if (cnt_out) NAFP_CUDA(cudaMemcpy(cnt_out, idx->cnt + static_cast<size_t>(idx->last_slot) * n, n * 4, cudaMemcpyDeviceToHost));
+    if (cnt_out) {
+        std::vector<int32_t> by_row;
+        NAFP_TRY(last_pass_counts(idx, by_row));
+        memcpy(cnt_out, by_row.data(), n * 4);
+    }
     if (first_out) {
         NAFP_CUDA(cudaMemcpy(first_out, idx->dbg_first, n * 4, cudaMemcpyDeviceToHost));
         NAFP_CUDA(cudaMemset(idx->dbg_first, 0xFF, n * 4));
@@ -1331,21 +1415,22 @@ int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_ou
     return NAFP_OK;
 }
 
-int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags256, float* thr256, int32_t* total256) {
-    NAFP_REQUIRE(idx && idx->scratch_ready && flags256 && thr256 && total256, NAFP_ERR_INVALID, "debug: bad arguments");
+// developer probe: state of the last scan pass (flags, shared thresholds as float, survivors per query row)
+int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags_out, float* thr_out, int32_t* total_out) {
+    NAFP_REQUIRE(idx && idx->scratch_ready && flags_out && thr_out && total_out, NAFP_ERR_INVALID, "debug: bad arguments");
     nafp_ctx* ctx = idx->ctx;
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
-    std::vector<int32_t> tg(NQ_MAX), cnt(static_cast<size_t>(idx->grid) * NQ_MAX);
-    NAFP_CUDA(cudaMemcpy(flags256, idx->flags + idx->last_slot * NQ_MAX, NQ_MAX * 4, cudaMemcpyDeviceToHost));
+    std::vector<int32_t> tg(NQ_MAX), cnt;
+    NAFP_CUDA(cudaMemcpy(flags_out, idx->flags + idx->last_slot * NQ_MAX, NQ_MAX * 4, cudaMemcpyDeviceToHost));
     NAFP_CUDA(cudaMemcpy(tg.data(), idx->Tg + idx->last_slot * NQ_MAX, NQ_MAX * 4, cudaMemcpyDeviceToHost));
-    NAFP_CUDA(cudaMemcpy(cnt.data(), idx->cnt + static_cast<size_t>(idx->last_slot) * cnt.size(), cnt.size() * 4, cudaMemcpyDeviceToHost));
+    NAFP_TRY(last_pass_counts(idx, cnt));
     for (int q = 0; q < NQ_MAX; ++q) {
         int32_t o = tg[q];
         uint32_t b = static_cast<uint32_t>(o >= 0 ? o : (o ^ 0x7FFFFFFF));
-        memcpy(&thr256[q], &b, 4);
+        memcpy(&thr_out[q], &b, 4);
         int64_t t = 0;
         for (int g = 0; g < idx->grid; ++g) t += cnt[static_cast<size_t>(g) * NQ_MAX + q];
-        total256[q] = static_cast<int32_t>(t);
+        total_out[q] = static_cast<int32_t>(t);
     }
     return NAFP_OK;
 }

@@ -9,7 +9,8 @@
 namespace nafp {
 
 constexpr int D128 = 128;            // fingerprint dimension the tensor-core scan is built for
-constexpr int NQ_MAX = 256;          // query rows per scan pass (two MMA M blocks of 128)
+constexpr int NQ_MAX = 512;          // query rows per scan pass: one CTA pair, NQ_CTA rows per CTA
+constexpr int NQ_CTA = 256;          // query rows of one scan CTA (two MMA M blocks of 128)
 constexpr int TILE_ROWS = 128;       // DB rows per TMA box / allocation granule
 constexpr int SCAN_TILE = 256;       // DB rows per scan tile (MMA N)
 constexpr int POOL_CAP = 128;        // candidate slots per (CTA, query) per pass
@@ -42,15 +43,16 @@ struct nafp_index {
 
     // per-pass scratch (allocated on first search); q32 .. gidx hold SEL_SLOTS passes
     int last_slot = 0;
+    int last_h = 0;                   // query rows per CTA of the last scan pass
     bool scratch_ready = false;
-    int grid = 0;
+    int grid = 0;                     // scan CTAs: 2 x the CTA pairs that fit on the device at once
     __nv_bfloat16* qbf = nullptr;     // [NQ_MAX][d]
     float* q32 = nullptr;             // [NQ_MAX][d] (pass-local copy, zero padded)
     float* qn2 = nullptr;             // [NQ_MAX]
-    int32_t* Mx = nullptr;            // [NQ_MAX][grid] per-CTA running max (ordered int)
+    int32_t* Mx = nullptr;            // [NQ_MAX][grid] running max per (cluster, accumulator column half) (ordered int)
     int32_t* Tg = nullptr;            // [NQ_MAX] shared threshold (ordered int)
-    uint64_t* pool = nullptr;         // [grid][NQ_MAX][POOL_CAP]
-    int32_t* cnt = nullptr;           // [grid][NQ_MAX]
+    uint64_t* pool = nullptr;         // [grid][NQ_CTA][POOL_CAP] per (CTA, local query row)
+    int32_t* cnt = nullptr;           // [grid][NQ_CTA]
     int32_t* flags = nullptr;         // [NQ_MAX] != 0 -> answered by the exact fallback
     int64_t* gidx = nullptr;          // [NQ_MAX] global query row of every pass row
     int32_t* fail_list = nullptr;     // [2 nq + 2] rows to retry / to scan exactly, + the two counters

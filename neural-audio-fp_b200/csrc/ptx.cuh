@@ -1,6 +1,7 @@
 // Thin inline-PTX wrappers for the sm_100a features the kernels use:
-// mbarrier, TMA (cp.async.bulk[.tensor]), tcgen05 (alloc / mma / commit / ld / fences).
-// Everything here is cta_group::1 (no CTA pairs yet).
+// mbarrier, TMA (cp.async.bulk[.tensor]), tcgen05 (alloc / mma / commit / ld / fences), and the cluster
+// forms the flat scan's CTA pairs use (multicast loads, remote arrives, st.async, cluster barrier).
+// Every MMA is cta_group::1: a pair shares its B operand through multicast, not through cta_group::2.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -69,6 +70,47 @@ __device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity)
         if (++spins > (1u << 24)) __trap();
     }
 }
+// Same, with cluster-scope acquire: for a barrier that a peer CTA completes (remote arrive, st.async), so that
+// what the peer wrote before it is visible here and to whatever this thread signals next.
+__device__ __forceinline__ void mbar_wait_parked_cluster(uint64_t* bar, uint32_t parity) {
+    uint32_t spins = 0;
+    for (;;) {
+        uint32_t ok;
+        asm volatile(
+            "{\n\t.reg .pred P;\n\t"
+            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2, %3;\n\t"
+            "selp.u32 %0, 1, 0, P;\n\t}\n"
+            : "=r"(ok)
+            : "r"(smem_u32(bar)), "r"(parity), "r"(2000u)
+            : "memory");
+        if (ok) return;
+        if (++spins > (1u << 24)) __trap();
+    }
+}
+
+// ---------------------------------------------------------------- clusters
+// all threads of all CTAs of the cluster; release / acquire order shared-memory accesses across it
+__device__ __forceinline__ void cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cluster address of the same object in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t map_shared_rank(const void* p, uint32_t rank) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
+    return r;
+}
+// arrive (+ expect bytes) on a peer CTA's mbarrier.  .relaxed: the data it announces carries its own completion,
+// and .release would cost a GPU-wide memory barrier per call
+__device__ __forceinline__ void mbar_arrive_expect_tx_remote(uint32_t bar_cluster, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.relaxed.cluster.shared::cluster.b64 _, [%0], %1;" ::"r"(bar_cluster), "r"(bytes)
+                 : "memory");
+}
+// 4-byte store into a peer CTA's shared memory that completes 4 bytes of transaction on the peer's mbarrier
+__device__ __forceinline__ void st_async_remote(uint32_t dst_cluster, int32_t v, uint32_t bar_cluster) {
+    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(dst_cluster), "r"(v),
+                 "r"(bar_cluster)
+                 : "memory");
+}
 
 // ---------------------------------------------------------------- TMA
 __device__ __forceinline__ void tma_prefetch_desc(const void* tmap) {
@@ -78,6 +120,15 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, ui
     asm volatile(
         "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+        : "memory");
+}
+// same box delivered to the same shared-memory offset, and completed on the same mbarrier offset, in every CTA of
+// `cta_mask` (bit i = cluster rank i); one read from L2 / HBM
+__device__ __forceinline__ void tma_load_2d_multicast(void* smem_dst, const void* tmap, uint64_t* bar, int32_t c0, int32_t c1,
+                                                      uint16_t cta_mask) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
+        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
         : "memory");
 }
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const void* tmap, uint64_t* bar, int32_t c0, int32_t c1, int32_t c2) {
@@ -153,6 +204,12 @@ __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, u
                  "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
+__device__ __forceinline__ void bulk_load_1d_multicast(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar,
+                                                       uint16_t cta_mask) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
+                 ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
+                 : "memory");
+}
 __device__ __forceinline__ void fence_proxy_async_smem() {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
@@ -183,6 +240,12 @@ __device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t adesc, uint
 // arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed
 __device__ __forceinline__ void tc_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+// same, arriving on the mbarrier at this offset in every CTA of `cta_mask` (bit i = cluster rank i)
+__device__ __forceinline__ void tc_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                 ::"r"(smem_u32(bar)), "h"(cta_mask)
+                 : "memory");
 }
 
 // 32 lanes x 32 consecutive fp32 columns: thread i of the warp gets lane (base_lane + i)

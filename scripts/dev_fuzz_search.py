@@ -11,7 +11,7 @@ rng = np.random.default_rng(int(sys.argv[1]) if len(sys.argv) > 1 else 0)
 n_cases = int(sys.argv[2]) if len(sys.argv) > 2 else 25
 for case in range(n_cases):
     n = int(rng.integers(8200, 260000))
-    nq = int(rng.choice([1, 2, 31, 32, 33, 127, 128, 129, 255, 256, 257, 300, 600]))
+    nq = int(rng.choice([1, 2, 31, 32, 33, 127, 128, 129, 255, 256, 257, 300, 511, 512, 513, 600, 1100]))
     k = int(rng.choice([1, 5, 20, 33, 64]))
     x = rng.standard_normal((n, 128)).astype(np.float32)
     mode = case % 3

@@ -24,12 +24,12 @@ idx.search_dev(q.data_ptr(), nq, 20, D.data_ptr(), I.data_ptr()); torch.cuda.syn
 g = ctypes.c_int32(); check(lib.nafp_index_debug_enable(idx.h, None, None, ctypes.byref(g))); G = g.value
 for rep in range(2):
     idx.search_dev(q.data_ptr(), nq, 20, D.data_ptr(), I.data_ptr()); torch.cuda.synchronize()
-    cnt = np.zeros((G, 256), np.int32); first = np.zeros((G, 256), np.int32)
+    cnt = np.zeros((G, 512), np.int32); first = np.zeros((G, 512), np.int32)
     check(lib.nafp_index_debug_enable(idx.h, ptr(cnt), ptr(first), None))
-    t = first[:, 248:256]
+    t = first[:, 504:512]
     print("rep", rep, "G", G, "ns since start: tile0 done / thresholds ok / first thresholded tile done / own tiles done / end / item 16 done / item 32 done / item 96 done")
     print(" median", np.median(t, 0).tolist(), " min", t.min(0).tolist(), " max", t.max(0).tolist())
-    print(" survivors per CTA-query: mean", cnt[:, :nq].mean(), "max", cnt[:, :nq].max())
+    print(" survivors per CTA-query: mean", cnt[:, :nq].sum() / (nq * G // 2), "max", cnt[:, :nq].max())   # G / 2 CTAs hold each row
     own = t[:, 3]
     order = np.argsort(own)
     print(" own-tiles-done ns by CTA (sorted): fastest", [(int(c), int(own[c])) for c in order[:6]], "slowest", [(int(c), int(own[c])) for c in order[-10:]])
