@@ -159,6 +159,15 @@ int nafp_index_ivfpq_set_params(nafp_index* idx, const float* coarse_host, const
  * the refinement codebooks ((4, 16, 32) float32) in addition to nafp_index_ivfpq_get/set_params. */
 int nafp_index_ivfpqr_get_refine(nafp_index* idx, float* refine_pq_host);
 int nafp_index_ivfpqr_set_refine(nafp_index* idx, const float* refine_pq_host);
+/* The two levels of an IVFPQR search, for a row-sharded index whose shards must return what one index over all rows
+ * returns: (1) every shard's first-level top kc (= 4 k) by ADC distance, all-gathered and merged by
+ * nafp_topk_merge_dev into the global top kc; (2) every shard re-ranks the merged candidates whose labels it owns
+ * (its searched rows) by |q - (xhat + rhat)|^2 and returns its own sorted top k (+inf / -1 padding); those
+ * lists merge into the global top k.  nafp_index_search_dev runs both on one index.  kc <= 128. */
+int nafp_index_ivfpqr_first_level_dev(nafp_index* idx, const float* q_dev, int64_t nq, int kc, float* D_dev,
+                                      int64_t* I_dev);
+int nafp_index_ivfpqr_rerank_dev(nafp_index* idx, const float* q_dev, int64_t nq, const int64_t* candI_dev, int kc,
+                                 int k, float* D_dev, int64_t* I_dev);
 /* IVF-Flat and IVF-PQ: the coarse quantizer alone ((nlist,128) float32); import only on an empty index
  * (an IVF-Flat index counts as trained afterwards). */
 int nafp_index_ivf_get_coarse(nafp_index* idx, float* coarse_host);

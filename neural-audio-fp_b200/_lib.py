@@ -73,6 +73,8 @@ _SIGS = {
     "nafp_index_ivfpq_set_params": (c_int, [c_void_p, c_void_p, c_void_p]),
     "nafp_index_ivfpqr_get_refine": (c_int, [c_void_p, c_void_p]),
     "nafp_index_ivfpqr_set_refine": (c_int, [c_void_p, c_void_p]),
+    "nafp_index_ivfpqr_first_level_dev": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "nafp_index_ivfpqr_rerank_dev": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "nafp_index_ivf_get_coarse": (c_int, [c_void_p, c_void_p]),
     "nafp_index_ivf_set_coarse": (c_int, [c_void_p, c_void_p]),
     "nafp_index_reserve": (c_int, [c_void_p, c_int64]),

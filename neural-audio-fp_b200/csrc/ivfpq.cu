@@ -718,9 +718,11 @@ ivfpqr_encode_kernel(const float* __restrict__ x32, const int32_t* __restrict__ 
     }
 }
 // search: block = query row; its kc first-level candidates are re-scored as |q - (xhat + rhat)|^2 (a warp per candidate),
-// sorted by (distance, label), the k best are returned (IndexIVFPQR::search_preassigned)
+// sorted by (distance, label), the k best are returned (IndexIVFPQR::search_preassigned).  Only labels of the index's
+// searched rows [label_offset, label_offset + n_search) are re-scored: a shard of a row-sharded index re-ranks the
+// candidates it owns out of the global first-level top kc.
 __global__ void __launch_bounds__(128)
-ivfpqr_rerank_kernel(const float* __restrict__ q, const float* __restrict__ candD, const int64_t* __restrict__ candI, int kc, int k,
+ivfpqr_rerank_kernel(const float* __restrict__ q, const int64_t* __restrict__ candI, int kc, int k, int64_t n_search,
                      const int32_t* __restrict__ assign, const uint8_t* __restrict__ codes, const uint8_t* __restrict__ rcodes,
                      const float* __restrict__ coarse, const float* __restrict__ pq, int m, int dsub, const float* __restrict__ rpq,
                      int64_t label_offset, float* __restrict__ D, int64_t* __restrict__ I) {
@@ -733,8 +735,8 @@ ivfpqr_rerank_kernel(const float* __restrict__ q, const float* __restrict__ cand
     __syncthreads();
     for (int c = warp; c < kc; c += 4) {
         const int64_t id = candI[qi * kc + c];
-        if (id < 0) continue;
         const int64_t row = id - label_offset;
+        if (id < 0 || row < 0 || row >= n_search) continue;
         float4 xh = pq_reconstruct_lane(coarse, pq, m, dsub, assign[row], codes + row * m, lane);
         const int sub = lane >> 3;
         const int code = (rcodes[row * 2 + (sub >> 1)] >> (4 * (sub & 1))) & 15;
@@ -1030,6 +1032,14 @@ int build_lists(nafp_index* idx) {
 
 __global__ void topk_merge_kernel(const float* __restrict__ D_all, const int64_t* __restrict__ I_all, int W, int64_t nq,
                                   int k, float* __restrict__ D_out, int64_t* __restrict__ I_out);
+constexpr int TOPK_MERGE_KEYS = 4096;     // keys one topk_merge_kernel block sorts (seq_match.cu)
+// merge blocks per query row of the LUT scan: 1 when the nprobe * k partial keys fit one block, else the number of
+// groups of floor(4096 / k) probes merged in a first round
+static int lut_merge_groups(int nprobe, int k) {
+    if (nprobe * k <= TOPK_MERGE_KEYS) return 1;
+    const int G = TOPK_MERGE_KEYS / k;
+    return (nprobe + G - 1) / G;
+}
 
 // the reference formulation: per (query row, probed list) LUT + ADC scan of the list's codes
 int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev) {
@@ -1037,8 +1047,9 @@ int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, flo
     nafp_ctx* ctx = idx->ctx;
     if (nq == 0) return NAFP_OK;
     const int nprobe = idx->nprobe < s->nlist ? idx->nprobe : s->nlist;
-    NAFP_REQUIRE(k >= 1 && k <= MAX_K && nprobe * k <= 4096, NAFP_ERR_INVALID,
-                 "ivfpq search: need k <= %d and nprobe*k <= 4096 (nprobe %d, k %d)", MAX_K, nprobe, k);
+    NAFP_REQUIRE(k >= 1 && k <= MAX_K && lut_merge_groups(nprobe, k) * k <= TOPK_MERGE_KEYS, NAFP_ERR_INVALID,
+                 "ivfpq search: need k <= %d and ceil(nprobe / floor(%d / k)) * k <= %d (nprobe %d, k %d)", MAX_K, TOPK_MERGE_KEYS,
+                 TOPK_MERGE_KEYS, nprobe, k);
     NAFP_TRY(build_lists(idx));
     const int64_t n_search = (idx->search_rows >= 0 && idx->search_rows < idx->n) ? idx->search_rows : idx->n;
     const int64_t chunk = 4096;       // query rows per launch group (bounds the partial buffers)
@@ -1069,8 +1080,21 @@ int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, flo
             ivfpq_scan_kernel<<<dim3(nprobe, static_cast<unsigned>(nc)), 256, lut_bytes, ctx->stream>>>(
                 qp, nc, s->coarse, s->pq, s->m, s->dsub, s->probes, nprobe, s->lcodes, s->lids, s->loff, s->lend, k, idx->label_offset,
                 n_search, s->partD, s->partI);
-        topk_merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(s->partD, s->partI, nprobe, nc, k, D_dev + q0 * k,
-                                                                              I_dev + q0 * k);
+        const int groups = lut_merge_groups(nprobe, k);
+        if (groups > 1) {
+            // nprobe * k keys exceed one merge block: merge groups of G probes first.  The result of group g lands in the
+            // partials of probe g of the same row, which group 0 (g < G) has already consumed; every block reads all its
+            // inputs before it writes, so group 0 may overwrite its own probe 0.  Then merge the `groups` partial lists.
+            const int G = TOPK_MERGE_KEYS / k;
+            for (int g = 0; g < groups; ++g) {
+                const int64_t in = static_cast<int64_t>(g) * G * nc * k, out = static_cast<int64_t>(g) * nc * k;
+                topk_merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(
+                    s->partD + in, s->partI + in, std::min(G, nprobe - g * G), nc, k, s->partD + out, s->partI + out);
+            }
+            ctx->launches += groups;
+        }
+        topk_merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(s->partD, s->partI, groups > 1 ? groups : nprobe, nc, k,
+                                                                              D_dev + q0 * k, I_dev + q0 * k);
         ctx->launches += 3;
     }
     NAFP_CUDA(cudaGetLastError());
@@ -1119,6 +1143,8 @@ int ivfpq_redo_rows(nafp_index* idx, const float* q_dev, int32_t n_redo, int k, 
 }
 
 static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev);
+static int ivfpqr_rerank(nafp_index* idx, const float* q_dev, int64_t nq, const int64_t* candI_dev, int kc, int k, float* D_dev,
+                         int64_t* I_dev);
 
 int ivfpq_search_dev(nafp_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev) {
     IvfPq* s = idx->ivf;
@@ -1139,8 +1165,18 @@ int ivfpq_search_dev(nafp_index* idx, const float* q_dev, int64_t nq, int k, flo
         s->ref_nq = nq;
     }
     NAFP_TRY(ivfpq_search_first_level(idx, q_dev, nq, kc, s->refD, s->refI));
-    ivfpqr_rerank_kernel<<<static_cast<unsigned>(nq), 128, 0, ctx->stream>>>(q_dev, s->refD, s->refI, kc, k, s->assign, s->codes, s->rcodes,
-                                                                             s->coarse, s->pq, s->m, s->dsub, s->rpq,
+    return ivfpqr_rerank(idx, q_dev, nq, s->refI, kc, k, D_dev, I_dev);
+}
+
+static int ivfpqr_rerank(nafp_index* idx, const float* q_dev, int64_t nq, const int64_t* candI_dev, int kc, int k, float* D_dev,
+                         int64_t* I_dev) {
+    IvfPq* s = idx->ivf;
+    nafp_ctx* ctx = idx->ctx;
+    NAFP_REQUIRE(k >= 1 && k <= kc && kc <= MAX_K, NAFP_ERR_INVALID, "ivfpq-rr re-rank: need 1 <= k <= kc <= %d (k %d, kc %d)", MAX_K, k, kc);
+    if (nq == 0) return NAFP_OK;
+    const int64_t n_search = (idx->search_rows >= 0 && idx->search_rows < idx->n) ? idx->search_rows : idx->n;
+    ivfpqr_rerank_kernel<<<static_cast<unsigned>(nq), 128, 0, ctx->stream>>>(q_dev, candI_dev, kc, k, n_search, s->assign, s->codes,
+                                                                             s->rcodes, s->coarse, s->pq, s->m, s->dsub, s->rpq,
                                                                              idx->label_offset, D_dev, I_dev);
     ctx->launches++;
     NAFP_CUDA(cudaGetLastError());
@@ -1154,8 +1190,9 @@ static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t
     NAFP_CUDA(cudaSetDevice(ctx->device));
     if (nq == 0) return NAFP_OK;
     const int nprobe = idx->nprobe < s->nlist ? idx->nprobe : s->nlist;
-    NAFP_REQUIRE(k >= 1 && k <= MAX_K && nprobe * k <= 4096, NAFP_ERR_INVALID,
-                 "ivfpq search: need k <= %d and nprobe*k <= 4096 (nprobe %d, k %d)", MAX_K, nprobe, k);
+    NAFP_REQUIRE(k >= 1 && k <= MAX_K && lut_merge_groups(nprobe, k) * k <= TOPK_MERGE_KEYS, NAFP_ERR_INVALID,
+                 "ivfpq search: need k <= %d and ceil(nprobe / floor(%d / k)) * k <= %d (nprobe %d, k %d)", MAX_K, TOPK_MERGE_KEYS,
+                 TOPK_MERGE_KEYS, nprobe, k);
     if (!s->flat_lists) idx->host_rows += nq;          // (the flat scan of an IVF-Flat index counts its own rows)
     if (nq >= (1ll << 31)) return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
     if (!s->flat_lists) {
@@ -1281,6 +1318,23 @@ int nafp_index_ivfpqr_set_refine(nafp_index* idx, const float* refine_pq_host) {
     NAFP_CUDA(cudaMemcpy(idx->ivf->rpq, refine_pq_host, static_cast<size_t>(REFINE_M) * REFINE_KSUB * REFINE_DSUB * sizeof(float),
                          cudaMemcpyHostToDevice));
     return NAFP_OK;
+}
+
+int nafp_index_ivfpqr_first_level_dev(nafp_index* idx, const float* q_dev, int64_t nq, int kc, float* D_dev, int64_t* I_dev) {
+    NAFP_RANGE("nafp_index_ivfpqr_first_level_dev");
+    NAFP_REQUIRE(idx && idx->ivf && idx->ivf->refine && nq >= 0 && (nq == 0 || (q_dev && D_dev && I_dev)), NAFP_ERR_INVALID,
+                 "nafp_index_ivfpqr_first_level_dev: not an IVFPQR index, or bad arguments");
+    return ivfpq_search_first_level(idx, q_dev, nq, kc, D_dev, I_dev);
+}
+
+int nafp_index_ivfpqr_rerank_dev(nafp_index* idx, const float* q_dev, int64_t nq, const int64_t* candI_dev, int kc, int k,
+                                 float* D_dev, int64_t* I_dev) {
+    NAFP_RANGE("nafp_index_ivfpqr_rerank_dev");
+    NAFP_REQUIRE(idx && idx->ivf && idx->ivf->refine && nq >= 0 && (nq == 0 || (q_dev && candI_dev && D_dev && I_dev)),
+                 NAFP_ERR_INVALID, "nafp_index_ivfpqr_rerank_dev: not an IVFPQR index, or bad arguments");
+    NAFP_REQUIRE(idx->ivf->trained, NAFP_ERR_STATE, "nafp_index_ivfpqr_rerank_dev: index is not trained");
+    NAFP_CUDA(cudaSetDevice(idx->ctx->device));
+    return ivfpqr_rerank(idx, q_dev, nq, candI_dev, kc, k, D_dev, I_dev);
 }
 
 }  // extern "C"

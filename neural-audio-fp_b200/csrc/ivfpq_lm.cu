@@ -27,6 +27,10 @@
 // enter the top k, so almost nothing is inserted.  ivfpq_lm_merge_kernel re-scores the survivors with the LUT
 // kernel's own fp32 arithmetic, sorts, and PROVES the answer (a full 32-entry list must end below the k-th exact
 // distance by more than the rounding bound); unproven rows -- duplicates, ties -- go to the LUT kernel.
+//
+// k > 24 (up to 128, the 4 k first-level candidates of IVFPQR): every (query row, probed list) pair becomes S = ceil(k / 24)
+// SLICES, each over a disjoint contiguous range of the list's tiles with its own two 32-entry lists; the waves, the bound
+// and the proof walk S times as many lists.  Wave 0 then keeps S * 64 >= 2.6 k candidates of the nearest list.
 #include <algorithm>
 #include <cfloat>
 #include <climits>
@@ -43,8 +47,10 @@ constexpr int LM_Q = 128;                 // query rows per work item (MMA M, TM
 constexpr int LM_KP = 32;                 // entries of one warp-wide sorted candidate list
 constexpr int LM_GROUPS = 2;              // epilogue warp groups: each keeps its own list per query for its half of a tile's columns
 constexpr int LM_SLOT = LM_KP * LM_GROUPS; // candidates kept per (query row, probed list)
-constexpr int LM_MAX_K = 24;              // k the path answers (k + 8 spare candidates for the proof)
-constexpr int LM_MAX_NPROBE = 64;         // nprobe * LM_SLOT candidates are sorted by one block
+constexpr int LM_SLICE_K = 24;            // k one slice of a list answers (k + 8 spare candidates for the proof)
+constexpr int LM_MAX_K = 128;             // k the path answers: ceil(k / LM_SLICE_K) slices per (query row, probed list)
+constexpr int LM_MAX_NPROBE = 64;
+constexpr int LM_MERGE_KEYS = LM_MAX_NPROBE * LM_SLOT;  // survivors one merge block sorts (every candidate when S = 1)
 constexpr int LM_STAGES = 2;
 constexpr int LM_WAVES = 3;               // launches per search: probe rank 0 | ranks 1 .. LM_WAVE1_END-1 | the rest
 constexpr int LM_WAVE1_END = 4;
@@ -59,14 +65,17 @@ constexpr int LM_B_BYTES = 3 * LM_KB_BYTES;             // 48 KB per stage: two 
 constexpr int LM_TAB_BYTES = 64 * PQ_KSUB * 4;          // 64 KB: [sub-quantizer][code] -> two bf16
 constexpr int LM_LIST_BYTES = LM_Q * LM_SLOT * 8;       // 64 KB
 constexpr int LM_SMEM = 1024 + LM_STAGES * LM_B_BYTES + LM_TAB_BYTES + LM_LIST_BYTES + 512;
-constexpr int64_t LM_CHUNK_Q = 32768;     // query rows per launch group (bounds the candidate buffer: 256 B per pair)
+constexpr int64_t LM_CHUNK_Q = 32768;     // query rows per launch group at S = 1, LM_CHUNK_Q / S at S slices (bounds the
+                                          // candidate buffer: 512 B per pair and slice)
 static_assert(LM_ROWS == 128, "the epilogue reads four 32-column chunks per tile");
 static_assert(LM_Q == LM_ROWS, "the query block and the tile share the K-block size");
 
 __host__ __device__ __forceinline__ int lm_wave(int p) { return p == 0 ? 0 : (p < LM_WAVE1_END ? 1 : 2); }
+static int lm_slices(int k) { return (k + LM_SLICE_K - 1) / LM_SLICE_K; }
 
 struct LmItem {
-    int32_t list, start, len, tiles;      // query pairs[start .. start + len) against list `list`
+    int32_t list, start, len, tiles;      // query pairs[start .. start + len) against tiles [t0, t0 + tiles) of list `list`
+    int32_t t0, slice;                    // ... which are slice `slice` of the list
 };
 
 struct LmState {
@@ -81,8 +90,8 @@ struct LmState {
     float* qE = nullptr;                  // [nq] rounding bound of the bf16 scores
     float* dkA = nullptr;                 // [nq] k-th exact distance inside the nearest list
     int32_t* pairs = nullptr;             // [nq * nprobe] (query, probe) pairs grouped by (phase, list)
-    uint64_t* cand = nullptr;             // [nq * nprobe][LM_GROUPS][LM_KP]
-    int64_t cap_pairs = 0, cap_q = 0;
+    uint64_t* cand = nullptr;             // [nq * nprobe][S][LM_GROUPS][LM_KP]
+    int64_t cap_pairs = 0, cap_q = 0, cap_cand = 0;
     int32_t* hist = nullptr;              // [LM_WAVES * nlist] bucket sizes, the same of scatter cursors, [LM_WAVES] item counters
     LmItem* items = nullptr;
     int64_t items_cap = 0;
@@ -358,7 +367,7 @@ __device__ __forceinline__ float lm_key_score(uint64_t key) {
 }
 
 __global__ void __launch_bounds__(LM_THREADS, 1)
-ivfpq_lm_scan_kernel(const float* __restrict__ q, int nprobe, const LmItem* __restrict__ items, int n_items,
+ivfpq_lm_scan_kernel(const float* __restrict__ q, int nprobe, int S, const LmItem* __restrict__ items, int n_items,
                      int32_t* __restrict__ item_counter, const int32_t* __restrict__ pairs, const uint32_t* __restrict__ tab,
                      const uint8_t* __restrict__ lcodes, const float* __restrict__ lh, const int32_t* __restrict__ loff,
                      const float* __restrict__ gdist, const float* __restrict__ dkA, const float* __restrict__ qE,
@@ -419,7 +428,7 @@ ivfpq_lm_scan_kernel(const float* __restrict__ q, int nprobe, const LmItem* __re
         const int it = bars->item;
         if (it >= n_items) break;
         const LmItem item = items[it];
-        const int lo = __ldg(loff + item.list);
+        const int lo = __ldg(loff + item.list) + item.t0 * LM_ROWS;      // first position of the slice
         const int T = item.tiles;
         // The item's query rows -> bf16 -> TENSOR MEMORY (columns [LM_TMEM_A, + 64) of the query's lane): the A operand of
         // every MMA of the item (no shared memory for it: the second set of candidate lists lives there instead).
@@ -624,14 +633,15 @@ ivfpq_lm_scan_kernel(const float* __restrict__ q, int nprobe, const LmItem* __re
             }
         }
         __syncthreads();            // every accumulator of the item was consumed, every candidate list is final
-        if (warp < LM_EPI_WARPS) {  // the item's candidate lists -> cand[pair][group][32]
+        if (warp < LM_EPI_WARPS) {  // the item's candidate lists -> cand[pair][slice][group][32]
             const int qd = warp & 3, half = warp >> 2;
             const int ql = qd * 32 + lane;
-            const int pid = ql < item.len ? __ldg(pairs + item.start + ql) : 0;
+            // (the lane's (pair, slice) row of cand, formed once so that the copy loop is the same as without slices)
+            const int row = ql < item.len ? __ldg(pairs + item.start + ql) * S + item.slice : 0;
             const uint64_t* wl = lst_s + (half * LM_Q + qd * 32) * LM_KP;
             for (int qi = 0; qi < 32; ++qi) {
-                const int pq_id = __shfl_sync(0xffffffffu, pid, qi);
-                if (qd * 32 + qi < item.len) cand[static_cast<int64_t>(pq_id) * LM_SLOT + half * LM_KP + lane] = wl[qi * LM_KP + lane];
+                const int cr = __shfl_sync(0xffffffffu, row, qi);
+                if (qd * 32 + qi < item.len) cand[static_cast<int64_t>(cr) * LM_SLOT + half * LM_KP + lane] = wl[qi * LM_KP + lane];
             }
         }
     }
@@ -669,39 +679,45 @@ __device__ __forceinline__ float lm_exact_adc(const float* __restrict__ qs, cons
 }
 
 // one warp per query row: Dk = the k-th smallest exact distance among the candidates of the lists scanned so far
-// (probe ranks [0, pend), pend <= LM_WAVE1_END; +inf if they gave fewer than k) -- the next wave's threshold
+// (probe ranks [0, pend), pend <= LM_WAVE1_END; +inf if they gave fewer than k) -- the next wave's threshold.
+// Dynamic shared memory: lm_bound_smem(S).  (S is a template parameter here and in the merge: at S = 1 their index
+// arithmetic compiles to the same shifts as before slices existed.)
+__host__ __device__ constexpr int lm_bound_smem(int S) { return 8 * (D128 + LM_WAVE1_END * S * LM_SLOT) * 4; }
+template <int S>
 __global__ void ivfpq_lm_bound_kernel(const float* __restrict__ q, int64_t nq, int nprobe, int pend, int k,
                                       const uint64_t* __restrict__ cand, const int32_t* __restrict__ probes,
                                       const float* __restrict__ gdist, const float* __restrict__ qE,
                                       const float* __restrict__ coarse, const float* __restrict__ pq,
                                       const uint8_t* __restrict__ lcodes, float* __restrict__ dkA) {
-    __shared__ float qs[8][D128];
-    __shared__ float ds[8][LM_WAVE1_END * LM_SLOT];
+    extern __shared__ float bsm[];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    float* qs = bsm + w * D128;                                       // [8 warps][128]
+    float* ds = bsm + 8 * D128 + w * (LM_WAVE1_END * S * LM_SLOT);    // [8 warps][LM_WAVE1_END * S * LM_SLOT]
     const int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
     if (i >= nq) return;
-    reinterpret_cast<float4*>(qs[w])[lane] = reinterpret_cast<const float4*>(q + i * D128)[lane];
+    reinterpret_cast<float4*>(qs)[lane] = reinterpret_cast<const float4*>(q + i * D128)[lane];
     __syncwarp();
     const float dk_prev = dkA[i];          // the previous wave's bound (3.4e38 before the first): what cannot beat it is not re-scored
     const float E = qE[i];
-    for (int p = 0; p < pend * LM_GROUPS; ++p) {               // (probe rank p / LM_GROUPS, list of epilogue group p % LM_GROUPS)
-        const uint64_t key = cand[(i * nprobe) * LM_SLOT + p * LM_KP + lane];
-        const int l = probes[i * nprobe + p / LM_GROUPS];
+    constexpr int per_probe = S * LM_GROUPS;   // lists of one (query row, probe rank): slice p / LM_GROUPS % S, epilogue group p % LM_GROUPS
+    for (int p = 0; p < pend * per_probe; ++p) {
+        const uint64_t key = cand[(i * nprobe) * S * LM_SLOT + p * LM_KP + lane];
+        const int l = probes[i * nprobe + p / per_probe];
         float d = INFINITY;
         // exact distance >= |q - c|^2 - 2 (bf16 score + E)
-        if (key != 0ull && l >= 0 && gdist[i * nprobe + p / LM_GROUPS] - 2.f * (lm_key_score(key) + E) <= dk_prev)
-            d = lm_exact_adc(qs[w], coarse + static_cast<int64_t>(l) * D128, pq, lcodes, static_cast<uint32_t>(key));
-        ds[w][p * LM_KP + lane] = d;
+        if (key != 0ull && l >= 0 && gdist[i * nprobe + p / per_probe] - 2.f * (lm_key_score(key) + E) <= dk_prev)
+            d = lm_exact_adc(qs, coarse + static_cast<int64_t>(l) * D128, pq, lcodes, static_cast<uint32_t>(key));
+        ds[p * LM_KP + lane] = d;
     }
     __syncwarp();
     // compact the re-scored distances (most slots were skipped), then rank them: the one of rank k - 1 is the bound
     int m = 0;
-    for (int p = 0; p < pend * LM_GROUPS; ++p) {
-        const float d = ds[w][p * LM_KP + lane];
+    for (int p = 0; p < pend * per_probe; ++p) {
+        const float d = ds[p * LM_KP + lane];
         const bool fin = d < INFINITY;
         const unsigned mask = __ballot_sync(0xffffffffu, fin);
         __syncwarp();
-        if (fin) ds[w][m + __popc(mask & ((1u << lane) - 1u))] = d;       // (target index <= source index: never an unread entry)
+        if (fin) ds[m + __popc(mask & ((1u << lane) - 1u))] = d;       // (target index <= source index: never an unread entry)
         m += __popc(mask);
         __syncwarp();
     }
@@ -710,17 +726,19 @@ __global__ void ivfpq_lm_bound_kernel(const float* __restrict__ q, int64_t nq, i
         return;
     }
     for (int r = lane; r < m; r += 32) {
-        const float d = ds[w][r];
+        const float d = ds[r];
         int rank = 0;
         for (int o = 0; o < m; ++o) {
-            const float od = ds[w][o];
+            const float od = ds[o];
             rank += (od < d || (od == d && o < r)) ? 1 : 0;
         }
         if (rank == k - 1) dkA[i] = d;
     }
 }
 
-// one block per query row: exact re-rank of the survivors of all probed lists, top k, proof
+// one block per query row: exact re-rank of the survivors of all probed lists, top k, proof.  At S = 1 every candidate
+// fits the key buffer; at S > 1 a row with more than LM_MERGE_KEYS survivors goes to the LUT kernel like an unproven one.
+template <int S>
 __global__ void __launch_bounds__(128)
 ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k, const uint64_t* __restrict__ cand,
                       const int32_t* __restrict__ probes, const float* __restrict__ gdist, const float* __restrict__ qE,
@@ -729,7 +747,7 @@ ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k
                       const int32_t* __restrict__ lids, int64_t label_offset, float* __restrict__ D, int64_t* __restrict__ I,
                       int32_t* __restrict__ redo_rows, int32_t* __restrict__ redo_count) {
     __shared__ float qs[D128];
-    __shared__ uint64_t keys[LM_MAX_NPROBE * LM_SLOT];
+    __shared__ uint64_t keys[LM_MERGE_KEYS];
     __shared__ int cnt_s, bound_s;
     const int64_t i = blockIdx.x;              // row inside the launch group
     const int tid = threadIdx.x;
@@ -737,22 +755,29 @@ ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k
     if (tid == 0) { cnt_s = 0; bound_s = INT_MAX; }
     __syncthreads();
     const float E = qE[i], dk = dkA[i];
-    const int total = nprobe * LM_SLOT;
+    constexpr int per_probe = S * LM_SLOT;
+    const int total = nprobe * per_probe;
     // 1. gather: compact (probe rank, list position) of every survivor; lower bound on the distance of what the
     //    full lists dropped: g - 2 (score of the list's last entry + E)
     for (int e = tid; e < total; e += blockDim.x) {
         const uint64_t key = cand[i * total + e];
         if (key != 0ull) {
-            const int p = e / LM_SLOT;
+            const int p = e / per_probe;
             // (a survivor whose distance cannot be below the last bound -- an upper bound of the k-th -- is not re-scored)
-            if (gdist[i * nprobe + p] - 2.f * (lm_key_score(key) + E) <= dk)
-                keys[atomicAdd(&cnt_s, 1)] = (static_cast<uint64_t>(p) << 32) | static_cast<uint32_t>(key);
+            if (gdist[i * nprobe + p] - 2.f * (lm_key_score(key) + E) <= dk) {
+                const int slot = atomicAdd(&cnt_s, 1);
+                if (slot < LM_MERGE_KEYS) keys[slot] = (static_cast<uint64_t>(p) << 32) | static_cast<uint32_t>(key);
+            }
             if ((e & (LM_KP - 1)) == LM_KP - 1)
                 atomicMin(&bound_s, f2ord(gdist[i * nprobe + p] - 2.f * (lm_key_score(key) + E)));
         }
     }
     __syncthreads();
     const int n = cnt_s;
+    if (n > LM_MERGE_KEYS) {
+        if (tid == 0) redo_rows[atomicAdd(redo_count, 1)] = static_cast<int32_t>(q0 + i);
+        return;
+    }
     int P = 32;
     while (P < n || P < k) P <<= 1;
     // 2. exact distances (the LUT kernel's arithmetic), key = (distance bits, row id): ascending order = faiss order,
@@ -793,23 +818,34 @@ ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k
 }
 
 // ------------------------------------------------------------------------------------------ host
-static int lm_reserve(nafp_index* idx, int64_t nc, int nprobe) {
+constexpr int LM_MAX_S = (LM_MAX_K + LM_SLICE_K - 1) / LM_SLICE_K;
+using LmBoundFn = decltype(&ivfpq_lm_bound_kernel<1>);
+using LmMergeFn = decltype(&ivfpq_lm_merge_kernel<1>);
+static const LmBoundFn lm_bound_fns[] = {ivfpq_lm_bound_kernel<1>, ivfpq_lm_bound_kernel<2>, ivfpq_lm_bound_kernel<3>,
+                                         ivfpq_lm_bound_kernel<4>, ivfpq_lm_bound_kernel<5>, ivfpq_lm_bound_kernel<6>};
+static const LmMergeFn lm_merge_fns[] = {ivfpq_lm_merge_kernel<1>, ivfpq_lm_merge_kernel<2>, ivfpq_lm_merge_kernel<3>,
+                                         ivfpq_lm_merge_kernel<4>, ivfpq_lm_merge_kernel<5>, ivfpq_lm_merge_kernel<6>};
+static_assert(sizeof(lm_bound_fns) / sizeof(lm_bound_fns[0]) == LM_MAX_S && sizeof(lm_merge_fns) / sizeof(lm_merge_fns[0]) == LM_MAX_S,
+              "one bound and one merge kernel per slice count");
+
+static int lm_reserve(nafp_index* idx, int64_t nc, int nprobe, int S) {
     LmState* L = idx->ivf->lm;
     const int64_t np = nc * nprobe;
-    if (L->cap_q < nc || L->cap_pairs < np) {
+    if (L->cap_q < nc || L->cap_pairs < np || L->cap_cand < np * S) {
         void* old[] = {L->probes, L->gdist, L->qE, L->dkA, L->pairs, L->cand};
         for (void* b : old) if (b) cudaFree(b);
         L->probes = nullptr; L->gdist = nullptr; L->qE = nullptr; L->dkA = nullptr; L->pairs = nullptr; L->cand = nullptr;
-        L->cap_q = 0; L->cap_pairs = 0;
-        const int64_t cq = std::max(nc, L->cap_q), cp = std::max(np, L->cap_pairs);
+        const int64_t cq = std::max(nc, L->cap_q), cp = std::max(np, L->cap_pairs), cc = std::max(np * S, L->cap_cand);
+        L->cap_q = 0; L->cap_pairs = 0; L->cap_cand = 0;
         NAFP_CUDA(cudaMalloc(&L->probes, static_cast<size_t>(cp) * sizeof(int32_t)));
         NAFP_CUDA(cudaMalloc(&L->gdist, static_cast<size_t>(cp) * sizeof(float)));
         NAFP_CUDA(cudaMalloc(&L->pairs, static_cast<size_t>(cp) * sizeof(int32_t)));
-        NAFP_CUDA(cudaMalloc(&L->cand, static_cast<size_t>(cp) * LM_SLOT * sizeof(uint64_t)));
+        NAFP_CUDA(cudaMalloc(&L->cand, static_cast<size_t>(cc) * LM_SLOT * sizeof(uint64_t)));
         NAFP_CUDA(cudaMalloc(&L->qE, static_cast<size_t>(cq) * sizeof(float)));
         NAFP_CUDA(cudaMalloc(&L->dkA, static_cast<size_t>(cq) * sizeof(float)));
         L->cap_q = cq;
         L->cap_pairs = cp;
+        L->cap_cand = cc;
     }
     return NAFP_OK;
 }
@@ -820,6 +856,8 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     const int nprobe = idx->nprobe < s->nlist ? idx->nprobe : s->nlist;
     const int nlist = s->nlist;
     const int64_t n_search = (idx->search_rows >= 0 && idx->search_rows < idx->n) ? idx->search_rows : idx->n;
+    const int S = lm_slices(k);
+    const int64_t chunk_q = LM_CHUNK_Q / S;
     NAFP_TRY(lm_prepare(idx, n_search));
     LmState* L = s->lm;
     NAFP_TRY(ivfpq_reserve_redo(idx, nq));
@@ -827,17 +865,20 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     NAFP_CUDA(cudaMemsetAsync(redo_count, 0, sizeof(int32_t), ctx->stream));
     NAFP_CUDA(cudaFuncSetAttribute(ivfpq_lm_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LM_SMEM));
     NAFP_CUDA(cudaFuncSetAttribute(lm_probe_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LM_PROBE_SMEM));
+    const LmBoundFn bound_kernel = lm_bound_fns[S - 1];
+    const LmMergeFn merge_kernel = lm_merge_fns[S - 1];
+    NAFP_CUDA(cudaFuncSetAttribute(bound_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lm_bound_smem(S)));
     int32_t* hist = L->hist;                                        // [LM_WAVES nlist]
     int32_t* cursor = L->hist + LM_WAVES * IVF_MAX_NLIST;           // [LM_WAVES nlist]
     int32_t* counters = L->hist + 2 * LM_WAVES * IVF_MAX_NLIST;     // [LM_WAVES]
     const int nb = LM_WAVES * nlist;
     std::vector<int32_t> h(nb), cur(nb);
     std::vector<LmItem> items;
-    for (int64_t q0 = 0; q0 < nq; q0 += LM_CHUNK_Q) {
-        const int64_t nc = nq - q0 < LM_CHUNK_Q ? nq - q0 : LM_CHUNK_Q;
+    for (int64_t q0 = 0; q0 < nq; q0 += chunk_q) {
+        const int64_t nc = nq - q0 < chunk_q ? nq - q0 : chunk_q;
         const int64_t np = nc * nprobe;
         const float* qp = q_dev + q0 * D128;
-        NAFP_TRY(lm_reserve(idx, nc, nprobe));
+        NAFP_TRY(lm_reserve(idx, nc, nprobe, S));
         if (nlist <= LM_PROBE_NLIST)
             lm_probe_smem_kernel<<<static_cast<unsigned>(std::min<int64_t>((nc + 7) / 8, ctx->sm_count)), 256, LM_PROBE_SMEM, ctx->stream>>>(
                 qp, nc, s->coarse, nlist, nprobe, L->dmax2, L->probes, L->gdist, L->qE);
@@ -849,7 +890,8 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
             L->probes, np, nprobe, nlist, hist);
         NAFP_CUDA(cudaMemcpyAsync(h.data(), hist, nb * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
         NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
-        // work items: (list, <= 128 of the query rows that probe it in this wave), longest lists first
+        // work items: (slice of a list, <= 128 of the query rows that probe it in this wave), longest first; slice s of a
+        // list of T tiles covers tiles [s T / S, (s + 1) T / S)
         items.clear();
         int n_items[LM_WAVES], first_item[LM_WAVES];
         int32_t run = 0;
@@ -859,8 +901,12 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
                 const int b = wv * nlist + l;
                 cur[b] = run;
                 const int tiles = (s->h_lend[l] - s->h_loff[l] + LM_ROWS - 1) / LM_ROWS;
-                if (tiles > 0)
-                    for (int o = 0; o < h[b]; o += LM_Q) items.push_back({l, run + o, std::min(LM_Q, h[b] - o), tiles});
+                for (int sl = 0; sl < S; ++sl) {
+                    const int t0 = static_cast<int>(static_cast<int64_t>(tiles) * sl / S);
+                    const int t1 = static_cast<int>(static_cast<int64_t>(tiles) * (sl + 1) / S);
+                    if (t1 > t0)
+                        for (int o = 0; o < h[b]; o += LM_Q) items.push_back({l, run + o, std::min(LM_Q, h[b] - o), t1 - t0, t0, sl});
+                }
                 run += h[b];
             }
             std::stable_sort(items.begin() + first, items.end(), [](const LmItem& a, const LmItem& b) { return a.tiles > b.tiles; });
@@ -879,14 +925,14 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
         NAFP_CUDA(cudaMemcpyAsync(cursor, cur.data(), nb * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
         NAFP_CUDA(cudaMemsetAsync(counters, 0, LM_WAVES * sizeof(int32_t), ctx->stream));
         lm_scatter_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, ctx->stream>>>(L->probes, np, nprobe, nlist, cursor, L->pairs);
-        NAFP_CUDA(cudaMemsetAsync(L->cand, 0, static_cast<size_t>(np) * LM_SLOT * sizeof(uint64_t), ctx->stream));
+        NAFP_CUDA(cudaMemsetAsync(L->cand, 0, static_cast<size_t>(np) * S * LM_SLOT * sizeof(uint64_t), ctx->stream));
         NAFP_CUDA(cudaMemsetAsync(L->dkA, 0x7f, static_cast<size_t>(nc) * sizeof(float), ctx->stream));     // 0x7f7f7f7f = 3.4e38: "no bound"
         ctx->launches += 3;
         for (int wv = 0; wv < LM_WAVES; ++wv) {
             if (n_items[wv] > 0) {
                 const int grid = std::min(n_items[wv], ctx->sm_count);
                 ivfpq_lm_scan_kernel<<<grid, LM_THREADS, LM_SMEM, ctx->stream>>>(
-                    qp, nprobe, L->items + first_item[wv], n_items[wv], counters + wv, L->pairs, L->tab, s->lcodes, L->lh, s->loff,
+                    qp, nprobe, S, L->items + first_item[wv], n_items[wv], counters + wv, L->pairs, L->tab, s->lcodes, L->lh, s->loff,
                     L->gdist, wv ? L->dkA : nullptr, L->qE, L->cand);
                 ctx->launches++;
                 for (int e = 0; e < n_items[wv]; ++e) L->tiles_run += items[first_item[wv] + e].tiles;
@@ -896,12 +942,12 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
             for (int x = wv + 1; x < LM_WAVES; ++x) later = later || n_items[x] > 0;
             if (later) {               // the bound the later waves' thresholds are built from
                 const int pend = std::min(wv == 0 ? 1 : LM_WAVE1_END, nprobe);
-                ivfpq_lm_bound_kernel<<<static_cast<unsigned>((nc + 7) / 8), 256, 0, ctx->stream>>>(
+                bound_kernel<<<static_cast<unsigned>((nc + 7) / 8), 256, lm_bound_smem(S), ctx->stream>>>(
                     qp, nc, nprobe, pend, k, L->cand, L->probes, L->gdist, L->qE, s->coarse, s->pq, s->lcodes, L->dkA);
                 ctx->launches++;
             }
         }
-        ivfpq_lm_merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(qp, q0, nprobe, k, L->cand, L->probes, L->gdist, L->qE, L->dkA,
+        merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(qp, q0, nprobe, k, L->cand, L->probes, L->gdist, L->qE, L->dkA,
                                                                                  s->coarse, s->pq, s->lcodes, s->lids, idx->label_offset,
                                                                                  D_dev + q0 * k, I_dev + q0 * k, s->redo_rows, redo_count);
         ctx->launches++;

@@ -9,7 +9,10 @@ locally.  Queries are replicated.  Per batch of test ids:
     ->  every rank scores the candidates it owns (-inf elsewhere)  ->  max all-reduce  ->  top-10
 
 The two collectives move k*12 bytes per query row per rank and 4 bytes per candidate score; they are
-the only exchange steps of the path.  The orchestration below is backend-agnostic (``ops`` does the
+the only exchange steps of the path.  An index with a second level (IVFPQR, ``ops.refine``) exchanges twice
+before the candidates are scored: the merged first-level top-kc (kc = 4k) is re-ranked by every rank over the
+labels it owns, and the per-rank top-k are all-gathered and merged again, which gives exactly the answer of one
+index over all rows.  The orchestration below is backend-agnostic (``ops`` does the
 local work, ``comm`` the collectives) so that the host logic is testable with gloo on CPU.
 """
 from __future__ import annotations
@@ -65,13 +68,19 @@ def sharded_seq_match(ops, comm, query, test_ids, seq_lens, k_probe):
     """Backend-agnostic orchestration; see the module docstring.  ``query`` is the whole query set
     (every rank holds it); returns (pred_ids, pred_scores)."""
     plan = ops.plan(query, test_ids)               # unique query rows + (test id, offset) -> row map
-    D_loc, I_loc = ops.local_topk(plan.qrows, k_probe)
+    D_loc, I_loc = ops.local_topk(plan.qrows, k_probe)        # (with ops.refine: the first level's top-kc)
     if comm is not None:
         D_all = comm.all_gather(D_loc)
         I_all = comm.all_gather(I_loc)
         _, I = ops.merge(D_all, I_all)
     else:
         I = I_loc
+    if hasattr(ops, "refine"):
+        D_loc, I_loc = ops.refine(plan.qrows, I, k_probe)
+        if comm is not None:
+            _, I = ops.merge(comm.all_gather(D_loc), comm.all_gather(I_loc))
+        else:
+            I = I_loc
     cand_ids, cand_scores, n_cand = ops.cand_scores(query, plan, test_ids, seq_lens, k_probe, I)
     if comm is not None:
         # a test id has at most k_probe x max_len distinct candidates (380 of the table's 1,024 columns at k_probe 20,
@@ -171,17 +180,41 @@ class GpuOps:
         return pid, psc
 
 
+class GpuRefineOps(GpuOps):
+    """``GpuOps`` of an IVFPQR shard: ``local_topk`` returns the first level's top 4k, ``refine`` re-ranks the merged
+    candidates this rank owns."""
+
+    K_FACTOR = 4                    # faiss IndexIVFPQR.k_factor
+
+    def local_topk(self, qrows, k):
+        n, kc = qrows.shape[0], k * self.K_FACTOR
+        D = self.torch.empty((n, kc), dtype=self.torch.float32, device=self.dev)
+        I = self.torch.empty((n, kc), dtype=self.torch.int64, device=self.dev)
+        self.check(self.lib.nafp_index_ivfpqr_first_level_dev(self.index.h, self._p(qrows), n, kc, self._p(D), self._p(I)))
+        return D, I
+
+    def refine(self, qrows, cand_I, k):
+        n, kc = cand_I.shape
+        cand_I = cand_I.contiguous()
+        D = self.torch.empty((n, k), dtype=self.torch.float32, device=self.dev)
+        I = self.torch.empty((n, k), dtype=self.torch.int64, device=self.dev)
+        self.check(self.lib.nafp_index_ivfpqr_rerank_dev(self.index.h, self._p(qrows), n, self._p(cand_I), kc, k,
+                                                         self._p(D), self._p(I)))
+        return D, I
+
+
 class ShardedFlatIndex:
     """Rank-local block (+ halo) of a row-sharded index and the collective sequence matcher.
 
-    ``index_type`` FLAT_L2 (default), IVFPQ or IVF_FLAT (``eval/utils/get_index.py``).  The IVF types shard their
-    codes / lists by the same row blocks with the quantizers replicated (SURVEY §8 e, the equivalent of
-    faiss.IndexShards over one trained index): ``train`` runs on rank 0 and the centroids / codebooks are
-    broadcast, after which every rank adds its own rows."""
+    ``index_type`` FLAT_L2 (default), IVFPQ, IVF_FLAT or IVFPQR (``eval/utils/get_index.py``).  The IVF types shard
+    their codes / lists by the same row blocks with the quantizers replicated (SURVEY §8 e, the equivalent of
+    faiss.IndexShards over one trained index): ``train`` runs on rank 0 and the centroids / codebooks (IVFPQR: also
+    the refinement codebooks) are broadcast, after which every rank adds its own rows.  IVFPQR re-ranks in a second
+    exchange (``GpuRefineOps``), so its answers equal one index's, unlike faiss.IndexShards over IVFPQR shards."""
 
     def __init__(self, n_rows_global, rank, world, max_len=19, device=None, comm=None, index_type=0, nlist=None,
                  pq_m=64, pq_nbits=8):
-        from .eval.utils.get_index import FLAT_L2, IVF_FLAT, IVFPQ, Index
+        from .eval.utils.get_index import FLAT_L2, IVF_FLAT, IVFPQ, IVFPQR, Index
         self.rank, self.world = int(rank), int(world)
         self.n_rows_global = int(n_rows_global)
         self.max_len = int(max_len)
@@ -191,8 +224,9 @@ class ShardedFlatIndex:
             nlist = 400 if self.index_type == IVF_FLAT else 256          # get_index_faiss.py:65,71
         self.index = Index(self.index_type, 128, nlist=nlist, pq_m=pq_m, pq_nbits=pq_nbits,
                            device=self.rank if device is None else device)
-        self._ivf = self.index_type in (IVFPQ, IVF_FLAT)
-        self._ivfpq = self.index_type == IVFPQ
+        self._ivf = self.index_type in (IVFPQ, IVF_FLAT, IVFPQR)
+        self._ivfpq = self.index_type in (IVFPQ, IVFPQR)
+        self._refine = self.index_type == IVFPQR
         if not self._ivf:
             self.index.reserve(self.hi_halo - self.lo)
         self.index.set_label_offset(self.lo)
@@ -212,6 +246,7 @@ class ShardedFlatIndex:
             dev = torch.device('cuda', self.index.ctx.device) if torch.cuda.is_available() else torch.device('cpu')
             coarse = torch.empty((self.index.nlist, 128), dtype=torch.float32, device=dev)
             pq = torch.empty((self.index.pq_m, 256, 128 // self.index.pq_m), dtype=torch.float32, device=dev) if self._ivfpq else None
+            rpq = torch.empty((4, 16, 32), dtype=torch.float32, device=dev) if self._refine else None
             if self.rank == 0:
                 if self._ivfpq:
                     c, p = self.index.ivfpq_params()
@@ -219,10 +254,16 @@ class ShardedFlatIndex:
                 else:
                     c = self.index.ivf_coarse()
                 coarse.copy_(torch.from_numpy(c))
+                if self._refine:
+                    rpq.copy_(torch.from_numpy(self.index.ivfpqr_refine()))
             self.comm.broadcast(coarse, 0)
             if self._ivfpq:
                 self.comm.broadcast(pq, 0)
+            if self._refine:
+                self.comm.broadcast(rpq, 0)
             if self.rank != 0:
+                if self._refine:
+                    self.index.set_ivfpqr_refine(rpq.cpu().numpy())
                 if self._ivfpq:
                     self.index.set_ivfpq_params(coarse.cpu().numpy(), pq.cpu().numpy())
                 else:
@@ -264,7 +305,8 @@ class ShardedFlatIndex:
 
     def ops(self, n_query_rows):
         if self._ops is None or self._ops.n_query_rows != n_query_rows:
-            self._ops = GpuOps(self.index, n_query_rows, self.n_rows_global, self.lo, self.hi, self.max_len)
+            cls = GpuRefineOps if self._refine else GpuOps
+            self._ops = cls(self.index, n_query_rows, self.n_rows_global, self.lo, self.hi, self.max_len)
         return self._ops
 
     def seq_match_dev(self, q_dev, test_ids_dev, seq_lens_dev, k_probe=20):

@@ -11,7 +11,8 @@ and ``--nogpu`` is refused (there is no CPU search path).
 
 Multi-GPU: started under ``torchrun`` (WORLD_SIZE > 1) the database is row-sharded over the ranks
 (``nafp_b200.dist.ShardedFlatIndex``: every rank reads only its block of the memmaps; per-rank top-k merged by an
-NCCL all-gather, candidate scores by a max all-reduce); rank 0 prints the table and writes the outputs.
+NCCL all-gather, candidate scores by a max all-reduce; 'ivfpq-rr' merges its first level and its re-ranked top-k in
+two such exchanges); rank 0 prints the table and writes the outputs.
 """
 from __future__ import annotations
 
@@ -66,11 +67,11 @@ def select_test_ids(test_ids, n_query, test_seq_len, rng=None):
 def _sharded_index(index_type, dummy_db, db, max_len, max_train, rank, world, device):
     """Row-sharded stand-in for ``get_index`` + the two ``index.add`` calls (``eval_faiss.py:141-151``)."""
     from ..dist import ShardedFlatIndex, TorchComm
-    from .utils.get_index import FLAT_L2, IVF_FLAT, IVFPQ
-    kinds = {'l2': FLAT_L2, 'ivfpq': IVFPQ, 'ivf': IVF_FLAT}
+    from .utils.get_index import FLAT_L2, IVF_FLAT, IVFPQ, IVFPQR
+    kinds = {'l2': FLAT_L2, 'ivfpq': IVFPQ, 'ivf': IVF_FLAT, 'ivfpq-rr': IVFPQR}
     mode = index_type.lower()
     if mode not in kinds:
-        raise NotImplementedError(f"index_type '{mode}' is not available row-sharded (l2, ivfpq, ivf are)")
+        raise NotImplementedError(f"index_type '{mode}' is not available row-sharded (l2, ivfpq, ivf, ivfpq-rr are)")
     comm = None
     if world > 1:
         import torch
@@ -203,7 +204,8 @@ def run_eval(emb_dir, emb_dummy_dir=None, index_type='ivfpq', nogpu=False, max_t
 @click.option('--emb_dummy_dir', default=None, type=click.STRING,
               help="Specify a directory containing 'dummy_db.mm' and 'dummy_db_shape.npy' to use. Default is EMB_DIR.")
 @click.option('--index_type', '-i', default='ivfpq', type=click.STRING,
-              help="Index type must be one of {'L2', 'IVF', 'IVFPQ', 'IVFPQ-RR'} ('IVFPQ-ONDISK' and 'HNSW' are CPU-only in the reference).")
+              help="Index type must be one of {'L2', 'IVF', 'IVFPQ', 'IVFPQ-RR'}; all four row-shard under torchrun "
+                   "('IVFPQ-ONDISK' and 'HNSW' are CPU-only in the reference).")
 @click.option('--nogpu', default=False, is_flag=True, help='Refused: this build has no CPU search path.')
 @click.option('--max_train', default=1e7, type=click.INT, help='Max number of items for index training. Default is 1e7.')
 @click.option('--test_seq_len', default='1 3 5 9 11 19', type=click.STRING,
