@@ -92,6 +92,21 @@ int nafp_weights_load(nafp_ctx* ctx, const float* const* conv_w, const float* co
                       const float* const* ln_g, const float* const* ln_b, const float* div_w1,
                       const float* div_b1, const float* div_w2, const float* div_b2);
 
+/* MODEL.BN of the weights (model/fp/nnfp.py:20-83: ConvLayer(norm=...)), TF 2.4 Keras semantics, eps 1e-3:
+ *   NAFP_NORM_LAYER_NORM2D  LayerNormalization(axis=(1,2,3)): gamma / beta (F,T,C)      = nafp_weights_load
+ *   NAFP_NORM_LAYER_NORM1D  LayerNormalization(axis=-1): over the C channels of each position, gamma / beta (C)
+ *   NAFP_NORM_BATCH_NORM    BatchNormalization(axis=-1) in inference mode (test_step sets trainable = False):
+ *                           gamma, beta, moving mean, moving variance (C) */
+enum { NAFP_NORM_LAYER_NORM2D = 0, NAFP_NORM_LAYER_NORM1D = 1, NAFP_NORM_BATCH_NORM = 2 };
+
+/* nafp_weights_load for any MODEL.BN: norm_g[l] / norm_b[l] hold F*T*C floats for NAFP_NORM_LAYER_NORM2D and C floats
+ * otherwise; norm_mean / norm_var (C floats per layer) are given for NAFP_NORM_BATCH_NORM and NULL otherwise.  The
+ * norm belongs to the loaded weights: the next load replaces it.  A failed load leaves no usable weights. */
+int nafp_weights_load_norm(nafp_ctx* ctx, int32_t norm, const float* const* conv_w, const float* const* conv_b,
+                           const float* const* norm_g, const float* const* norm_b, const float* const* norm_mean,
+                           const float* const* norm_var, const float* div_w1, const float* div_b1,
+                           const float* div_w2, const float* div_b2);
+
 /* Log-mel front end.  x_dev: (n_seg, 8000) float32 segments (the (B,1,8000) batches of
  * model/generate.py:178 flattened).  Rows are processed in consecutive groups of `group_size`
  * (= BSZ.TS_BATCH_SZ; the last group may be partial), each group sharing the batch-global max
@@ -133,7 +148,7 @@ int nafp_fingerprint_pcm16_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t 
 int nafp_fingerprint_pcm16_tracks_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t n_samples,
                                        const int64_t* seg_off_host, const int32_t* seg_valid_host,
                                        int64_t n_seg, int64_t group_size, float* emb_host);
-/* Debug/parity taps: post-LayerNorm activation of conv `layer` (0..15) for the LAST
+/* Debug/parity taps: activation of conv `layer` (0..15) after its normalisation (any MODEL.BN) for the LAST
  * nafp_encoder_forward call, as float32 (n_seg, F, T, C) into out_host. */
 int nafp_encoder_activation_host(nafp_ctx* ctx, int layer, int64_t n_seg, float* out_host);
 

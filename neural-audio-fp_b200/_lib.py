@@ -55,6 +55,8 @@ _SIGS = {
     "nafp_synth_fp_rows": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int32, c_float, c_void_p]),
     "nafp_synth_audio": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p]),
     "nafp_weights_load": (c_int, [c_void_p, POINTER(_fp), POINTER(_fp), POINTER(_fp), POINTER(_fp), _fp, _fp, _fp, _fp]),
+    "nafp_weights_load_norm": (c_int, [c_void_p, c_int32, POINTER(_fp), POINTER(_fp), POINTER(_fp), POINTER(_fp), POINTER(_fp),
+                                       POINTER(_fp), _fp, _fp, _fp, _fp]),
     "nafp_logmel_forward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "nafp_logmel_forward_raw": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "nafp_logmel_set_segment_norm": (c_int, [c_void_p, c_int32]),

@@ -24,11 +24,14 @@
 //                      6-stage smem ring, fp32 accumulators double-buffered in TMEM, 16 epilogue warps;
 //                      layers with K <= 384 keep their weights resident in shared memory.
 //   fold_kernel        (weights load) Cg / Cb of every layer in fp64
+//   ln1d_kernel        MODEL.BN 'layer_norm1d': per-position LayerNorm over C, in place (L1a: fused into conv0_kernel)
+//   (MODEL.BN 'batch_norm' is the fold with constant factors, all layers split precision: nafp_weights_load_norm)
 //   divenc_kernel      last LayerNorm + divide-and-encode head (128 x [8->32 ELU, 32->1]); l2norm_kernel.
 // fp16 operands / fp32 accumulation; the six small layers from L6a on run split precision (hi + lo operands).
 // Measured against the fp64 oracle the fingerprints agree to a few 1e-4 (gate: cosine >= 0.9999, max abs <= 1e-3).
 #include <cuda_fp16.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -114,6 +117,10 @@ struct EncoderState {
                                                // (measured: 7.5 vs 6.9 ms per 4,000 segments -- the UTMAPF requests compete
                                                // with the loads for the same TMA / L2 request slots; kept as a switch)
     int64_t last_n = 0;                        // segments of the last pass (activation probe)
+    int norm = NAFP_NORM_LAYER_NORM2D;         // MODEL.BN of the loaded weights (nafp_weights_load_norm)
+    int split_from = 0;                        // first split-precision layer of g (split_point(norm))
+    float* ln_c = nullptr;                     // [16][gamma 1024 | beta 1024] per-channel LayerNorm of 'layer_norm1d'
+    float2* unit = nullptr;                    // [cap] (1, 0): the stat buffer of layers whose output is stored normalised
 };
 constexpr int PART_SLOTS = 256;                // most partial-sum slots per segment of any layer (L1b: 64 groups x <= 4 parts)
 
@@ -127,7 +134,9 @@ static void same_pad(int n_in, int k, int s, int* n_out, int* lo) {
     *lo = total / 2;
 }
 
-static void build_geometry(ConvGeom* g) {
+// split_from: first layer whose operands are split (hi + lo); the default, ENC_SPLIT_FROM, or what the norm needs
+// (split_point)
+static void build_geometry(ConvGeom* g, int split_from) {
     int f = 256, t = 32, c = 1;
     for (int i = 0; i < 8; ++i) {
         for (int half = 0; half < 2; ++half) {
@@ -163,8 +172,6 @@ static void build_geometry(ConvGeom* g) {
     if (const char* e = getenv("NAFP_ENC_NT256")) nt256 = static_cast<unsigned>(strtoul(e, nullptr, 0));
     for (int l = 1; l < 16; ++l)
         if (((nt256 >> l) & 1u) && g[l].c_out >= 256 && g[l].ms < 128) g[l].nt = 256;
-    int split_from = ENC_SPLIT_FROM;           // NAFP_ENC_SPLIT_FROM: A/B of the error / speed trade (16 = no split layer)
-    if (const char* e = getenv("NAFP_ENC_SPLIT_FROM")) split_from = atoi(e);
     for (int l = 0; l < 16; ++l) g[l].ksplit = l >= split_from ? 3 : 1;
     for (int l = 0; l < 16; ++l) g[l].osplit = l + 1 < 16 ? g[l + 1].ksplit : 3;     // the head reads hi + lo too
 }
@@ -226,15 +233,25 @@ __device__ __forceinline__ void conv0_row(float v, const Conv0Lane& L, int tp, u
 // the first segment.  One slot of partial sums per (segment, block, warp): CONV0_SLOTS per segment.
 constexpr int CONV0_ROWS = 16, CONV0_SEGS = 16;
 constexpr int CONV0_SLOTS = (256 / CONV0_ROWS) * 8;
+// LN1D ('layer_norm1d'): every output position is normalised over its 128 channels before the store -- a lane holds
+// 4 channels of the position, so its statistics are a warp reduction (two passes, fp32, fixed order); ln_c holds
+// gamma [0, 128) and beta [1024, 1152) of the layer, and no partial sums are written.
+// SPLIT: the output is stored [hi | hi | lo] per position (L1b runs split precision: 'batch_norm', see build_geometry).
+template <bool LN1D, bool SPLIT = false>
 __global__ void __launch_bounds__(256)
 conv0_kernel(const float* __restrict__ mel, const int32_t* __restrict__ gmax, int64_t group_size, int n_seg,
              const float* __restrict__ w0, const float* __restrict__ b0, const float* __restrict__ gamma,
-             __half* __restrict__ x, float* __restrict__ part) {
+             __half* __restrict__ x, float* __restrict__ part, const float* __restrict__ ln_c) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int seg0 = blockIdx.y * CONV0_SEGS;
     constexpr int PER_SEG = 256 * 16 * 128;
     Conv0Lane L;
     conv0_load_lane(w0, b0, lane, L);
+    float4 lg, lb;
+    if constexpr (LN1D) {
+        lg = reinterpret_cast<const float4*>(ln_c)[lane];
+        lb = reinterpret_cast<const float4*>(ln_c + 1024)[lane];
+    }
     const bool raw = gmax != nullptr;
 #pragma unroll 1
     for (int k = 0; k < CONV0_SEGS; ++k) {
@@ -253,19 +270,51 @@ conv0_kernel(const float* __restrict__ mel, const int32_t* __restrict__ gmax, in
             for (int tp = 0; tp < 16; ++tp) {
                 uint64_t o[2];
                 conv0_row(v, L, tp, o);
-                const ulonglong2 g = __ldg(g_row + tp * 32);
-                s1 = add2(s1, add2(o[0], o[1]));
-                s2 = fma2(o[0], o[0], fma2(o[1], o[1], s2));
                 float z0, z1, z2, z3;
-                upk2(mul2(o[0], g.x), z0, z1);
-                upk2(mul2(o[1], g.y), z2, z3);
+                if constexpr (LN1D) {
+                    float y0, y1, y2, y3;
+                    upk2(o[0], y0, y1);
+                    upk2(o[1], y2, y3);
+                    float m = (y0 + y1) + (y2 + y3);
+#pragma unroll
+                    for (int off = 16; off > 0; off >>= 1) m += __shfl_xor_sync(0xffffffffu, m, off);
+                    m *= 1.f / 128.f;
+                    y0 -= m; y1 -= m; y2 -= m; y3 -= m;
+                    float q = (y0 * y0 + y1 * y1) + (y2 * y2 + y3 * y3);
+#pragma unroll
+                    for (int off = 16; off > 0; off >>= 1) q += __shfl_xor_sync(0xffffffffu, q, off);
+                    const float rstd = rsqrtf(q * (1.f / 128.f) + LN_EPS);
+                    z0 = fmaf(lg.x, y0 * rstd, lb.x);
+                    z1 = fmaf(lg.y, y1 * rstd, lb.y);
+                    z2 = fmaf(lg.z, y2 * rstd, lb.z);
+                    z3 = fmaf(lg.w, y3 * rstd, lb.w);
+                } else {
+                    const ulonglong2 g = __ldg(g_row + tp * 32);
+                    s1 = add2(s1, add2(o[0], o[1]));
+                    s2 = fma2(o[0], o[0], fma2(o[1], o[1], s2));
+                    upk2(mul2(o[0], g.x), z0, z1);
+                    upk2(mul2(o[1], g.y), z2, z3);
+                }
                 __half2 h0 = __floats2half2_rn(z0, z1), h1 = __floats2half2_rn(z2, z3);
                 uint2 pk;
                 pk.x = *reinterpret_cast<uint32_t*>(&h0);
                 pk.y = *reinterpret_cast<uint32_t*>(&h1);
-                orow[tp * 32] = pk;
+                if constexpr (SPLIT) {
+                    const float2 b0 = __half22float2(h0), b1 = __half22float2(h1);
+                    __half2 l0 = __floats2half2_rn(z0 - b0.x, z1 - b0.y), l1 = __floats2half2_rn(z2 - b1.x, z3 - b1.y);
+                    uint2 lo;
+                    lo.x = *reinterpret_cast<uint32_t*>(&l0);
+                    lo.y = *reinterpret_cast<uint32_t*>(&l1);
+                    uint2* srow = reinterpret_cast<uint2*>(x + (static_cast<int64_t>(seg) * PER_SEG + static_cast<int64_t>(f) * (16 * 128)) * 3) + lane;
+                    srow[tp * 96] = pk;                 // 384 halves per position: hi (32 uint2), hi, lo
+                    srow[tp * 96 + 32] = pk;
+                    srow[tp * 96 + 64] = lo;
+                } else {
+                    orow[tp * 32] = pk;
+                }
             }
         }
+        if constexpr (LN1D) continue;
         float a1, b1, a2, b2;
         upk2(s1, a1, b1);
         upk2(s2, a2, b2);
@@ -305,6 +354,88 @@ ln_stats_kernel(const float* __restrict__ part, int slots, int per_seg, int n_se
         const float var = fmaxf(static_cast<float>(b) * inv_n - mean * mean, 0.f);
         const float rstd = rsqrtf(var + LN_EPS);
         stat[seg] = make_float2(rstd, -rstd * mean);
+    }
+}
+
+// 'layer_norm1d' after conv layers 1 .. 14: one warp per output position normalises its C = 32 PER channels in
+// place, gamma (.) (y - mean) rstd + beta, in the stored format (fp16, or [hi | hi | lo] re-split).  Two passes in
+// fp32 over the lane's registers, then a fixed shuffle tree: bit-reproducible, independent of the pass size.
+template <int PER>
+__global__ void __launch_bounds__(256)
+ln1d_kernel(__half* __restrict__ x, int64_t n_pos, int split, const float* __restrict__ gamma, const float* __restrict__ beta) {
+    constexpr int C = PER * 32;
+    constexpr int VEC = PER < 8 ? PER : 8;            // halves per load: 8 or 16 bytes, consecutive lanes adjacent
+    constexpr int NV = PER / VEC;
+    const int lane = threadIdx.x & 31;
+    const int64_t pos = static_cast<int64_t>(blockIdx.x) * 8 + (threadIdx.x >> 5);
+    if (pos >= n_pos) return;
+    __half* row = x + pos * C * (split ? 3 : 1);
+    float v[PER];
+#pragma unroll
+    for (int j = 0; j < NV; ++j) {
+        const int c0 = (j * 32 + lane) * VEC;
+        __half2 h[VEC / 2], l[VEC / 2];
+        if constexpr (VEC == 8) *reinterpret_cast<uint4*>(h) = *reinterpret_cast<const uint4*>(row + c0);
+        else                    *reinterpret_cast<uint2*>(h) = *reinterpret_cast<const uint2*>(row + c0);
+        if (split) {
+            if constexpr (VEC == 8) *reinterpret_cast<uint4*>(l) = *reinterpret_cast<const uint4*>(row + 2 * C + c0);
+            else                    *reinterpret_cast<uint2*>(l) = *reinterpret_cast<const uint2*>(row + 2 * C + c0);
+        }
+#pragma unroll
+        for (int k = 0; k < VEC / 2; ++k) {
+            float2 f = __half22float2(h[k]);
+            if (split) {
+                const float2 g = __half22float2(l[k]);
+                f.x += g.x;
+                f.y += g.y;
+            }
+            v[j * VEC + 2 * k] = f.x;
+            v[j * VEC + 2 * k + 1] = f.y;
+        }
+    }
+    float m = 0.f;
+#pragma unroll
+    for (int i = 0; i < PER; ++i) m += v[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m += __shfl_xor_sync(0xffffffffu, m, o);
+    m *= 1.f / C;
+    float q = 0.f;
+#pragma unroll
+    for (int i = 0; i < PER; ++i) {
+        v[i] -= m;
+        q = fmaf(v[i], v[i], q);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
+    const float rstd = rsqrtf(q * (1.f / C) + LN_EPS);
+#pragma unroll
+    for (int j = 0; j < NV; ++j) {
+        const int c0 = (j * 32 + lane) * VEC;
+        __half2 h[VEC / 2], l[VEC / 2];
+#pragma unroll
+        for (int k = 0; k < VEC / 2; ++k) {
+            const int c = c0 + 2 * k;
+            const float z0 = fmaf(__ldg(gamma + c), v[j * VEC + 2 * k] * rstd, __ldg(beta + c));
+            const float z1 = fmaf(__ldg(gamma + c + 1), v[j * VEC + 2 * k + 1] * rstd, __ldg(beta + c + 1));
+            h[k] = __floats2half2_rn(z0, z1);
+            if (split) {
+                const float2 back = __half22float2(h[k]);
+                l[k] = __floats2half2_rn(z0 - back.x, z1 - back.y);
+            }
+        }
+        if constexpr (VEC == 8) {
+            *reinterpret_cast<uint4*>(row + c0) = *reinterpret_cast<const uint4*>(h);
+            if (split) {
+                *reinterpret_cast<uint4*>(row + C + c0) = *reinterpret_cast<const uint4*>(h);
+                *reinterpret_cast<uint4*>(row + 2 * C + c0) = *reinterpret_cast<const uint4*>(l);
+            }
+        } else {
+            *reinterpret_cast<uint2*>(row + c0) = *reinterpret_cast<const uint2*>(h);
+            if (split) {
+                *reinterpret_cast<uint2*>(row + C + c0) = *reinterpret_cast<const uint2*>(h);
+                *reinterpret_cast<uint2*>(row + 2 * C + c0) = *reinterpret_cast<const uint2*>(l);
+            }
+        }
     }
 }
 
@@ -793,31 +924,26 @@ l2norm_kernel(const float* __restrict__ raw, int n_seg, float* __restrict__ emb)
 // ------------------------------------------------------------------------------------------
 // host
 // ------------------------------------------------------------------------------------------
-static int encoder_init(nafp_ctx* ctx) {
-    if (ctx->encoder) return NAFP_OK;
-    EncoderState* s = new EncoderState();
-    ctx->encoder = s;              // before the first fallible call: nafp_ctx_destroy releases it
-    build_geometry(s->g);
-    if (const char* e = getenv("NAFP_ENC_L2PF")) s->l2_prefetch = atoi(e) != 0;
-    if (const char* e = getenv("NAFP_ENC_TMASTORE")) s->tma_store = atoi(e) != 0;
-    NAFP_CUDA(cudaMalloc(&s->w0, 3 * 128 * sizeof(float)));
-    NAFP_CUDA(cudaMalloc(&s->bias0, 128 * sizeof(float)));
-    NAFP_CUDA(cudaMalloc(&s->ln_b15, 1024 * sizeof(float)));
-    for (int l = 0; l < ENC_LAYERS; ++l) {
-        const ConvGeom& L = s->g[l];
-        const size_t per = static_cast<size_t>(L.ms) * L.c_out;
-        NAFP_CUDA(cudaMalloc(&s->ln_g[l], per * sizeof(float)));
-        if (l == 0) continue;
-        NAFP_CUDA(cudaMalloc(&s->cbeta[l], per * sizeof(float)));
-        NAFP_CUDA(cudaMalloc(&s->cgam[l], per * sizeof(__half)));
-        NAFP_CUDA(cudaMalloc(&s->wt[l], static_cast<size_t>(L.c_out) * 3 * L.c_in * L.ksplit * sizeof(__half)));
-    }
-    NAFP_CUDA(cudaMalloc(&s->dw1, 128 * 8 * 32 * sizeof(float)));
-    NAFP_CUDA(cudaMalloc(&s->db1, 128 * 32 * sizeof(float)));
-    NAFP_CUDA(cudaMalloc(&s->dw2, 128 * 32 * sizeof(float)));
-    NAFP_CUDA(cudaMalloc(&s->db2, 128 * sizeof(float)));
+// First split-precision layer for a MODEL.BN.  'batch_norm' needs every layer split: its per-channel scale
+// gamma / sqrt(var + eps) reaches ~30 on channels ELU saturates (variance near 0), and any fp16 rounding of an
+// activation before that scale -- even L1a's output, or the normalised value -- carries the fingerprints past 1e-3
+// (measured on B200 with the default split point: max-abs 1.6-4.6e-3; an fp16-storage model of the network on the
+// host gives 0.9-3e-3 for every split point from L1b's output on and rounding-level error with L1a's output split).
+static int split_point(int norm) {
+    if (norm == NAFP_NORM_BATCH_NORM) return 1;
+    int split_from = ENC_SPLIT_FROM;           // NAFP_ENC_SPLIT_FROM: A/B of the error / speed trade (16 = no split layer)
+    if (const char* e = getenv("NAFP_ENC_SPLIT_FROM")) split_from = atoi(e);
+    if (split_from < 2) split_from = 2;        // conv0_kernel writes split output only without the fused layer_norm1d
+    return split_from;
+}
+
+// the weight operands and their tensor maps: sized by the split point of the geometry
+static int encoder_weight_buffers(EncoderState* s) {
     for (int l = 1; l < ENC_LAYERS; ++l) {
         const ConvGeom& L = s->g[l];
+        if (s->wt[l]) cudaFree(s->wt[l]);
+        s->wt[l] = nullptr;
+        NAFP_CUDA(cudaMalloc(&s->wt[l], static_cast<size_t>(L.c_out) * 3 * L.c_in * L.ksplit * sizeof(__half)));
         const uint64_t C = static_cast<uint64_t>(L.c_in) * L.ksplit;
         const uint64_t wd[2] = {3 * C, static_cast<uint64_t>(L.c_out)};
         const uint64_t ws[2] = {2, 3 * C * 2};
@@ -825,6 +951,34 @@ static int encoder_init(nafp_ctx* ctx) {
         NAFP_TRY(make_tensor_map(&s->tmB[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, s->wt[l], wd, ws, wb, nullptr,
                                  CU_TENSOR_MAP_SWIZZLE_128B));
     }
+    return NAFP_OK;
+}
+
+static int encoder_init(nafp_ctx* ctx) {
+    if (ctx->encoder) return NAFP_OK;
+    EncoderState* s = new EncoderState();
+    ctx->encoder = s;              // before the first fallible call: nafp_ctx_destroy releases it
+    s->split_from = split_point(NAFP_NORM_LAYER_NORM2D);
+    build_geometry(s->g, s->split_from);
+    if (const char* e = getenv("NAFP_ENC_L2PF")) s->l2_prefetch = atoi(e) != 0;
+    if (const char* e = getenv("NAFP_ENC_TMASTORE")) s->tma_store = atoi(e) != 0;
+    NAFP_CUDA(cudaMalloc(&s->w0, 3 * 128 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->bias0, 128 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->ln_b15, 1024 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->ln_c, ENC_LAYERS * 2048 * sizeof(float)));
+    for (int l = 0; l < ENC_LAYERS; ++l) {
+        const ConvGeom& L = s->g[l];
+        const size_t per = static_cast<size_t>(L.ms) * L.c_out;
+        NAFP_CUDA(cudaMalloc(&s->ln_g[l], per * sizeof(float)));
+        if (l == 0) continue;
+        NAFP_CUDA(cudaMalloc(&s->cbeta[l], per * sizeof(float)));
+        NAFP_CUDA(cudaMalloc(&s->cgam[l], per * sizeof(__half)));
+    }
+    NAFP_CUDA(cudaMalloc(&s->dw1, 128 * 8 * 32 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->db1, 128 * 32 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->dw2, 128 * 32 * sizeof(float)));
+    NAFP_CUDA(cudaMalloc(&s->db2, 128 * sizeof(float)));
+    NAFP_TRY(encoder_weight_buffers(s));
     NAFP_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, CONV_SMEM));
     NAFP_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, CONV_SMEM));
     NAFP_CUDA(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
@@ -840,7 +994,7 @@ static void encoder_release_arena(EncoderState* s) {
         if (s->x[l]) cudaFree(s->x[l]);
         s->x[l] = nullptr;
     }
-    void** bufs[] = {reinterpret_cast<void**>(&s->stat), reinterpret_cast<void**>(&s->part),
+    void** bufs[] = {reinterpret_cast<void**>(&s->stat), reinterpret_cast<void**>(&s->unit), reinterpret_cast<void**>(&s->part),
                      reinterpret_cast<void**>(&s->raw), reinterpret_cast<void**>(&s->mel), &s->xin[0], &s->xin[1],
                      reinterpret_cast<void**>(&s->emb)};
     for (void** b : bufs) {
@@ -871,6 +1025,11 @@ static int encoder_reserve(nafp_ctx* ctx, int64_t n) {
         NAFP_CUDA(cudaMemset(s->x[l], 0, x_elems * sizeof(__half)));
     }
     NAFP_CUDA(cudaMalloc(&s->stat, static_cast<size_t>(ENC_LAYERS) * cap * sizeof(float2)));
+    {
+        const std::vector<float2> unit(static_cast<size_t>(cap), make_float2(1.f, 0.f));
+        NAFP_CUDA(cudaMalloc(&s->unit, unit.size() * sizeof(float2)));
+        NAFP_CUDA(cudaMemcpy(s->unit, unit.data(), unit.size() * sizeof(float2), cudaMemcpyHostToDevice));
+    }
     NAFP_CUDA(cudaMalloc(&s->part, static_cast<size_t>(cap) * PART_SLOTS * 2 * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&s->mel, static_cast<size_t>(cap) * 8192 * sizeof(float)));
     for (int b = 0; b < 2; ++b) NAFP_CUDA(cudaMalloc(&s->xin[b], static_cast<size_t>(cap) * 8000 * sizeof(float)));
@@ -920,7 +1079,7 @@ void encoder_destroy(nafp_ctx* ctx) {
         void* bufs[] = {s->ln_g[l], s->cbeta[l], s->cgam[l], s->wt[l]};
         for (void* b : bufs) if (b) cudaFree(b);
     }
-    void* bufs[] = {s->w0, s->bias0, s->ln_b15, s->dw1, s->db1, s->dw2, s->db2};
+    void* bufs[] = {s->w0, s->bias0, s->ln_b15, s->ln_c, s->dw1, s->db1, s->dw2, s->db2};
     for (void* b : bufs) if (b) cudaFree(b);
     for (int b = 0; b < 2; ++b) {
         if (s->ev_up[b]) cudaEventDestroy(s->ev_up[b]);
@@ -931,18 +1090,31 @@ void encoder_destroy(nafp_ctx* ctx) {
     ctx->encoder = nullptr;
 }
 
+// (a, c) of layer l's stored activation: per-segment LayerNorm statistics, or (1, 0) where the stored values need no
+// per-segment factor -- layers 0 .. 14 of 'layer_norm1d' (stored normalised by conv0 / ln1d_kernel; the last layer's
+// output is one position, where the per-channel LayerNorm is the per-segment one) and every layer of 'batch_norm'
+// (its affine map is in the planes)
+static bool layer_has_stats(const EncoderState* s, int l) {
+    return s->norm == NAFP_NORM_LAYER_NORM2D || (s->norm == NAFP_NORM_LAYER_NORM1D && l == ENC_LAYERS - 1);
+}
+static float2* layer_stat(const EncoderState* s, int l) {
+    return layer_has_stats(s, l) ? s->stat + static_cast<size_t>(l) * s->cap : s->unit;
+}
+
 // one pass over n <= cap segments (encoder_reserve); mel is either final (gmax == nullptr) or raw log-mel + group maxima
 static int encoder_pass(nafp_ctx* ctx, const float* mel, const int32_t* gmax, int64_t group_size, int n, float* emb_dev) {
     EncoderState* s = ctx->encoder;
     cudaStream_t st = ctx->stream;
+    const bool ln1d = s->norm == NAFP_NORM_LAYER_NORM1D;
     for (int l = 0; l < ENC_LAYERS; ++l) {
         const ConvGeom& L = s->g[l];
         float2* stat = s->stat + static_cast<size_t>(l) * s->cap;
         const int per = L.ms * L.c_out;
         int slots;
         if (l == 0) {
-            conv0_kernel<<<dim3(256 / CONV0_ROWS, (n + CONV0_SEGS - 1) / CONV0_SEGS), 256, 0, st>>>(
-                mel, gmax, group_size, n, s->w0, s->bias0, s->ln_g[0], s->x[0], s->part);
+            auto kern = ln1d ? conv0_kernel<true> : L.osplit != 1 ? conv0_kernel<false, true> : conv0_kernel<false>;
+            kern<<<dim3(256 / CONV0_ROWS, (n + CONV0_SEGS - 1) / CONV0_SEGS), 256, 0, st>>>(
+                mel, gmax, group_size, n, s->w0, s->bias0, s->ln_g[0], s->x[0], s->part, ln1d ? s->ln_c : nullptr);
             slots = CONV0_SLOTS;
         } else {
             ConvParams p;
@@ -962,13 +1134,26 @@ static int encoder_pass(nafp_ctx* ctx, const float* mel, const int32_t* gmax, in
             slots = p.groups * p.n_ntiles * CONV_EPI_PARTS;
             auto kern = L.nt == 128 ? conv_gemm_kernel<128> : conv_gemm_kernel<256>;
             kern<<<p.combos * p.n_streams, CONV_THREADS, CONV_SMEM, st>>>(
-                s->tmA[l], s->tmB[l], s->tmO[l], p, s->stat + static_cast<size_t>(l - 1) * s->cap, s->ln_g[l], s->cbeta[l], s->cgam[l],
+                s->tmA[l], s->tmB[l], s->tmO[l], p, layer_stat(s, l - 1), s->ln_g[l], s->cbeta[l], s->cgam[l],
                 s->x[l], s->part);
+            if (ln1d && l < ENC_LAYERS - 1) {
+                const int64_t n_pos = static_cast<int64_t>(n) * L.ms;
+                const unsigned blocks = static_cast<unsigned>((n_pos + 7) / 8);
+                const float* g1 = s->ln_c + static_cast<size_t>(l) * 2048;
+                const int sp = L.osplit != 1;
+                auto kern1 = L.c_out == 128 ? ln1d_kernel<4> : L.c_out == 256 ? ln1d_kernel<8>
+                           : L.c_out == 512 ? ln1d_kernel<16> : ln1d_kernel<32>;
+                kern1<<<blocks, 256, 0, st>>>(s->x[l], n_pos, sp, g1, g1 + 1024);
+                ctx->launches += 1;
+            }
         }
-        ln_stats_kernel<<<(n + 7) / 8, 256, 0, st>>>(s->part, slots, per, n, stat);
-        ctx->launches += 2;
+        ctx->launches += 1;
+        if (layer_has_stats(s, l)) {
+            ln_stats_kernel<<<(n + 7) / 8, 256, 0, st>>>(s->part, slots, per, n, stat);
+            ctx->launches += 1;
+        }
     }
-    divenc_kernel<<<dim3(EMB, (n + 127) / 128), 128, 0, st>>>(s->x[ENC_LAYERS - 1], s->stat + static_cast<size_t>(ENC_LAYERS - 1) * s->cap,
+    divenc_kernel<<<dim3(EMB, (n + 127) / 128), 128, 0, st>>>(s->x[ENC_LAYERS - 1], layer_stat(s, ENC_LAYERS - 1),
                                                               s->ln_g[ENC_LAYERS - 1], s->ln_b15, n, s->dw1, s->db1, s->dw2,
                                                               s->db2, s->raw);
     l2norm_kernel<<<(n * 32 + 255) / 256, 256, 0, st>>>(s->raw, n, emb_dev);
@@ -1011,13 +1196,90 @@ extern "C" {
 int nafp_weights_load(nafp_ctx* ctx, const float* const* conv_w, const float* const* conv_b, const float* const* ln_g,
                       const float* const* ln_b, const float* div_w1, const float* div_b1, const float* div_w2,
                       const float* div_b2) {
+    return nafp_weights_load_norm(ctx, NAFP_NORM_LAYER_NORM2D, conv_w, conv_b, ln_g, ln_b, nullptr, nullptr, div_w1, div_b1,
+                                  div_w2, div_b2);
+}
+
+// The other MODEL.BN values run through the same GEMM kernels with other per-element planes and per-segment factors:
+//   'layer_norm1d': layers 0 .. 14 store their output normalised (conv0_kernel<true> / ln1d_kernel, per-channel
+//                gamma / beta in ln_c), so their planes are 1 / 0 and their consumers read (a, c) = (1, 0); the last
+//                layer's output is one position, where the per-channel LayerNorm is the per-segment one with (1, 1, C)
+//                parameters: the layer_norm2d path;
+//   'batch_norm' (inference): y -> s y + t per channel, s = gamma / sqrt(var + eps), t = beta - mean s (fp64 here),
+//                is the fold with (a, c) = (1, 0) and the planes s / t broadcast over (F,T): the layers store
+//                z = s (.) y, fold_kernel gives Cb = bias + conv(t), the head adds t.  No statistics, no extra pass;
+//                every layer runs split precision (split_point), so z keeps what t cancels later.
+// The split point belongs to the norm: a load that changes it rebuilds the geometry, the weight operands and the
+// activation arena.  Every pointer is checked before the first device write.
+int nafp_weights_load_norm(nafp_ctx* ctx, int32_t norm, const float* const* conv_w, const float* const* conv_b,
+                           const float* const* norm_g, const float* const* norm_b, const float* const* norm_mean,
+                           const float* const* norm_var, const float* div_w1, const float* div_b1, const float* div_w2,
+                           const float* div_b2) {
     NAFP_RANGE("nafp_weights_load");
-    NAFP_REQUIRE(ctx && conv_w && conv_b && ln_g && ln_b && div_w1 && div_b1 && div_w2 && div_b2, NAFP_ERR_INVALID,
+    NAFP_REQUIRE(ctx && conv_w && conv_b && norm_g && norm_b && div_w1 && div_b1 && div_w2 && div_b2, NAFP_ERR_INVALID,
                  "nafp_weights_load: NULL argument");
+    NAFP_REQUIRE(norm == NAFP_NORM_LAYER_NORM2D || norm == NAFP_NORM_LAYER_NORM1D || norm == NAFP_NORM_BATCH_NORM,
+                 NAFP_ERR_INVALID, "nafp_weights_load_norm: norm %d (0 layer_norm2d, 1 layer_norm1d, 2 batch_norm)", (int)norm);
+    const bool bn = norm == NAFP_NORM_BATCH_NORM;
+    NAFP_REQUIRE(bn ? (norm_mean && norm_var) : (!norm_mean && !norm_var), NAFP_ERR_INVALID,
+                 "nafp_weights_load_norm: norm_mean / norm_var are given exactly for batch_norm");
+    for (int l = 0; l < ENC_LAYERS; ++l)
+        NAFP_REQUIRE(conv_w[l] && conv_b[l] && norm_g[l] && norm_b[l] && (!bn || (norm_mean[l] && norm_var[l])),
+                     NAFP_ERR_INVALID, "nafp_weights_load: layer %d NULL", l);
     NAFP_CUDA(cudaSetDevice(ctx->device));
     NAFP_TRY(encoder_init(ctx));
     EncoderState* s = ctx->encoder;
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
+    s->weights = false;                // until this load completes
+    const int split_from = split_point(norm);
+    if (split_from != s->split_from) {
+        encoder_release_arena(s);      // activation sizes and maps follow the split point (encoder_reserve)
+        build_geometry(s->g, split_from);
+        s->split_from = split_from;
+        NAFP_TRY(encoder_weight_buffers(s));
+    }
+    // per-layer planes: the caller's (F,T,C) arrays for layer_norm2d, built here otherwise
+    std::vector<float> plane_g[ENC_LAYERS], plane_b[ENC_LAYERS];
+    const float* ln_g[ENC_LAYERS];
+    const float* ln_b[ENC_LAYERS];
+    std::vector<float> lnc;
+    if (norm == NAFP_NORM_LAYER_NORM1D) lnc.assign(static_cast<size_t>(ENC_LAYERS) * 2048, 0.f);
+    for (int l = 0; l < ENC_LAYERS; ++l) {
+        const ConvGeom& L = s->g[l];
+        if (norm == NAFP_NORM_LAYER_NORM2D) {
+            ln_g[l] = norm_g[l];
+            ln_b[l] = norm_b[l];
+            continue;
+        }
+        const int C = L.c_out;
+        std::vector<float> sc(C), sh(C);
+        for (int c = 0; c < C; ++c) {
+            const float g = norm_g[l][c], b = norm_b[l][c];
+            if (bn) {
+                const double k = static_cast<double>(g) / std::sqrt(static_cast<double>(norm_var[l][c]) + LN_EPS);
+                sc[c] = static_cast<float>(k);
+                sh[c] = static_cast<float>(static_cast<double>(b) - static_cast<double>(norm_mean[l][c]) * k);
+            } else if (l == ENC_LAYERS - 1) {
+                sc[c] = g;
+                sh[c] = b;
+            } else {
+                sc[c] = 1.f;
+                sh[c] = 0.f;
+                lnc[static_cast<size_t>(l) * 2048 + c] = g;
+                lnc[static_cast<size_t>(l) * 2048 + 1024 + c] = b;
+            }
+        }
+        plane_g[l].resize(static_cast<size_t>(L.ms) * C);
+        plane_b[l].resize(static_cast<size_t>(L.ms) * C);
+        for (int pos = 0; pos < L.ms; ++pos) {
+            std::copy(sc.begin(), sc.end(), plane_g[l].begin() + static_cast<size_t>(pos) * C);
+            std::copy(sh.begin(), sh.end(), plane_b[l].begin() + static_cast<size_t>(pos) * C);
+        }
+        ln_g[l] = plane_g[l].data();
+        ln_b[l] = plane_b[l].data();
+    }
+    if (!lnc.empty())
+        NAFP_CUDA(cudaMemcpy(s->ln_c, lnc.data(), lnc.size() * sizeof(float), cudaMemcpyHostToDevice));
     struct Tmp {                       // fp32 weights / beta of the running layer, only needed by fold_kernel
         float *w = nullptr, *bias = nullptr, *beta_prev = nullptr, *beta_cur = nullptr;
         ~Tmp() { cudaFree(w); cudaFree(bias); cudaFree(beta_prev); cudaFree(beta_cur); }
@@ -1072,6 +1334,7 @@ int nafp_weights_load(nafp_ctx* ctx, const float* const* conv_w, const float* co
     NAFP_CUDA(cudaMemcpy(s->db1, div_b1, 128 * 32 * sizeof(float), cudaMemcpyHostToDevice));
     NAFP_CUDA(cudaMemcpy(s->dw2, div_w2, 128 * 32 * sizeof(float), cudaMemcpyHostToDevice));
     NAFP_CUDA(cudaMemcpy(s->db2, div_b2, 128 * sizeof(float), cudaMemcpyHostToDevice));
+    s->norm = norm;
     s->weights = true;
     return NAFP_OK;
 }
@@ -1212,8 +1475,10 @@ int nafp_encoder_activation_host(nafp_ctx* ctx, int layer, int64_t n_seg, float*
     std::vector<float2> st(static_cast<size_t>(n_seg));
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
     NAFP_CUDA(cudaMemcpy(tmp.data(), s->x[layer], tmp.size() * sizeof(__half), cudaMemcpyDeviceToHost));
-    NAFP_CUDA(cudaMemcpy(st.data(), s->stat + static_cast<size_t>(layer) * s->cap, st.size() * sizeof(float2), cudaMemcpyDeviceToHost));
+    NAFP_CUDA(cudaMemcpy(st.data(), layer_stat(s, layer), st.size() * sizeof(float2), cudaMemcpyDeviceToHost));
     // the device keeps z = gamma (.) ELU(...); LN(y) = a z + c gamma + beta with (a, c) = (rstd, -rstd mean) of the segment
+    // ('layer_norm1d' before the last layer: z is the normalised value, (a, c) = (1, 0), gamma = 1, beta = 0;
+    // 'batch_norm': (a, c) = (1, 0) and the planes are the folded scale / shift)
     const size_t C = L.c_out;
     for (size_t i = 0; i < n; ++i) {
         const size_t b = i / per, e = i % per;

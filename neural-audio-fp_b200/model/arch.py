@@ -19,6 +19,23 @@ EMB_SZ = 128
 DIVENC_UNITS = (32, 1)
 LN_EPS = 1e-3
 L2_EPS = 1e-12
+# MODEL.BN (nnfp.py:20-83, ConvLayer(norm=...)): LayerNormalization over (F,T,C), LayerNormalization over C, or
+# BatchNormalization over C (inference mode); eps 1e-3 for all three (Keras defaults)
+NORMS = ("layer_norm2d", "layer_norm1d", "batch_norm")
+
+
+def norm_shapes(spec: "ConvSpec", norm: str = "layer_norm2d") -> dict:
+    """Variables of the normalisation after conv ``spec``: suffix -> shape (``g``, ``b``; ``mean``, ``var`` for
+    batch_norm -- Keras' moving statistics)."""
+    if norm not in NORMS:
+        raise ValueError(f"norm {norm!r}: one of {NORMS}")
+    if norm == "layer_norm2d":
+        shp = (spec.f_out, spec.t_out, spec.c_out)
+        return {"g": shp, "b": shp}
+    out = {"g": (spec.c_out,), "b": (spec.c_out,)}
+    if norm == "batch_norm":
+        out.update(mean=(spec.c_out,), var=(spec.c_out,))
+    return out
 
 
 def tf_same(n_in: int, k: int, s: int) -> Tuple[int, int, int]:
@@ -69,11 +86,17 @@ def conv_specs(input_shape=(256, 32, 1)) -> List[ConvSpec]:
     return specs
 
 
-def n_params(input_shape=(256, 32, 1)) -> int:
+def n_params(input_shape=(256, 32, 1), norm="layer_norm2d") -> int:
+    """Keras' ``count_params`` of the FingerPrinter (batch_norm's moving statistics included)."""
     n = 0
     specs = conv_specs(input_shape)
     for s in specs:
-        n += 3 * s.c_in * s.c_out + s.c_out + 2 * s.f_out * s.t_out * s.c_out
+        n += 3 * s.c_in * s.c_out + s.c_out
+        for shp in norm_shapes(s, norm).values():
+            k = 1
+            for d in shp:
+                k *= d
+            n += k
     last = specs[-1]
     flat = last.f_out * last.t_out * last.c_out
     sl = flat // EMB_SZ

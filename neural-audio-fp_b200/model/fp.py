@@ -13,6 +13,9 @@ from . import arch
 from .weights import init_weights, load_weights
 
 _FP = ctypes.POINTER(ctypes.c_float)
+def _check_norm(norm):
+    if norm not in arch.NORMS:
+        raise NotImplementedError(f"MODEL.BN={norm!r}: one of {arch.NORMS}")
 
 
 def _check_model_cfg(cfg):
@@ -25,8 +28,7 @@ def _check_model_cfg(cfg):
         raise NotImplementedError("MODEL.DUR/F_MIN/F_MAX other than 1 s / 300 Hz / 4000 Hz are not built")
     if m['FEAT'] not in ('melspec', 'melspec_maxnorm'):      # model/generate.py:17-20 raises for anything else, too
         raise NotImplementedError(m['FEAT'])
-    if m['BN'] != 'layer_norm2d':
-        raise NotImplementedError(f"MODEL.BN={m['BN']!r}: only 'layer_norm2d' is on the hot path")
+    _check_norm(m['BN'])
 
 
 class Melspec:
@@ -62,12 +64,15 @@ class Melspec:
 
 
 class FingerPrinter:
-    """``m_fp`` (+ the fused ``test_step``).  Weights live on the device after ``load``."""
+    """``m_fp`` (+ the fused ``test_step``).  Weights live on the device after ``load``; ``norm`` is MODEL.BN
+    (``FingerPrinter(norm=...)``, nnfp.py:186) and decides which normalisation variables ``load`` expects."""
 
-    def __init__(self, ctx=None, device=0, segment_norm=False):
+    def __init__(self, ctx=None, device=0, segment_norm=False, norm='layer_norm2d'):
+        _check_norm(norm)
         self.ctx = ctx or Context.get(device)
         self.loaded = False
         self.segment_norm = bool(segment_norm)       # feature variant of the fused test_step entry points
+        self.norm = norm
 
     def load(self, weights):
         specs = arch.conv_specs()
@@ -80,16 +85,25 @@ class FingerPrinter:
             keep.append(a)
             return a.ctypes.data_as(_FP)
 
-        cw, cb, lg, lb = [(_FP * 16)() for _ in range(4)]
+        cw, cb, lg, lb, lm, lv = [(_FP * 16)() for _ in range(6)]
         for l, s in enumerate(specs):
             kshape = (1, 3, s.c_in, s.c_out) if s.axis == "t" else (3, 1, s.c_in, s.c_out)
             ln = s.name.replace("conv", "ln")
             cw[l] = arr(f"{s.name}_w", kshape)
             cb[l] = arr(f"{s.name}_b", (s.c_out,))
-            lg[l] = arr(f"{ln}_g", (s.f_out, s.t_out, s.c_out))
-            lb[l] = arr(f"{ln}_b", (s.f_out, s.t_out, s.c_out))
-        check(lib.nafp_weights_load(self.ctx.h, cw, cb, lg, lb, arr("div_w1", (128, 8, 32)), arr("div_b1", (128, 32)),
-                                    arr("div_w2", (128, 32, 1)), arr("div_b2", (128, 1))))
+            shapes = arch.norm_shapes(s, self.norm)
+            lg[l] = arr(f"{ln}_g", shapes["g"])
+            lb[l] = arr(f"{ln}_b", shapes["b"])
+            if self.norm == 'batch_norm':
+                lm[l] = arr(f"{ln}_mean", shapes["mean"])
+                lv[l] = arr(f"{ln}_var", shapes["var"])
+        div = (arr("div_w1", (128, 8, 32)), arr("div_b1", (128, 32)), arr("div_w2", (128, 32, 1)), arr("div_b2", (128, 1)))
+        if self.norm == 'layer_norm2d':
+            check(lib.nafp_weights_load(self.ctx.h, cw, cb, lg, lb, *div))
+        else:
+            bn = self.norm == 'batch_norm'
+            check(lib.nafp_weights_load_norm(self.ctx.h, arch.NORMS.index(self.norm), cw, cb, lg, lb, lm if bn else None,
+                                             lv if bn else None, *div))
         self.loaded = True
         return self
 
@@ -151,7 +165,7 @@ class FingerPrinter:
         return emb
 
     def activation(self, layer, n_seg):
-        """Post-LayerNorm activation (n_seg, F, T, C) of conv ``layer`` from the last encoder pass."""
+        """Activation (n_seg, F, T, C) of conv ``layer`` after its normalisation, from the last encoder pass."""
         s = arch.conv_specs()[layer]
         out = np.empty((n_seg, s.f_out, s.t_out, s.c_out), dtype=np.float32)
         check(lib.nafp_encoder_activation_host(self.ctx.h, int(layer), int(n_seg), ptr(out)))
@@ -163,7 +177,7 @@ def build_fp(cfg, device=0):
     _check_model_cfg(cfg)
     ctx = Context.get(device)
     seg_norm = cfg['MODEL']['FEAT'] == 'melspec_maxnorm'
-    return Melspec(ctx, segment_norm=seg_norm), FingerPrinter(ctx, segment_norm=seg_norm)
+    return Melspec(ctx, segment_norm=seg_norm), FingerPrinter(ctx, segment_norm=seg_norm, norm=cfg['MODEL']['BN'])
 
 
 def test_step(X, m_pre, m_fp, group_size=None):

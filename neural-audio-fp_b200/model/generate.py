@@ -33,7 +33,7 @@ def load_checkpoint(checkpoint_root_dir, checkpoint_name, checkpoint_index, m_fp
     """Mirror of ``generate.py:26-52``: restore the latest or the given checkpoint into m_fp."""
     if checkpoint_name.startswith('random-init'):
         seed = int(checkpoint_name.split(':')[1]) if ':' in checkpoint_name else 7
-        m_fp.load(init_weights(seed))
+        m_fp.load(init_weights(seed, norm=m_fp.norm))
         print(f'---Initialised random weights (seed {seed})---')
         return 0 if checkpoint_index is None else checkpoint_index
     checkpoint_dir = checkpoint_root_dir + f'/{checkpoint_name}/'
@@ -59,7 +59,7 @@ def load_checkpoint(checkpoint_root_dir, checkpoint_name, checkpoint_index, m_fp
         m_fp.load(load_weights(prefix + '.npz'))
         print(f'---Restored from {prefix}.npz---')
     elif os.path.exists(prefix + '.index'):
-        m_fp.load(load_tf_checkpoint(prefix))
+        m_fp.load(load_tf_checkpoint(prefix, norm=m_fp.norm))
         print(f'---Restored from {prefix} (TensorFlow checkpoint)---')
     else:
         raise FileNotFoundError(prefix + '.npz / .index')

@@ -12,11 +12,14 @@ format of ``model/weights.py``:
     model/front_conv/layer_with_weights-{i}/BN_1x3/{gamma,beta}          -> ln{i}_a_g,  ln{i}_a_b
     model/front_conv/layer_with_weights-{i}/conv2d_3x1/{kernel,bias}     -> conv{i}_b_w, conv{i}_b_b
     model/front_conv/layer_with_weights-{i}/BN_3x1/{gamma,beta}          -> ln{i}_b_g,  ln{i}_b_b
+    model/front_conv/layer_with_weights-{i}/BN_*/{moving_mean,moving_variance} -> ln{i}_*_mean, ln{i}_*_var
+                                                                            (MODEL.BN 'batch_norm' only)
     model/div_enc/split_fc_layers/{q}/layer_with_weights-{0,1}/{kernel,bias} -> div_w1/div_b1, div_w2/div_b2 [q]
 
 (each followed by ``/.ATTRIBUTES/VARIABLE_VALUE``; the same variables reached through ``.../forward/
 layer_with_weights-{0..3}`` are accepted too; optimizer slots are ignored).  Every tensor is checked against the
-shape ``model/arch.py`` derives for it, and against its stored crc32c.
+shape ``model/arch.py`` derives for it under the configured MODEL.BN (gamma / beta (F,T,C) for 'layer_norm2d', (C,)
+otherwise), and against its stored crc32c.
 
 STATUS: the file format is restated from TensorFlow's published sources (tensorflow/core/util/tensor_bundle,
 tensorflow/core/lib/io/table*) -- no TensorFlow and no reference checkpoint exist in the build container, so the
@@ -32,7 +35,7 @@ import struct
 
 import numpy as np
 
-from .arch import DIVENC_UNITS, EMB_SZ, conv_specs
+from .arch import DIVENC_UNITS, EMB_SZ, conv_specs, norm_shapes
 
 TABLE_MAGIC = 0xdb4775248b80fb57
 FOOTER_LEN = 48
@@ -321,7 +324,7 @@ def _crc32c_fast(blob, lanes=1024):
 
 # ------------------------------------------------------------------------------------------ name mapping
 _CONV_RE = re.compile(r"front_conv/layer_with_weights-(\d+)/(?:forward/layer_with_weights-(\d)/|"
-                      r"(conv2d_1x3|BN_1x3|conv2d_3x1|BN_3x1)/)(kernel|bias|gamma|beta)$")
+                      r"(conv2d_1x3|BN_1x3|conv2d_3x1|BN_3x1)/)(kernel|bias|gamma|beta|moving_mean|moving_variance)$")
 _DIV_RE = re.compile(r"div_enc/split_fc_layers/(\d+)/layer_with_weights-(\d)/(kernel|bias)$")
 _FORWARD_SLOTS = ("conv2d_1x3", "BN_1x3", "conv2d_3x1", "BN_3x1")        # nnfp.py:73-79 (ELU layers have no weights)
 
@@ -330,9 +333,12 @@ def is_model_variable(key):
     return key.endswith(_SUFFIX) and "/.OPTIMIZER_SLOT/" not in key and ("front_conv/" in key or "div_enc/" in key)
 
 
-def map_variables(tensors, input_shape=(256, 32, 1)):
-    """Bundle tensors (``read_bundle``) -> the weights dict of ``model/weights.py``; raises with the list of what is
-    missing or has an unexpected shape."""
+_BN_VARS = {"gamma": "g", "beta": "b", "moving_mean": "mean", "moving_variance": "var"}
+
+
+def map_variables(tensors, input_shape=(256, 32, 1), norm="layer_norm2d"):
+    """Bundle tensors (``read_bundle``) -> the weights dict of ``model/weights.py`` for MODEL.BN ``norm``; raises with
+    the list of what is missing, has an unexpected shape or belongs to another MODEL.BN."""
     specs = conv_specs(input_shape)
     n_blocks = len(specs) // 2
     w = {}
@@ -362,9 +368,14 @@ def map_variables(tensors, input_shape=(256, 32, 1)):
                     else (spec.c_out,)
                 dst = f"conv{blk}_{half}_{'w' if what == 'kernel' else 'b'}"
             else:
-                want = (spec.f_out, spec.t_out, spec.c_out)
-                dst = f"ln{blk}_{half}_{'g' if what == 'gamma' else 'b'}"
-            if what not in (("kernel", "bias") if layer.startswith("conv") else ("gamma", "beta")) or tuple(arr.shape) != want:
+                shapes = norm_shapes(spec, norm)
+                sfx = _BN_VARS.get(what)
+                if sfx not in shapes:
+                    problems.append(f"{key}: not a variable of MODEL.BN={norm!r}")
+                    continue
+                want = shapes[sfx]
+                dst = f"ln{blk}_{half}_{sfx}"
+            if what not in (("kernel", "bias") if layer.startswith("conv") else _BN_VARS) or tuple(arr.shape) != want:
                 problems.append(f"{key}: shape {tuple(arr.shape)}, expected {want}")
                 continue
             w[dst] = np.ascontiguousarray(arr, dtype=np.float32)
@@ -382,7 +393,7 @@ def map_variables(tensors, input_shape=(256, 32, 1)):
         problems.append(f"unrecognised model variable {key}")
     for s in specs:
         ln = s.name.replace("conv", "ln")
-        for k in (f"{s.name}_w", f"{s.name}_b", f"{ln}_g", f"{ln}_b"):
+        for k in (f"{s.name}_w", f"{s.name}_b", *(f"{ln}_{sfx}" for sfx in norm_shapes(s, norm))):
             if k not in w:
                 problems.append(f"missing {k}")
     for q in range(EMB_SZ):
@@ -390,14 +401,15 @@ def map_variables(tensors, input_shape=(256, 32, 1)):
             if (q, dst) not in div_seen:
                 problems.append(f"missing div_enc slice {q} {dst}")
     if problems:
-        raise ValueError("checkpoint does not match the FingerPrinter of model/fp/nnfp.py:\n  " + "\n  ".join(problems[:40]))
+        raise ValueError(f"checkpoint does not match the FingerPrinter of model/fp/nnfp.py (MODEL.BN={norm!r}):\n  "
+                         + "\n  ".join(problems[:40]))
     w.update({"div_w1": div["w1"], "div_b1": div["b1"], "div_w2": div["w2"], "div_b2": div["b2"]})
     return w
 
 
-def load_tf_checkpoint(prefix, verify=True, input_shape=(256, 32, 1)):
-    """``prefix`` = path without extension (``.../ckpt-100``) -> weights dict."""
-    return map_variables(read_bundle(prefix, verify, only=is_model_variable), input_shape)
+def load_tf_checkpoint(prefix, verify=True, input_shape=(256, 32, 1), norm="layer_norm2d"):
+    """``prefix`` = path without extension (``.../ckpt-100``) -> weights dict for MODEL.BN ``norm``."""
+    return map_variables(read_bundle(prefix, verify, only=is_model_variable), input_shape, norm)
 
 
 def latest_checkpoint(checkpoint_dir):
@@ -420,10 +432,11 @@ def latest_checkpoint(checkpoint_dir):
     return max(found) if found else (None, None)
 
 
-def convert(prefix, npz_path=None):
-    """CLI helper: write the ``.npz`` exchange file next to the checkpoint (or to ``npz_path``)."""
+def convert(prefix, npz_path=None, norm="layer_norm2d"):
+    """CLI helper: write the ``.npz`` exchange file next to the checkpoint (or to ``npz_path``); 'batch_norm' adds the
+    moving statistics as ``ln*_mean`` / ``ln*_var``."""
     from .weights import save_weights
-    w = load_tf_checkpoint(prefix)
+    w = load_tf_checkpoint(prefix, norm=norm)
     npz_path = npz_path or prefix + ".npz"
     save_weights(npz_path, w)
     return npz_path
@@ -432,5 +445,6 @@ def convert(prefix, npz_path=None):
 if __name__ == "__main__":
     import sys
     if len(sys.argv) < 2:
-        raise SystemExit("usage: python -m nafp_b200.model.tf_checkpoint CKPT_PREFIX [OUT.npz]")
-    print(convert(*sys.argv[1:3]))
+        raise SystemExit("usage: python -m nafp_b200.model.tf_checkpoint CKPT_PREFIX [OUT.npz] [MODEL.BN]")
+    print(convert(sys.argv[1], sys.argv[2] if len(sys.argv) > 2 and sys.argv[2] else None,
+                  sys.argv[3] if len(sys.argv) > 3 else "layer_norm2d"))
