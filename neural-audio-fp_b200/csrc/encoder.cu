@@ -33,7 +33,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -84,7 +83,6 @@ struct ConvParams {
     int combos;      // (position tiles per segment) x (channel tiles): what a CTA stays on
     int n_streams;   // CTAs per combo; CTA c works on combo c % combos, unit c / combos, + n_streams, ...
     int n_units;     // units per combo: segments (ms >= 128) or 128-row groups of whole segments (ms < 128)
-    int l2_prefetch; // 1 = the producer prefetches the next units' A boxes into L2
     int tma_store;   // 1 = z leaves through a swizzled shared-memory tile and TMA stores (full-tile layers, fp16 output)
 };
 
@@ -112,10 +110,6 @@ struct EncoderState {
     float* raw = nullptr;                      // (cap, 128) head outputs before the L2 normalisation
     CUtensorMap tmA[ENC_LAYERS], tmB[ENC_LAYERS], tmO[ENC_LAYERS];     // activation in, weights, activation out (TMA store)
     bool weights = false;
-    int tma_store = 1;                         // NAFP_ENC_TMASTORE=0: direct 32-byte stores from the epilogue registers (A/B)
-    int l2_prefetch = 0;                       // NAFP_ENC_L2PF=1 makes the producers prefetch the next unit's A boxes into L2
-                                               // (measured: 7.5 vs 6.9 ms per 4,000 segments -- the UTMAPF requests compete
-                                               // with the loads for the same TMA / L2 request slots; kept as a switch)
     int64_t last_n = 0;                        // segments of the last pass (activation probe)
     int norm = NAFP_NORM_LAYER_NORM2D;         // MODEL.BN of the loaded weights (nafp_weights_load_norm)
     int split_from = 0;                        // first split-precision layer of g (split_point(norm))
@@ -134,8 +128,7 @@ static void same_pad(int n_in, int k, int s, int* n_out, int* lo) {
     *lo = total / 2;
 }
 
-// split_from: first layer whose operands are split (hi + lo); the default, ENC_SPLIT_FROM, or what the norm needs
-// (split_point)
+// split_from: first layer whose operands are split (hi + lo), split_point(norm)
 static void build_geometry(ConvGeom* g, int split_from) {
     int f = 256, t = 32, c = 1;
     for (int i = 0; i < 8; ++i) {
@@ -167,9 +160,8 @@ static void build_geometry(ConvGeom* g, int split_from) {
         }
     }
     // N = 256 where measured faster (4,000-segment pass, round 2): L5b, L6b, L7b, L8a, L8b -- the layers whose A
-    // operand is tiny and whose time is the re-streaming of the weights; NAFP_ENC_NT256 (bit mask of layers) overrides
-    unsigned nt256 = (1u << 9) | (1u << 11) | (1u << 13) | (1u << 14) | (1u << 15);
-    if (const char* e = getenv("NAFP_ENC_NT256")) nt256 = static_cast<unsigned>(strtoul(e, nullptr, 0));
+    // operand is tiny and whose time is the re-streaming of the weights
+    constexpr unsigned nt256 = (1u << 9) | (1u << 11) | (1u << 13) | (1u << 14) | (1u << 15);
     for (int l = 1; l < 16; ++l)
         if (((nt256 >> l) & 1u) && g[l].c_out >= 256 && g[l].ms < 128) g[l].nt = 256;
     for (int l = 0; l < 16; ++l) g[l].ksplit = l >= split_from ? 3 : 1;
@@ -572,7 +564,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     for (int kb = 0; kb < p.kb_per_tap; ++kb, ++k)
                         tma_load_2d(b_s + k * CONV_B_BYTES, &tmB, &bars->bfull, tap * p.c_in + kb * 64, n0);
             }
-            // A boxes of unit u: either into the ring (dst != nullptr) or as an L2 prefetch
+            // A box (tap, channels c0 ..) of unit u into ring slot dst
+            // (an L2 prefetch of the next unit's A boxes was measured slower: 7.5 vs 6.9 ms per 4,000 segments -- the
+            // prefetch requests compete with the loads for the same TMA / L2 request slots)
             auto a_box = [&](uint8_t* dst, uint64_t* bar, int u, int tap, int c0) {
                 int b0, f0;
                 if (p.ms >= 128) { b0 = u;        f0 = ptile * p.bf; }
@@ -581,29 +575,12 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 // mode 1: (c,tp,th,f,b)    time conv stride 2: t = 2 t' + tap -> parity tap&1, half t' + (tap>>1)
                 // mode 2: (c,t,fp,fh,b)    freq conv stride 2: f = 2 f' + tap
                 // mode 3: (c,t,f,b)        freq conv with a single output row: f = tap - pad
-                if (dst) {
-                    if (p.mode == 0)      tma_load_4d(dst, &tmA, bar, c0, tap - p.pad_lo, f0, b0);
-                    else if (p.mode == 1) tma_load_5d(dst, &tmA, bar, c0, tap & 1, tap >> 1, f0, b0);
-                    else if (p.mode == 2) tma_load_5d(dst, &tmA, bar, c0, 0, tap & 1, f0 + (tap >> 1), b0);
-                    else                  tma_load_4d(dst, &tmA, bar, c0, 0, f0 + tap - p.pad_lo, b0);
-                } else {
-                    if (p.mode == 0)      tma_prefetch_4d(&tmA, c0, tap - p.pad_lo, f0, b0);
-                    else if (p.mode == 1) tma_prefetch_5d(&tmA, c0, tap & 1, tap >> 1, f0, b0);
-                    else if (p.mode == 2) tma_prefetch_5d(&tmA, c0, 0, tap & 1, f0 + (tap >> 1), b0);
-                    else                  tma_prefetch_4d(&tmA, c0, 0, f0 + tap - p.pad_lo, b0);
-                }
+                if (p.mode == 0)      tma_load_4d(dst, &tmA, bar, c0, tap - p.pad_lo, f0, b0);
+                else if (p.mode == 1) tma_load_5d(dst, &tmA, bar, c0, tap & 1, tap >> 1, f0, b0);
+                else if (p.mode == 2) tma_load_5d(dst, &tmA, bar, c0, 0, tap & 1, f0 + (tap >> 1), b0);
+                else                  tma_load_4d(dst, &tmA, bar, c0, 0, f0 + tap - p.pad_lo, b0);
             };
-            // The ring holds about one unit of A, and its slots are re-requested only as the MMAs of the previous
-            // unit retire: without help the stream is bound by DRAM latency (ncu: 55 % of DRAM, nothing saturated).
-            // The DRAM -> L2 leg of the NEXT unit is therefore started (UTMAPF.L2) before this unit's loads queue up.
-            auto prefetch_unit = [&](int u) {
-                if (u >= p.n_units || p.l2_prefetch == 0) return;
-                for (int tap = p.tap_lo; tap <= p.tap_hi; ++tap)
-                    for (int kb = 0; kb < p.kb_per_tap; ++kb) a_box(nullptr, nullptr, u, tap, kb * 64);
-            };
-            prefetch_unit(stream + p.n_streams);
             for (int u = stream; u < p.n_units; u += p.n_streams) {
-                prefetch_unit(u + 2 * p.n_streams);
                 for (int tap = p.tap_lo; tap <= p.tap_hi; ++tap) {
                     for (int kb = 0; kb < p.kb_per_tap; ++kb, ++it) {
                         const int s = it % CONV_STAGES;
@@ -924,18 +901,13 @@ l2norm_kernel(const float* __restrict__ raw, int n_seg, float* __restrict__ emb)
 // ------------------------------------------------------------------------------------------
 // host
 // ------------------------------------------------------------------------------------------
+static_assert(ENC_SPLIT_FROM >= 2, "conv0_kernel writes split output only without the fused layer_norm1d");
 // First split-precision layer for a MODEL.BN.  'batch_norm' needs every layer split: its per-channel scale
 // gamma / sqrt(var + eps) reaches ~30 on channels ELU saturates (variance near 0), and any fp16 rounding of an
 // activation before that scale -- even L1a's output, or the normalised value -- carries the fingerprints past 1e-3
 // (measured on B200 with the default split point: max-abs 1.6-4.6e-3; an fp16-storage model of the network on the
 // host gives 0.9-3e-3 for every split point from L1b's output on and rounding-level error with L1a's output split).
-static int split_point(int norm) {
-    if (norm == NAFP_NORM_BATCH_NORM) return 1;
-    int split_from = ENC_SPLIT_FROM;           // NAFP_ENC_SPLIT_FROM: A/B of the error / speed trade (16 = no split layer)
-    if (const char* e = getenv("NAFP_ENC_SPLIT_FROM")) split_from = atoi(e);
-    if (split_from < 2) split_from = 2;        // conv0_kernel writes split output only without the fused layer_norm1d
-    return split_from;
-}
+static int split_point(int norm) { return norm == NAFP_NORM_BATCH_NORM ? 1 : ENC_SPLIT_FROM; }
 
 // the weight operands and their tensor maps: sized by the split point of the geometry
 static int encoder_weight_buffers(EncoderState* s) {
@@ -960,8 +932,6 @@ static int encoder_init(nafp_ctx* ctx) {
     ctx->encoder = s;              // before the first fallible call: nafp_ctx_destroy releases it
     s->split_from = split_point(NAFP_NORM_LAYER_NORM2D);
     build_geometry(s->g, s->split_from);
-    if (const char* e = getenv("NAFP_ENC_L2PF")) s->l2_prefetch = atoi(e) != 0;
-    if (const char* e = getenv("NAFP_ENC_TMASTORE")) s->tma_store = atoi(e) != 0;
     NAFP_CUDA(cudaMalloc(&s->w0, 3 * 128 * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&s->bias0, 128 * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&s->ln_b15, 1024 * sizeof(float)));
@@ -1129,8 +1099,7 @@ static int encoder_pass(nafp_ctx* ctx, const float* mel, const int32_t* gmax, in
             p.n_streams = ctx->sm_count / p.combos;
             if (p.n_streams > p.n_units) p.n_streams = p.n_units;
             if (p.n_streams < 1) p.n_streams = 1;
-            p.l2_prefetch = s->l2_prefetch;
-            p.tma_store = (s->tma_store && L.nt == 128 && L.ms >= 128 && L.osplit == 1 && CONV_EPI_PARTS == 2) ? 1 : 0;
+            p.tma_store = (L.nt == 128 && L.ms >= 128 && L.osplit == 1 && CONV_EPI_PARTS == 2) ? 1 : 0;
             slots = p.groups * p.n_ntiles * CONV_EPI_PARTS;
             auto kern = L.nt == 128 ? conv_gemm_kernel<128> : conv_gemm_kernel<256>;
             kern<<<p.combos * p.n_streams, CONV_THREADS, CONV_SMEM, st>>>(

@@ -6,19 +6,18 @@
 //           quantizer, then one k-means per sub-space on the residuals; deterministic (fixed-order sums)
 //   add     ivfpq_encode_kernel: nearest coarse centroid + 64 one-byte codes per row; the inverted
 //           lists are a stable counting sort of (list, row) rebuilt lazily before the next search
-//   search  ivfpq_probe_kernel (nprobe nearest lists per query row) ->
+//   search  by default the list-major tensor-core scan of the compressed lists (ivfpq_lm.cu).  The LUT kernel
+//           below is the reference formulation: it answers the query rows and shapes the list-major scan cannot
+//           (and every search of an index created with NAFP_IVFPQ_PATH=lut):
+//           ivfpq_probe_kernel (nprobe nearest lists per query row) ->
 //           ivfpq_scan_kernel  (one CTA per (query row, probed list): 64 x 256 fp32 look-up table in
 //                               shared memory, ADC scan of the list's codes, block top-k) ->
 //           topk merge of the nprobe partial lists.
-//           -- that is the reference formulation and the fallback.  The fast path uses the identity
-//           ADC(q, code) = |q - xhat|^2 (xhat = the row's reconstruction): a flat index over xhat (same row
-//           order) is searched with the tensor-core scan for the 64 nearest reconstructions, the candidates
-//           outside the nprobe nearest lists are dropped, and k survivors in order ARE the IVF-PQ answer.
 //
 // IVF-Flat ('ivf', faiss.IndexIVFFlat(IndexFlatL2(d), d, nlist=400), get_index_faiss.py:63-66) shares the coarse
-// quantizer, the probe and the filter: the exact flat scan of the index's own rows gives the 64 nearest rows,
-// the ones outside the probed lists are dropped; rows left with fewer than k answers get an exact scan of
-// their probed lists (ivfflat_scan_kernel).
+// quantizer and the probe: the exact flat scan of the index's own rows gives the 64 nearest rows, the filter drops
+// the ones outside the probed lists; rows left with fewer than k answers get an exact scan of their probed lists
+// (ivfflat_scan_kernel).
 #include <algorithm>
 #include <cfloat>
 #include <climits>
@@ -572,27 +571,8 @@ ivfflat_scan_kernel(const float* __restrict__ q, int64_t nq, const int32_t* __re
     }
 }
 
-// xhat[row] = coarse[assign[row]] + concat_m pq[m][code[row][m]]; one warp per row, lane owns 4 dims
-__global__ void ivfpq_decode_kernel(const int32_t* __restrict__ assign, const uint8_t* __restrict__ codes, int64_t row0, int64_t n,
-                                    const float* __restrict__ coarse, const float* __restrict__ pq, int m, int dsub,
-                                    float* __restrict__ out) {
-    const int lane = threadIdx.x & 31;
-    const int64_t r = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-    if (r >= n) return;
-    const int64_t row = row0 + r;
-    const int l = assign[row];
-    float4 v = reinterpret_cast<const float4*>(coarse + static_cast<int64_t>(l) * D128)[lane];
-    float* vv = reinterpret_cast<float*>(&v);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int d = 4 * lane + j, sub = d / dsub, w = d - sub * dsub;
-        vv[j] += pq[(static_cast<int64_t>(sub) * PQ_KSUB + codes[row * m + sub]) * dsub + w];
-    }
-    reinterpret_cast<float4*>(out + r * D128)[lane] = v;
-}
-
-// One warp per query row: keep the flat scan's candidates whose list is probed, in order.  k of them (or all
-// stored rows of the probed lists) ARE the restricted top-k; otherwise the row goes to the LUT kernel.
+// IVF-Flat, one warp per query row: keep the flat scan's candidates whose list is probed, in order.  k of them (or
+// all stored rows of the probed lists) ARE the restricted top-k; otherwise the row goes to ivfflat_scan_kernel.
 __global__ void ivfpq_filter_kernel(const float* __restrict__ candD, const int64_t* __restrict__ candI, int64_t nq, int k,
                                     const int32_t* __restrict__ probes, int nprobe, const int32_t* __restrict__ assign,
                                     int64_t label_offset, float* __restrict__ D, int64_t* __restrict__ I,
@@ -601,10 +581,10 @@ __global__ void ivfpq_filter_kernel(const float* __restrict__ candD, const int64
     const int64_t q = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
     if (q >= nq) return;
     int kept = 0;
-    bool exhausted = false;            // fewer than RECON_K rows exist at all: the candidate list is complete
-    for (int c0 = 0; c0 < RECON_K && kept < k; c0 += 32) {
+    bool exhausted = false;            // fewer than IVFFLAT_K rows exist at all: the candidate list is complete
+    for (int c0 = 0; c0 < IVFFLAT_K && kept < k; c0 += 32) {
         const int c = c0 + lane;
-        const int64_t id = candI[q * RECON_K + c];
+        const int64_t id = candI[q * IVFFLAT_K + c];
         bool in = false;
         if (id >= 0) {
             const int l = assign[id];
@@ -614,7 +594,7 @@ __global__ void ivfpq_filter_kernel(const float* __restrict__ candD, const int64
         const unsigned mask = __ballot_sync(0xffffffffu, in);
         const int pos = kept + __popc(mask & ((1u << lane) - 1));
         if (in && pos < k) {
-            D[q * k + pos] = candD[q * RECON_K + c];
+            D[q * k + pos] = candD[q * IVFFLAT_K + c];
             I[q * k + pos] = id + label_offset;
         }
         kept += __popc(mask);
@@ -808,24 +788,18 @@ int ivfpq_create(nafp_index* idx, int nlist, int m, int nbits) {
     NAFP_CUDA(cudaMalloc(&s->pq, static_cast<size_t>(m) * PQ_KSUB * s->dsub * sizeof(float)));
     NAFP_CUDA(cudaMalloc(&s->loff, (nlist + 1) * sizeof(int32_t)));
     NAFP_CUDA(cudaMalloc(&s->lend, nlist * sizeof(int32_t)));
-    // search path: the list-major compressed-domain scan (ivfpq_lm.cu) unless NAFP_IVFPQ_PATH says otherwise; only
-    // the reconstruction path keeps a flat index over the decoded rows (772 B per row)
+    // search path: the list-major compressed-domain scan (ivfpq_lm.cu) unless NAFP_IVFPQ_PATH=lut asks for the LUT kernel
     const char* e = getenv("NAFP_IVFPQ_PATH");
-    s->path = !e ? IVFPQ_PATH_LM : !strcmp(e, "recon") ? IVFPQ_PATH_RECON : !strcmp(e, "lut") ? IVFPQ_PATH_LUT : IVFPQ_PATH_LM;
-    if (s->path == IVFPQ_PATH_RECON) {
-        NAFP_CUDA(cudaMalloc(&s->xhat_tmp, static_cast<size_t>(RECON_CHUNK) * D128 * sizeof(float)));
-        NAFP_TRY(nafp_index_create(idx->ctx, NAFP_INDEX_FLAT_L2, D128, 0, 0, 8, &s->recon));
-    }
+    s->lut_only = e && !strcmp(e, "lut");
     return NAFP_OK;
 }
 
 void ivfpq_destroy(nafp_index* idx) {
     IvfPq* s = idx->ivf;
     if (!s) return;
-    if (s->recon) nafp_index_destroy(s->recon);
     ivfpq_lm_destroy(s);
     void* bufs[] = {s->coarse, s->pq, s->assign, s->codes, s->lcodes, s->lids, s->loff, s->lend, s->probes, s->partD, s->partI,
-                    s->xhat_tmp, s->candD, s->candI, s->probes_all, s->redo_rows, s->redo_q, s->redo_D, s->redo_I,
+                    s->candD, s->candI, s->probes_all, s->redo_rows, s->redo_q, s->redo_D, s->redo_I,
                     s->rpq, s->rcodes, s->refD, s->refI};
     for (void* b : bufs) if (b) cudaFree(b);
     delete s;
@@ -953,15 +927,6 @@ int ivfpq_add_rows(nafp_index* idx, int64_t row0, int64_t n) {
     }
     NAFP_CUDA(cudaGetLastError());
     s->dirty = true;
-    if (!s->recon) return NAFP_OK;
-    NAFP_TRY(index_reserve(s->recon, idx->cap));
-    for (int64_t r0 = 0; r0 < n; r0 += RECON_CHUNK) {
-        const int64_t nc = n - r0 < RECON_CHUNK ? n - r0 : RECON_CHUNK;
-        ivfpq_decode_kernel<<<static_cast<unsigned>((nc * 32 + 255) / 256), 256, 0, ctx->stream>>>(
-            s->assign, s->codes, row0 + r0, nc, s->coarse, s->pq, s->m, s->dsub, s->xhat_tmp);
-        ctx->launches++;
-        NAFP_TRY(flat_add_dev(s->recon, s->xhat_tmp, nc, false));
-    }
     return NAFP_OK;
 }
 
@@ -1023,7 +988,7 @@ int build_lists(nafp_index* idx) {
     s->h_lend = end;
     s->lists_version++;
     s->dirty = false;
-    if (!s->flat_lists && !s->refine && !s->recon && s->codes) {      // (IVFPQR re-ranks, the reconstruction path decodes, by row)
+    if (!s->flat_lists && !s->refine && s->codes) {      // (IVFPQR re-ranks by row)
         cudaFree(s->codes);
         s->codes = nullptr;
     }
@@ -1196,18 +1161,19 @@ static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t
     if (!s->flat_lists) idx->host_rows += nq;          // (the flat scan of an IVF-Flat index counts its own rows)
     if (nq >= (1ll << 31)) return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
     if (!s->flat_lists) {
-        if (s->path == IVFPQ_PATH_LM && ivfpq_lm_supported(idx, k)) return ivfpq_search_lm(idx, q_dev, nq, k, D_dev, I_dev);
-        if (s->path != IVFPQ_PATH_RECON || !s->recon) return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
+        if (!s->lut_only && ivfpq_lm_supported(idx, k)) return ivfpq_search_lm(idx, q_dev, nq, k, D_dev, I_dev);
+        return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
     }
-    if (k > RECON_K / 2) return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
 
-    // 1. exact top-RECON_K over the reconstructed rows (tensor-core scan + fp32 re-rank)
+    // IVF-Flat
+    if (k > IVFFLAT_K / 2) return ivfpq_search_lut(idx, q_dev, nq, k, D_dev, I_dev);
+    // 1. exact top-IVFFLAT_K over the stored rows (tensor-core scan + fp32 re-rank)
     if (s->cand_nq < nq) {
         if (s->candD) cudaFree(s->candD);
         if (s->candI) cudaFree(s->candI);
         s->candD = nullptr; s->candI = nullptr; s->cand_nq = 0;
-        NAFP_CUDA(cudaMalloc(&s->candD, static_cast<size_t>(nq) * RECON_K * sizeof(float)));
-        NAFP_CUDA(cudaMalloc(&s->candI, static_cast<size_t>(nq) * RECON_K * sizeof(int64_t)));
+        NAFP_CUDA(cudaMalloc(&s->candD, static_cast<size_t>(nq) * IVFFLAT_K * sizeof(float)));
+        NAFP_CUDA(cudaMalloc(&s->candI, static_cast<size_t>(nq) * IVFFLAT_K * sizeof(int64_t)));
         s->cand_nq = nq;
     }
     if (s->probes_all_elems < nq * nprobe) {
@@ -1220,16 +1186,11 @@ static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t
     NAFP_TRY(ivfpq_reserve_redo(idx, nq));
     int32_t* redo_count = s->redo_rows + s->redo_cap;
     NAFP_CUDA(cudaMemsetAsync(redo_count, 0, sizeof(int32_t), ctx->stream));
-    if (s->flat_lists) {               // the stored rows are the "reconstructions": scan the index itself
-        const int64_t off = idx->label_offset;      // the filter wants local rows and adds the offset itself
-        idx->label_offset = 0;
-        const int st = flat_search_dev(idx, q_dev, nq, RECON_K, s->candD, s->candI);
-        idx->label_offset = off;
-        NAFP_TRY(st);
-    } else {
-        s->recon->search_rows = idx->search_rows;
-        NAFP_TRY(flat_search_dev(s->recon, q_dev, nq, RECON_K, s->candD, s->candI));
-    }
+    const int64_t off = idx->label_offset;      // the filter wants local rows and adds the offset itself
+    idx->label_offset = 0;
+    const int st = flat_search_dev(idx, q_dev, nq, IVFFLAT_K, s->candD, s->candI);
+    idx->label_offset = off;
+    NAFP_TRY(st);
     // 2. the nprobe nearest lists of every row, 3. keep the candidates that live in them
     ivfpq_probe_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, ctx->stream>>>(q_dev, nq, s->coarse, s->nlist, nprobe, probes_all);
     ivfpq_filter_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, ctx->stream>>>(s->candD, s->candI, nq, k, probes_all, nprobe,
@@ -1240,7 +1201,7 @@ static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t
     int32_t n_redo = 0;
     NAFP_CUDA(cudaMemcpyAsync(&n_redo, redo_count, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
-    // 4. rows with fewer than k probed rows among their RECON_K nearest: the LUT scan of their lists
+    // 4. rows with fewer than k probed rows among their IVFFLAT_K nearest: the exact scan of their lists
     if (n_redo > 0) NAFP_TRY(ivfpq_redo_rows(idx, q_dev, n_redo, k, D_dev, I_dev));
     return NAFP_OK;
 }

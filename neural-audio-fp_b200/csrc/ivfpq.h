@@ -1,4 +1,4 @@
-// IVF-PQ state shared by ivfpq.cu (training, encoding, lists, LUT scan, reconstruction path) and ivfpq_lm.cu
+// IVF-PQ state shared by ivfpq.cu (training, encoding, lists, LUT scan, IVF-Flat scan + filter) and ivfpq_lm.cu
 // (the list-major compressed-domain tensor-core scan).
 #pragma once
 #include "index.h"
@@ -11,12 +11,10 @@ constexpr int IVF_MAX_NLIST = 1024;
 constexpr int REFINE_M = 4, REFINE_KSUB = 16, REFINE_DSUB = 32, REFINE_KFACTOR = 4;
 constexpr int IVF_SCAN_CAP = 512;         // candidate buffer per (query, list) CTA: two 512-key sorts per list instead of two 1024-key ones
 
-// search paths of an IVF-PQ index (NAFP_IVFPQ_PATH = lm | recon | lut, read when the index is created)
-enum IvfPqPath { IVFPQ_PATH_LM = 0, IVFPQ_PATH_RECON = 1, IVFPQ_PATH_LUT = 2 };
 struct LmState;                       // ivfpq_lm.cu
 
 struct IvfPq {
-    int path = IVFPQ_PATH_LM;
+    bool lut_only = false;        // NAFP_IVFPQ_PATH=lut when the index was created: every search runs the LUT kernel
     LmState* lm = nullptr;        // list-major scan: per-position row terms, bf16 codebook table, work lists, candidates
     int nlist = 256, m = 64, dsub = 2;
     bool flat_lists = false;      // IVF-Flat: the lists hold the stored rows themselves (no product quantizer)
@@ -54,26 +52,21 @@ struct IvfPq {
     int64_t* partI = nullptr;
     int64_t scratch_nq = 0;
     int scratch_nprobe = 0, scratch_k = 0;
-    // reconstruction path: ADC(q, code) = |q - xhat|^2 with xhat = coarse[list] + pq[m][code_m], so the IVF-PQ
-    // answer is the EXACT nearest-neighbour search over the reconstructed rows restricted to the probed
-    // lists.  B200 has the HBM to keep xhat resident: a flat index over it lets the tensor-core scan replace
-    // nq * nprobe * |list| * M shared-memory LUT gathers; the LUT kernel answers what the filter cannot prove.
-    nafp_index* recon = nullptr;  // flat index over xhat, same row order
-    float* xhat_tmp = nullptr;    // [RECON_CHUNK][128] decode staging
-    float* candD = nullptr;       // [nq_cap][RECON_K]
+    // IVF-Flat: the flat scan of the stored rows gives IVFFLAT_K candidates per query row, the filter keeps the ones
+    // in probed lists; rows it cannot answer are redone by an exact scan of their probed lists (ivfpq_redo_rows)
+    float* candD = nullptr;       // [nq_cap][IVFFLAT_K]
     int64_t* candI = nullptr;
     int64_t cand_nq = 0;
     int32_t* probes_all = nullptr;    // [nq][nprobe] of the whole call
     int64_t probes_all_elems = 0;
-    int32_t* redo_rows = nullptr; // query rows the filter could not answer, + counter at [cap]
+    int32_t* redo_rows = nullptr; // query rows the filter or the list-major scan could not answer, + counter at [cap]
     float* redo_q = nullptr;      // gathered copies of those rows, and their results
     float* redo_D = nullptr;
     int64_t* redo_I = nullptr;
     int64_t redo_cap = 0;
     unsigned long long lut_rows = 0;      // rows answered by the LUT kernel since creation (statistics)
 };
-constexpr int RECON_K = 64;               // candidates fetched from the flat scan per query row
-constexpr int64_t RECON_CHUNK = 1 << 20;  // rows decoded per add step
+constexpr int IVFFLAT_K = 64;             // IVF-Flat candidates per query row, fetched from the flat scan
 
 
 

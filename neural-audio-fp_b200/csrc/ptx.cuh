@@ -159,21 +159,6 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 // all committed stores are complete
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-// L2 prefetch of a tensor box (no shared-memory destination, no barrier): the DRAM -> L2 leg of a later TMA load is
-// started early, so the bytes in flight towards DRAM are not limited by the shared-memory ring
-__device__ __forceinline__ void tma_prefetch_2d(const void* tmap, int32_t c0, int32_t c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_4d(const void* tmap, int32_t c0, int32_t c1, int32_t c2, int32_t c3) {
-    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_5d(const void* tmap, int32_t c0, int32_t c1, int32_t c2, int32_t c3, int32_t c4) {
-    asm volatile("cp.async.bulk.prefetch.tensor.5d.L2.global.tile [%0, {%1, %2, %3, %4, %5}];"
-                 ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4) : "memory");
-}
 // packed fp32 pairs (FFMA2 / FADD2 / FMUL2: two fp32 operations per issue slot)
 __device__ __forceinline__ uint64_t pk2(float a, float b) {
     uint64_t r;

@@ -1,5 +1,5 @@
-"""Developer helper: fingerprint error against the fp64 oracle (max |err|, rms, min cosine) and throughput for the
-current encoder settings (NAFP_ENC_SPLIT_FROM, NAFP_ENC_NT256, ...).  usage: dev_encoder_err.py [n_segments]"""
+"""Developer helper: fingerprint error against the fp64 oracle (max |err|, rms, min cosine) and throughput of the
+encoder.  usage: dev_encoder_err.py [n_segments]"""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -30,6 +30,5 @@ check(lib.nafp_timer_start(ctx.h))
 for _ in range(10):
     check(lib.nafp_fingerprint(ctx.h, xd, 4000, 125, ed))
 check(lib.nafp_timer_stop(ctx.h, ctypes.byref(ms)))
-print(f"split_from={os.environ.get('NAFP_ENC_SPLIT_FROM', 'default')} nt256={os.environ.get('NAFP_ENC_NT256', 'default')}: "
-      f"{4000 / (ms.value / 10) * 1e3:,.0f} seg/s; " +
+print(f"{4000 / (ms.value / 10) * 1e3:,.0f} seg/s; " +
       "; ".join(f"w{s}{'a' if a else ''}: max {mx:.2e} rms {r:.2e} cos {c:.7f}" for s, a, mx, r, c in out))

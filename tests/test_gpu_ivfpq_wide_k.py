@@ -110,8 +110,8 @@ def test_wide_k_more_query_rows_than_one_launch_group(monkeypatch):
     _same(a, b, q, 128)
 
 
-def test_wide_k_fallback_rows_on_the_three_paths_set(monkeypatch):
-    """The 60,000-row set of test_ivfpq_three_search_paths_agree at k = 80: the list-major path answers (passes > 0),
+def test_wide_k_fallback_rows_on_the_search_paths_set(monkeypatch):
+    """The 60,000-row set of test_ivfpq_search_paths_agree at k = 80: the list-major path answers (passes > 0),
     bit-identical to the LUT kernel, with at most 1 % of the rows sent to the LUT kernel."""
     from nafp_b200 import synth
     dummy, db, query = synth.synth_search_set(60000, 1180, seed=23)
