@@ -219,14 +219,6 @@ int nafp_index_last_search_stats(nafp_index* idx, int64_t* out8);
  * previous call (at most 8192 launches are recorded between calls). */
 int nafp_index_profile_scans(nafp_index* idx, int enable, double* total_ms, int64_t* n_scans);
 
-/* developer probe of the last flat scan pass (512 entries each, one per query row of a pass): fallback flags,
- * shared thresholds, survivors per query row */
-int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags512, float* thr512, int32_t* total512);
-/* developer probe: per-CTA survivor counts [grid][512] (0 where a CTA does not hold the query row) and the tile index
- * at which each CTA first saw a shared threshold per query row [grid][512] (-1 = never; entries 504..511 are in-kernel
- * timestamps when the pass has <= 504 rows); the first call arms the probe */
-int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_out, int32_t* grid_out);
-
 /* ------------------------------------------------------------------ sequence matcher
  * Replaces the body of the hot loop eval/eval_faiss.py:204-232 for a batch of test ids.
  *   q_host      (n_query_rows, d) float32 -- the whole `query` memmap (or a slice)

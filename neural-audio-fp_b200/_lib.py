@@ -90,8 +90,6 @@ _SIGS = {
     "nafp_index_reconstruct_host": (c_int, [c_void_p, c_int64, c_int64, c_void_p]),
     "nafp_index_last_search_stats": (c_int, [c_void_p, _i64p]),
     "nafp_index_profile_scans": (c_int, [c_void_p, c_int, POINTER(ctypes.c_double), _i64p]),
-    "nafp_index_debug_last_pass": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
-    "nafp_index_debug_enable": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "nafp_seq_match": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
     "nafp_seq_plan_dev": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int64, c_void_p, c_void_p, c_void_p, _i64p]),
     "nafp_seq_gather_rows_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),

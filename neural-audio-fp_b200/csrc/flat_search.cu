@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1)
 flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_db,
                  const float* __restrict__ hn, int32_t* __restrict__ tile_counter, int64_t n_search, int n_tiles, int nq,
                  int n_half, int kg, int32_t* __restrict__ Mx, int32_t* __restrict__ Tg, uint64_t* __restrict__ pool,
-                 int32_t* __restrict__ cnt, int32_t* __restrict__ flags, int32_t* __restrict__ dbg_first, int tune) {
+                 int32_t* __restrict__ cnt, int32_t* __restrict__ flags) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t* q_s = smem;                                   // [kb 2][256 query rows][128 B]
@@ -234,9 +234,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     // rate: with a static split the slowest CTA finished 35 % after the fastest), then the warm tiles again
     // (with thresholds), then the end marker.  Rank 0's TMA producer draws the tiles and tells the MMA issuers and
     // the epilogues of both CTAs through bars->tile_of.
-    // bits 8..11 of the tune word override the number of warm tiles (A/B measurements)
-    const int warm_cap = ((tune >> 8) & 15) ? ((tune >> 8) & 15) : WARM_TILES;
-    const int warm = (tune & 2) ? 1 : max(1, min(warm_cap, n_tiles / C));
+    const int warm = max(1, min(WARM_TILES, n_tiles / C));
 
     for (int i = threadIdx.x; i < NQ_CTA; i += blockDim.x) {
         lmax_s[i] = INT_MIN;
@@ -419,14 +417,12 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
 #pragma unroll
             for (int hq = 0; hq < 2; ++hq) tg[hq] = active[hq] ? ld_relaxed(&Tg[qrow0 + hq * 128 + qd * 32 + lane]) : INT_MIN;
         };
-        auto apply_thresholds = [&](const int (&tg)[2], int i) -> bool {
+        auto apply_thresholds = [&](const int (&tg)[2]) -> bool {
             bool valid = true;
 #pragma unroll
             for (int hq = 0; hq < 2; ++hq) {
                 if (active[hq]) {
                     if (tg[hq] > thr_ord[hq]) {
-                        if (dbg_first && part == 0 && thr_ord[hq] == NEG_INF_ORD)
-                            dbg_first[cta * NQ_MAX + qrow0 + hq * 128 + qd * 32 + lane] = i;
                         thr_ord[hq] = tg[hq];
                         const float t = ord2f(tg[hq]);
                         t_exact[hq] = t;
@@ -449,17 +445,6 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 }
             }
         };
-        // developer probe (nq <= NQ_MAX - 8): ns since kernel start at which tile 0 / the threshold wait / the scan ended
-        const bool probe = dbg_first != nullptr && threadIdx.x == 0 && nq <= NQ_MAX - 8;
-        unsigned long long t_start = 0;
-        if (probe) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_start));
-        auto stamp = [&](int slot) {
-            if (probe) {
-                unsigned long long t;
-                asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-                dbg_first[cta * NQ_MAX + NQ_MAX - 8 + slot] = static_cast<int>(t - t_start);
-            }
-        };
         const uint32_t tlane = tmem_base + (static_cast<uint32_t>(qd * 32) << 16) + part * PART_COLS;
         uint32_t uc = 0;
 
@@ -472,7 +457,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             // rows of (numerically) equal norm, all searchable -- fingerprints are unit vectors --: the best score of a
             // chunk is its maximum minus the common 0.5|x|^2 (FMNMX3 chain).  Otherwise (reconstructions of an
             // IVF-PQ index, raw vectors, halo / padding rows): exact, column by column.
-            bool edge = (static_cast<uint32_t>(clu + w * C) + 1u) * SCAN_TILE > ns32 || (tune & 4);
+            bool edge = (static_cast<uint32_t>(clu + w * C) + 1u) * SCAN_TILE > ns32;
             float hx = 0.f;
             for (int hq = 0; hq < n_half; ++hq, ++uc) {
                 const int acc = uc & 1;
@@ -515,7 +500,6 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 mbar_arrive_lane0(&bars->tempty[acc], lane);
             }
             publish_maxima();
-            if (w == 0) stamp(0);
         }
         // ---- wait (bounded) for the thresholds of this warp's queries
         {
@@ -524,12 +508,11 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             for (int spin = 0; spin < 4096 && !ok; ++spin) {
                 publish_maxima();          // the other warps' tile-0 maxima of the queries this warp publishes
                 load_thresholds(tg);
-                ok = apply_thresholds(tg, 1);
+                ok = apply_thresholds(tg);
                 if (!ok) __nanosleep(100);
             }
             // not ok after ~0.5 ms: scan on with -inf thresholds; the pools overflow and the exact fallback
             // answers those queries
-            stamp(1);
         }
         // ---- the items the producer draws for this CTA, ending with the warm tiles again and the end marker
         for (int i = warm;; ++i) {
@@ -537,7 +520,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             // one refresh every four tiles: a coherent load takes ~2 us under the scan's own traffic -- longer than a
             // tile -- and after the warm tiles the thresholds move slowly (refreshing every tile cost 8 % of a
             // 7 M-row pass).  Loads issued now, consumed after the tile.
-            const bool rf = i > warm && (((tune & 8) && i < warm + 32) || (i & 3) == 0);
+            const bool rf = i > warm && (i & 3) == 0;
             if (rf) load_thresholds(tg);
             const float* h_part = h_s + (i % H_RING) * SCAN_TILE + part * PART_COLS;
             uint32_t row0 = 0;
@@ -559,7 +542,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                         __uint_as_float(__reduce_min_sync(0xffffffffu, __float_as_uint(fminf(h_part[lane], h_part[32 + lane]))));
                     hm = hmin_w * (1.f - 1.f / 1048576.f);
                     // the tile holds rows that do not take part in the search (halo, padding)
-                    edge = (static_cast<uint32_t>(tile) + 1u) * SCAN_TILE > ns32 || (tune & 4);
+                    edge = (static_cast<uint32_t>(tile) + 1u) * SCAN_TILE > ns32;
                 }
                 const float tp = (hq == 0 ? t_pre[0] : t_pre[1]) + hm;
                 tc_fence_after();
@@ -599,16 +582,10 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
                 mbar_arrive_lane0(&bars->tempty[acc], lane);
             }
             if (end) break;
-            if (rf) apply_thresholds(tg, i);
+            if (rf) apply_thresholds(tg);
             if (i < warm + 32 || (i & 3) == 0) publish_maxima();
-            if (i == warm) stamp(2);
-            if (i == 16) stamp(5);
-            if (i == 32) stamp(6);
-            if (i == 96) stamp(7);
         }
-        stamp(3);
         publish_maxima();
-        stamp(4);
         __syncwarp();
         // all epilogue warps are done appending before counts are published
         asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
@@ -653,8 +630,8 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             ++round;
             // the select competes with four epilogue warps for its sub-partition's issue slots: once the first
             // thresholds are out (a few rounds), one refresh every few tiles is as good as a continuous one
-            if ((tune & 1) || round < 6) {
-                __nanosleep((tune & 1) ? (round < 48 ? 100 : (round < 96 ? 1000 : 4000)) : 100);
+            if (round < 6) {
+                __nanosleep(100);
             } else {
                 for (int nap = 0; nap < 8 && smem_ld_volatile(&bars->done) < EPI_WARPS; ++nap) __nanosleep(500);   // prompt exit
             }
@@ -1093,14 +1070,6 @@ static int brute_rounds(nafp_index* idx, const float* q_dev, const int32_t* list
     return NAFP_OK;
 }
 
-// developer knob NAFP_SCAN_TUNE (A/B switches of flat_scan_kernel; every setting returns the same answers):
-// 1 = reducer polls continuously, 2 = one warm tile, 4 = exact per-column candidate path in every tile (the path
-// of tiles with halo / padding rows), 8 = thresholds re-read every tile during the first 32 tiles
-static int scan_tune() {
-    static const int v = [] { const char* e = getenv("NAFP_SCAN_TUNE"); return e ? atoi(e) : 0; }();
-    return v;
-}
-
 static int scan_pass(nafp_index* idx, const float* q_dev, const int32_t* src_list, int src_off, int64_t p0, int np, int kg,
                      int grid_scan, int n_tiles, int64_t n_search, int slot) {
     nafp_ctx* ctx = idx->ctx;
@@ -1121,14 +1090,12 @@ static int scan_pass(nafp_index* idx, const float* q_dev, const int32_t* src_lis
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t cfg = scan_launch_config(grid_scan, ctx->stream, attr);
     NAFP_CUDA(cudaLaunchKernelEx(&cfg, flat_scan_kernel, idx->tmap_q, idx->tmap_db, static_cast<const float*>(idx->hn),
-                                 idx->tile_counter, n_search, n_tiles, np, n_half, kg, idx->Mx, Tg, pool, cnt, flags,
-                                 idx->dbg_first, scan_tune()));
+                                 idx->tile_counter, n_search, n_tiles, np, n_half, kg, idx->Mx, Tg, pool, cnt, flags));
     if (prof) {
         cudaEventRecord(idx->prof_ev[2 * idx->prof_n + 1], ctx->stream);
         idx->prof_n++;
     }
     ctx->launches += 2;
-    idx->last_slot = slot;
     idx->last_h = n_half * 128;
     return NAFP_OK;
 }
@@ -1264,7 +1231,7 @@ int nafp_index_destroy(nafp_index* idx) {
     if (idx->ivf) ivfpq_destroy(idx);
     for (auto& e : idx->prof_ev) cudaEventDestroy(e);
     void* bufs[] = {idx->x32, idx->x16, idx->hn, idx->tile_counter, idx->maxn2, idx->qbf, idx->q32, idx->qn2, idx->Mx, idx->Tg,
-                    idx->pool, idx->cnt, idx->flags, idx->gidx, idx->fail_list, idx->brute_part, idx->stats, idx->dbg_first, idx->stage_q, idx->stage_D,
+                    idx->pool, idx->cnt, idx->flags, idx->gidx, idx->fail_list, idx->brute_part, idx->stats, idx->stage_q, idx->stage_D,
                     idx->stage_I};
     for (void* b : bufs)
         if (b) cudaFree(b);
@@ -1378,60 +1345,6 @@ int nafp_index_reconstruct_host(nafp_index* idx, int64_t i0, int64_t n, float* o
     NAFP_CUDA(cudaMemcpyAsync(out_host, idx->x32 + i0 * idx->d, static_cast<size_t>(n) * idx->d * sizeof(float),
                               cudaMemcpyDeviceToHost, idx->ctx->stream));
     NAFP_CUDA(cudaStreamSynchronize(idx->ctx->stream));
-    return NAFP_OK;
-}
-
-// survivor counts of pass row q of the last scan pass: [grid][NQ_MAX], 0 in the CTAs that do not hold row q
-static int last_pass_counts(nafp_index* idx, std::vector<int32_t>& by_row) {
-    const size_t n_cta = static_cast<size_t>(idx->grid) * NQ_CTA;
-    std::vector<int32_t> cnt(n_cta);
-    NAFP_CUDA(cudaMemcpy(cnt.data(), idx->cnt + idx->last_slot * n_cta, n_cta * 4, cudaMemcpyDeviceToHost));
-    by_row.assign(static_cast<size_t>(idx->grid) * NQ_MAX, 0);
-    for (int g = 0; g < idx->grid; ++g)
-        for (int ql = 0; ql < idx->last_h; ++ql) by_row[static_cast<size_t>(g) * NQ_MAX + (g & 1) * idx->last_h + ql] = cnt[g * NQ_CTA + ql];
-    return NAFP_OK;
-}
-
-int nafp_index_debug_enable(nafp_index* idx, int32_t* cnt_out, int32_t* first_out, int32_t* grid_out) {
-    // first call allocates the probe buffer; later calls copy cnt[grid][NQ_MAX] / first-threshold tile[grid][NQ_MAX]
-    NAFP_REQUIRE(idx && idx->scratch_ready, NAFP_ERR_STATE, "debug: search once first");
-    nafp_ctx* ctx = idx->ctx;
-    NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
-    const size_t n = static_cast<size_t>(idx->grid) * NQ_MAX;
-    if (!idx->dbg_first) {
-        NAFP_CUDA(cudaMalloc(&idx->dbg_first, n * 4));
-        NAFP_CUDA(cudaMemset(idx->dbg_first, 0xFF, n * 4));
-    }
-    if (grid_out) *grid_out = idx->grid;
-    if (cnt_out) {
-        std::vector<int32_t> by_row;
-        NAFP_TRY(last_pass_counts(idx, by_row));
-        memcpy(cnt_out, by_row.data(), n * 4);
-    }
-    if (first_out) {
-        NAFP_CUDA(cudaMemcpy(first_out, idx->dbg_first, n * 4, cudaMemcpyDeviceToHost));
-        NAFP_CUDA(cudaMemset(idx->dbg_first, 0xFF, n * 4));
-    }
-    return NAFP_OK;
-}
-
-// developer probe: state of the last scan pass (flags, shared thresholds as float, survivors per query row)
-int nafp_index_debug_last_pass(nafp_index* idx, int32_t* flags_out, float* thr_out, int32_t* total_out) {
-    NAFP_REQUIRE(idx && idx->scratch_ready && flags_out && thr_out && total_out, NAFP_ERR_INVALID, "debug: bad arguments");
-    nafp_ctx* ctx = idx->ctx;
-    NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
-    std::vector<int32_t> tg(NQ_MAX), cnt;
-    NAFP_CUDA(cudaMemcpy(flags_out, idx->flags + idx->last_slot * NQ_MAX, NQ_MAX * 4, cudaMemcpyDeviceToHost));
-    NAFP_CUDA(cudaMemcpy(tg.data(), idx->Tg + idx->last_slot * NQ_MAX, NQ_MAX * 4, cudaMemcpyDeviceToHost));
-    NAFP_TRY(last_pass_counts(idx, cnt));
-    for (int q = 0; q < NQ_MAX; ++q) {
-        int32_t o = tg[q];
-        uint32_t b = static_cast<uint32_t>(o >= 0 ? o : (o ^ 0x7FFFFFFF));
-        memcpy(&thr_out[q], &b, 4);
-        int64_t t = 0;
-        for (int g = 0; g < idx->grid; ++g) t += cnt[static_cast<size_t>(g) * NQ_MAX + q];
-        total_out[q] = static_cast<int32_t>(t);
-    }
     return NAFP_OK;
 }
 

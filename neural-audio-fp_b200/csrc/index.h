@@ -17,8 +17,8 @@ constexpr int POOL_CAP = 128;        // candidate slots per (CTA, query) per pas
 constexpr int MAX_K = 128;
 constexpr int BRUTE_CHUNKS = 296;        // CTAs per query of the exact fallback scan (2 per SM)
 constexpr int BRUTE_SLOTS = 32;          // queries per fallback launch
-constexpr int SELECT_CAP = 4096;
-constexpr int SEL_SLOTS = 16;        // scan passes whose survivors are re-ranked by ONE flat_select launch     // candidates re-ranked in fp32 per query, at most
+constexpr int SELECT_CAP = 4096;     // candidates re-ranked in fp32 per query, at most
+constexpr int SEL_SLOTS = 16;        // scan passes whose survivors are re-ranked by ONE flat_select launch
 
 struct IvfPq;                        // ivfpq.cu
 
@@ -42,7 +42,6 @@ struct nafp_index {
     bool tmap_db_valid = false;
 
     // per-pass scratch (allocated on first search); q32 .. gidx hold SEL_SLOTS passes
-    int last_slot = 0;
     int last_h = 0;                   // query rows per CTA of the last scan pass
     bool scratch_ready = false;
     int grid = 0;                     // scan CTAs: 2 x the CTA pairs that fit on the device at once
@@ -60,7 +59,6 @@ struct nafp_index {
     uint64_t* brute_part = nullptr;   // [BRUTE_SLOTS][BRUTE_CHUNKS][MAX_K]
     unsigned long long* stats = nullptr;   // [8] device counters
     int32_t* tile_counter = nullptr;  // device scalar: next DB tile the scan's producers draw
-    int32_t* dbg_first = nullptr;     // developer probe: [grid][NQ_MAX] tile index of the first shared threshold
     // staging for the host entry points
     float* stage_q = nullptr;  int64_t stage_q_rows = 0;
     float* stage_D = nullptr;  int64_t* stage_I = nullptr;  int64_t stage_out_elems = 0;

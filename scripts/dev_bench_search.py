@@ -27,13 +27,3 @@ for nq in (19, 64, 128, 247, 256, 512, 1024):
     print(f"N={N} nq={nq}: {ms*1e3:.1f} us/search  scan-bytes {N*256*passes/ms/1e6:.0f} GB/s-equivalent  "
           f"{nq/ms*1e3:.0f} rows/s  {2*nq*N*128/ms/1e9:.1f} TFLOP/s stats/rep={ {k: v/reps for k, v in st.items()} }")
 
-from nafp_b200._lib import lib, check, ptr
-for nq in (19, 256, 512):
-    q = np.concatenate([query[i * 59: i * 59 + 19] for i in range(60)])[:nq]
-    D, I = idx.search(q, 20)
-    fl = np.zeros(512, np.int32); th = np.zeros(512, np.float32); tot = np.zeros(512, np.int32)
-    check(lib.nafp_index_debug_last_pass(idx.h, ptr(fl), ptr(th), ptr(tot)))
-    print("nq", nq, "flags", fl[:nq].tolist())
-    print("thr", np.round(th[:nq], 3).tolist()[:64])
-    print("tot", tot[:nq].tolist()[:64])
-    print("s20", np.round(0.5 - 0.5 * D[:nq, 19] - 0.0, 3).tolist()[:64])
