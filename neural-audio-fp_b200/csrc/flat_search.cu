@@ -36,6 +36,7 @@
 
 #include "index.h"
 #include "ptx.cuh"
+#include "topk.cuh"
 
 namespace nafp {
 
@@ -646,34 +647,6 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
 // ------------------------------------------------------------------------------------------
 // survivors -> exact fp32 re-rank + proof
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint64_t score_key(float s, uint32_t row) {
-    return (static_cast<uint64_t>(static_cast<uint32_t>(f2ord(s)) ^ 0x80000000u) << 32) | (0xFFFFFFFFu - row);
-}
-__device__ __forceinline__ float key_score(uint64_t key) {
-    return ord2f(static_cast<int>(static_cast<uint32_t>(key >> 32) ^ 0x80000000u));
-}
-__device__ __forceinline__ uint32_t key_row(uint64_t key) { return 0xFFFFFFFFu - static_cast<uint32_t>(key); }
-
-// descending bitonic sort of n (power of two) keys in shared memory
-__device__ void bitonic_sort_desc(uint64_t* keys, int n) {
-    for (int k = 2; k <= n; k <<= 1) {
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int i = threadIdx.x; i < n; i += blockDim.x) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const uint64_t a = keys[i], b = keys[ixj];
-                    const bool desc = (i & k) == 0;
-                    if (desc ? (a < b) : (a > b)) {
-                        keys[i] = b;
-                        keys[ixj] = a;
-                    }
-                }
-            }
-            __syncthreads();
-        }
-    }
-}
-
 struct SelBatch {
     int np[SEL_SLOTS];       // query rows of the pass held in every slot
     int h[SEL_SLOTS];        // query rows per CTA of that pass: row q is local row q % h of the CTAs of rank q / h
@@ -776,7 +749,7 @@ flat_select_kernel(SelBatch batch, int k, int grid_scan, int64_t n_rows, const f
     __syncthreads();
     for (int i = total + threadIdx.x; i < npow; i += blockDim.x) keys[i] = 0;
     __syncthreads();
-    bitonic_sort_desc(keys, npow);
+    block_sort_u64<false>(keys, npow);
     // proof: every row that is not a survivor has bf16 score <= T, hence exact score <= T + eps
     const int tgo = Tg[q];
     if (tgo > NEG_INF_ORD) {
@@ -854,13 +827,8 @@ flat_brute_scan_kernel(int k, int64_t n_rows, const float* __restrict__ q_all, c
         uint64_t* out = part + (static_cast<int64_t>(e) * BRUTE_CHUNKS + chunk) * MAX_K;
         int head = 0;     // lane w < 8 owns the read cursor of list w
         for (int j = 0; j < k; ++j) {
-            uint64_t cand = (lane < 8 && head < k) ? lists[lane][head] : 0;
-            uint64_t best = cand;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const uint64_t other = __shfl_xor_sync(0xffffffffu, best, o);
-                best = other > best ? other : best;
-            }
+            const uint64_t cand = (lane < 8 && head < k) ? lists[lane][head] : 0;
+            const uint64_t best = warp_max_u64(cand);
             if (lane < 8 && cand == best && best != 0) ++head;   // keys are unique (row id inside)
             if (lane == 0) out[j] = best;
         }
@@ -872,7 +840,6 @@ flat_brute_merge_kernel(int k, const float* __restrict__ q_all, const int32_t* _
                         uint64_t* __restrict__ part, int64_t label_offset, float* __restrict__ D,
                         int64_t* __restrict__ I, unsigned long long* __restrict__ stats) {
     __shared__ uint64_t red[8];
-    __shared__ uint64_t winner;
     __shared__ float qn2_s;
     const int e = blockIdx.x;
     const int64_t g = list ? static_cast<int64_t>(list[list_off + e]) : list_off + e;
@@ -892,27 +859,16 @@ flat_brute_merge_kernel(int k, const float* __restrict__ q_all, const int32_t* _
             const uint64_t v = p[(c / k) * MAX_K + (c % k)];
             best = v > best ? v : best;
         }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const uint64_t other = __shfl_xor_sync(0xffffffffu, best, o);
-            best = other > best ? other : best;
-        }
-        if (lane == 0) red[warp] = best;
-        __syncthreads();
+        const uint64_t w = block_max_u64(best, red);
         if (threadIdx.x == 0) {
-            uint64_t b = 0;
-            for (int w = 0; w < 8; ++w) b = red[w] > b ? red[w] : b;
-            winner = b;
-            if (b != 0) {
-                D[g * k + j] = fmaxf(qn2_s - 2.f * key_score(b), 0.f);
-                I[g * k + j] = static_cast<int64_t>(key_row(b)) + label_offset;
+            if (w != 0) {
+                D[g * k + j] = fmaxf(qn2_s - 2.f * key_score(w), 0.f);
+                I[g * k + j] = static_cast<int64_t>(key_row(w)) + label_offset;
             } else {
                 D[g * k + j] = INFINITY;
                 I[g * k + j] = -1;
             }
         }
-        __syncthreads();
-        const uint64_t w = winner;
         if (w != 0)
             for (int c = threadIdx.x; c < BRUTE_CHUNKS * k; c += blockDim.x) {
                 uint64_t* slot = &p[(c / k) * MAX_K + (c % k)];

@@ -4,12 +4,13 @@
 //
 //   train   k-means (Lloyd, 25 iterations, <= 256 points per centroid, seeded) for the coarse
 //           quantizer, then one k-means per sub-space on the residuals; deterministic (fixed-order sums)
-//   add     ivfpq_encode_kernel: nearest coarse centroid + 64 one-byte codes per row; the inverted
-//           lists are a stable counting sort of (list, row) rebuilt lazily before the next search
+//   add     coarse_probe with nprobe = 1 (the nearest coarse centroid), then 64 one-byte codes per row
+//           (ivfpq_encode_kernel); the inverted lists are a stable counting sort of (list, row) rebuilt lazily
+//           before the next search
 //   search  by default the list-major tensor-core scan of the compressed lists (ivfpq_lm.cu).  The LUT kernel
 //           below is the reference formulation: it answers the query rows and shapes the list-major scan cannot
 //           (and every search of an index created with NAFP_IVFPQ_PATH=lut):
-//           ivfpq_probe_kernel (nprobe nearest lists per query row) ->
+//           coarse_probe       (nprobe nearest lists per query row) ->
 //           ivfpq_scan_kernel  (one CTA per (query row, probed list): 64 x 256 fp32 look-up table in
 //                               shared memory, ADC scan of the list's codes, block top-k) ->
 //           topk merge of the nprobe partial lists.
@@ -29,6 +30,7 @@
 
 #include "ivfpq.h"
 #include "ptx.cuh"
+#include "topk.cuh"
 
 namespace nafp {
 
@@ -56,12 +58,7 @@ __global__ void kmeans_assign_kernel(const float* __restrict__ x, int64_t n, int
         }
         if (d < best) { best = d; bi = c; }
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-    }
+    warp_argmin(best, bi);
     if (lane == 0) {
         assign[i] = bi;
         if (dist_out) dist_out[i] = best;
@@ -165,10 +162,10 @@ static int run_kmeans(nafp_ctx* ctx, const float* x_dev, int64_t n, int ld, int 
 }
 
 // ------------------------------------------------------------------------------------------ add
-// one warp per row: nearest coarse centroid, residual, then lane l encodes sub-spaces l and l + 32
+// one warp per row: the residual against the row's list, then lane l encodes sub-spaces l and l + 32
 __global__ void __launch_bounds__(256)
 ivfpq_encode_kernel(const float* __restrict__ x32, int64_t row0, int64_t n, const float* __restrict__ coarse,
-                    int nlist, const float* __restrict__ pq, int m, int dsub, int32_t* __restrict__ assign,
+                    const int32_t* __restrict__ assign, const float* __restrict__ pq, int m, int dsub,
                     uint8_t* __restrict__ codes) {
     __shared__ float xs[8][D128];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -176,35 +173,10 @@ ivfpq_encode_kernel(const float* __restrict__ x32, int64_t row0, int64_t n, cons
     for (int64_t r = ((static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5); r < n; r += nwarps) {
         const int64_t row = row0 + r;
         float* xr = xs[w];
-        reinterpret_cast<float4*>(xr)[lane] = reinterpret_cast<const float4*>(x32 + row * D128)[lane];
-        __syncwarp();
-        float best = FLT_MAX;
-        int bi = INT_MAX;
-        for (int c = lane; c < nlist; c += 32) {
-            const float* cr = coarse + static_cast<int64_t>(c) * D128;
-            float d = 0.f;
-#pragma unroll 8
-            for (int j = 0; j < D128; ++j) {
-                const float t = xr[j] - __ldg(cr + j);
-                d += t * t;
-            }
-            if (d < best) { best = d; bi = c; }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-        }
-        if (lane == 0) assign[row] = bi;
-        // residual in place
-        {
-            const float4 cv = reinterpret_cast<const float4*>(coarse + static_cast<int64_t>(bi) * D128)[lane];
-            float4 v = reinterpret_cast<float4*>(xr)[lane];
-            v.x -= cv.x; v.y -= cv.y; v.z -= cv.z; v.w -= cv.w;
-            __syncwarp();
-            reinterpret_cast<float4*>(xr)[lane] = v;
-        }
+        const float4 cv = reinterpret_cast<const float4*>(coarse + static_cast<int64_t>(assign[row]) * D128)[lane];
+        float4 v = reinterpret_cast<const float4*>(x32 + row * D128)[lane];
+        v.x -= cv.x; v.y -= cv.y; v.z -= cv.z; v.w -= cv.w;
+        reinterpret_cast<float4*>(xr)[lane] = v;
         __syncwarp();
         for (int sub = lane; sub < m; sub += 32) {
             const float* pc = pq + static_cast<int64_t>(sub) * PQ_KSUB * dsub;
@@ -224,56 +196,10 @@ ivfpq_encode_kernel(const float* __restrict__ x32, int64_t row0, int64_t n, cons
     }
 }
 
-// The same two steps for the reference's shape (nlist <= 256, M = 64, dsub = 2) with the tables in shared memory: the
-// 56 M-row build spent 13.5 s in the kernel above, whose 128 KB codebook thrashes L1.  Arithmetic and tie-breaking are
-// the kernel's above (fma chains, dimensions ascending, first minimum wins), so assignments and codes are identical.
-constexpr int ENC_NLIST = 256;
-constexpr int ENC_ASSIGN_SMEM = (D128 * ENC_NLIST + 8 * D128) * 4;          // transposed centroids + 8 rows
+// The same for the reference's shape (M = 64, dsub = 2) with the codebooks in shared memory: the 56 M-row build spent
+// 13.5 s in the kernel above, whose 128 KB codebook thrashes L1.  Arithmetic and tie-breaking are the kernel's above
+// (fma chains, first minimum wins), so the codes are identical.
 constexpr int ENC_CODE_SMEM = PQ_KSUB * 64 * 8 + 8 * D128 * 4;              // [code][sub] float2 + 8 residual rows
-__global__ void __launch_bounds__(256)
-ivfpq_assign_smem_kernel(const float* __restrict__ x32, int64_t row0, int64_t n, const float* __restrict__ coarse, int nlist,
-                         int32_t* __restrict__ assign) {
-    extern __shared__ float esm[];
-    float* cs = esm;                                   // [dim][256 centroids]
-    float* xs = esm + D128 * ENC_NLIST;                // [8 warps][128]
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int e = threadIdx.x; e < D128 * ENC_NLIST; e += blockDim.x) {
-        const int j = e / ENC_NLIST, c = e % ENC_NLIST;
-        cs[e] = c < nlist ? __ldg(coarse + static_cast<int64_t>(c) * D128 + j) : 0.f;
-    }
-    __syncthreads();
-    float* xr = xs + w * D128;
-    for (int64_t r = static_cast<int64_t>(blockIdx.x) * 8 + w; r < n; r += static_cast<int64_t>(gridDim.x) * 8) {
-        __syncwarp();
-        reinterpret_cast<float4*>(xr)[lane] = reinterpret_cast<const float4*>(x32 + (row0 + r) * D128)[lane];
-        __syncwarp();
-        float d[ENC_NLIST / 32];
-#pragma unroll
-        for (int t = 0; t < ENC_NLIST / 32; ++t) d[t] = 0.f;
-#pragma unroll 4
-        for (int j = 0; j < D128; ++j) {
-            const float xj = xr[j];
-            const float* cr = cs + j * ENC_NLIST + lane;
-#pragma unroll
-            for (int t = 0; t < ENC_NLIST / 32; ++t) {
-                const float v = xj - cr[32 * t];
-                d[t] = fmaf(v, v, d[t]);
-            }
-        }
-        float best = FLT_MAX;
-        int bi = INT_MAX;
-#pragma unroll
-        for (int t = 0; t < ENC_NLIST / 32; ++t)              // centroid lane + 32 t, ascending: the first minimum wins
-            if (lane + 32 * t < nlist && d[t] < best) { best = d[t]; bi = lane + 32 * t; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-        }
-        if (lane == 0) assign[row0 + r] = bi;
-    }
-}
 __global__ void __launch_bounds__(256)
 ivfpq_code_smem_kernel(const float* __restrict__ x32, int64_t row0, int64_t n, const float* __restrict__ coarse,
                        const float* __restrict__ pq, const int32_t* __restrict__ assign, uint8_t* __restrict__ codes) {
@@ -377,15 +303,59 @@ __global__ void ivf_unscatter_kernel(const uint8_t* __restrict__ lcodes, const i
     for (int sub = 0; sub < m; ++sub) codes[static_cast<int64_t>(row) * m + sub] = lcodes[lcode_off(pos, sub, m)];
 }
 
-// ------------------------------------------------------------------------------------------ search
-// one warp per query row: the nprobe nearest coarse centroids, ascending (ties -> lower list id)
-__global__ void ivfpq_probe_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse,
-                                   int nlist, int nprobe, int32_t* __restrict__ probes) {
+// ------------------------------------------------------------------------------------------ coarse probe
+// One warp per row: the nprobe nearest coarse centroids of a 128-d row, ascending, ties to the lower list id.  Every
+// search path and `add` (nprobe = 1) use these two kernels, so that a stored row lies in the list its own copy probes
+// first, and the list-major scan, the LUT scan and IVF-Flat visit the same lists.  A centroid distance is one
+// fma(v, v, acc) chain over ascending dimensions, starting from 0 (the oracle's k-means, oracle.c, rounds identically).
+// Optional outputs, null when unused: gdist[nq][nprobe] the centroid distances, qE[nq] the rounding bound of the row's
+// bf16 scores in the list-major scan (dmax2: bits of max |d|^2 of the index).
+
+// lane owns centroids lane + 32 t (d[t] = FLT_MAX past nlist); nprobe rounds of arg-min, the winner leaves
+template <int NT>
+__device__ __forceinline__ void probe_rounds(float (&d)[NT], int lane, int64_t i, int nprobe, int32_t* __restrict__ probes,
+                                             float* __restrict__ gdist) {
+    probes += i * nprobe;
+    if (gdist) gdist += i * nprobe;
+    for (int p = 0; p < nprobe; ++p) {
+        float best = FLT_MAX;
+        int bi = INT_MAX;
+#pragma unroll
+        for (int t = 0; t < NT; ++t)
+            if (d[t] < best) { best = d[t]; bi = lane + 32 * t; }
+        warp_argmin(best, bi);
+        if (lane == 0) {
+            probes[p] = bi == INT_MAX ? -1 : bi;
+            if (gdist) gdist[p] = best;
+        }
+#pragma unroll
+        for (int t = 0; t < NT; ++t)
+            if (lane + 32 * t == bi) d[t] = FLT_MAX;
+    }
+}
+// |sum bf(q_i) bf(d_i) - sum q_i d_i| <= |q| |d| (2^-8 + 2^-18) for round-to-nearest bf16 operands; 3 % on top for the
+// norms' own rounding and the tensor core's fp32 accumulation (<= 128 * 2^-23 relative).  dm = max |d|.
+__device__ __forceinline__ float probe_score_bound(float4 qv, float dm) {
+    float qq = qv.x * qv.x + qv.y * qv.y + qv.z * qv.z + qv.w * qv.w;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(0xffffffffu, qq, o);
+    return sqrtf(qq) * dm * (1.03f / 256.f) + 1e-7f;
+}
+
+// centroids read from global memory: any nlist <= IVF_MAX_NLIST
+__global__ void coarse_probe_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse, int nlist, int nprobe,
+                                    const int32_t* __restrict__ dmax2, int32_t* __restrict__ probes, float* __restrict__ gdist,
+                                    float* __restrict__ qE) {
     __shared__ float qs[8][D128];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
     if (i >= nq) return;
-    reinterpret_cast<float4*>(qs[w])[lane] = reinterpret_cast<const float4*>(q + i * D128)[lane];
+    const float4 qv = reinterpret_cast<const float4*>(q + i * D128)[lane];
+    reinterpret_cast<float4*>(qs[w])[lane] = qv;
+    if (qE) {
+        const float e = probe_score_bound(qv, sqrtf(__int_as_float(*dmax2)));
+        if (lane == 0) qE[i] = e;
+    }
     __syncwarp();
     float d[IVF_MAX_NLIST / 32];
 #pragma unroll
@@ -402,25 +372,74 @@ __global__ void ivfpq_probe_kernel(const float* __restrict__ q, int64_t nq, cons
         }
         d[t] = acc;
     }
-    for (int p = 0; p < nprobe; ++p) {
-        float best = FLT_MAX;
-        int bi = INT_MAX;
-#pragma unroll
-        for (int t = 0; t < IVF_MAX_NLIST / 32; ++t)
-            if (d[t] < best) { best = d[t]; bi = lane + 32 * t; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
+    probe_rounds(d, lane, i, nprobe, probes, gdist);
+}
+
+// nlist <= 256 with the centroids transposed in shared memory (128 KB, loaded once per block; the block then walks over
+// its share of the rows): lane l owns centroids l, l + 32, ...; conflict-free reads.  12x the kernel above at 22 k rows
+// (2.7 ms -> 0.2 ms).
+constexpr int PROBE_SMEM_NLIST = 256;
+constexpr int PROBE_SMEM = (D128 * PROBE_SMEM_NLIST + 8 * D128) * 4;
+__global__ void __launch_bounds__(256)
+coarse_probe_smem_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse, int nlist, int nprobe,
+                         const int32_t* __restrict__ dmax2, int32_t* __restrict__ probes, float* __restrict__ gdist,
+                         float* __restrict__ qE) {
+    extern __shared__ float psm[];
+    float* cs = psm;                                   // [dim][256 centroids]
+    float* qs = psm + D128 * PROBE_SMEM_NLIST;         // [8 warps][128]
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    for (int e = threadIdx.x; e < D128 * PROBE_SMEM_NLIST; e += blockDim.x) {
+        const int j = e / PROBE_SMEM_NLIST, c = e % PROBE_SMEM_NLIST;
+        cs[e] = c < nlist ? __ldg(coarse + static_cast<int64_t>(c) * D128 + j) : 0.f;
+    }
+    __syncthreads();
+    const float dm = qE ? sqrtf(__int_as_float(*dmax2)) : 0.f;
+    float* qr = qs + w * D128;
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * 8 + w; i < nq; i += static_cast<int64_t>(gridDim.x) * 8) {
+        const float4 qv = reinterpret_cast<const float4*>(q + i * D128)[lane];
+        __syncwarp();
+        reinterpret_cast<float4*>(qr)[lane] = qv;
+        if (qE) {
+            const float e = probe_score_bound(qv, dm);
+            if (lane == 0) qE[i] = e;
         }
-        if (lane == 0) probes[i * nprobe + p] = bi == INT_MAX ? -1 : bi;
+        __syncwarp();
+        float d[PROBE_SMEM_NLIST / 32];
 #pragma unroll
-        for (int t = 0; t < IVF_MAX_NLIST / 32; ++t)
-            if (lane + 32 * t == bi) d[t] = FLT_MAX;
+        for (int t = 0; t < PROBE_SMEM_NLIST / 32; ++t) d[t] = 0.f;
+#pragma unroll 4
+        for (int j = 0; j < D128; ++j) {
+            const float qj = qr[j];
+            const float* cr = cs + j * PROBE_SMEM_NLIST + lane;
+#pragma unroll
+            for (int t = 0; t < PROBE_SMEM_NLIST / 32; ++t) {
+                const float v = qj - cr[32 * t];
+                d[t] = fmaf(v, v, d[t]);
+            }
+        }
+#pragma unroll
+        for (int t = 0; t < PROBE_SMEM_NLIST / 32; ++t)
+            if (lane + 32 * t >= nlist) d[t] = FLT_MAX;
+        probe_rounds(d, lane, i, nprobe, probes, gdist);
     }
 }
 
+int coarse_probe(nafp_ctx* ctx, const float* q, int64_t nq, const float* coarse, int nlist, int nprobe, int32_t* probes,
+                 float* gdist, float* qE, const int32_t* dmax2) {
+    if (nq == 0) return NAFP_OK;
+    if (nlist <= PROBE_SMEM_NLIST) {
+        NAFP_CUDA(cudaFuncSetAttribute(coarse_probe_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PROBE_SMEM));
+        coarse_probe_smem_kernel<<<static_cast<unsigned>(std::min<int64_t>((nq + 7) / 8, ctx->sm_count)), 256, PROBE_SMEM, ctx->stream>>>(
+            q, nq, coarse, nlist, nprobe, dmax2, probes, gdist, qE);
+    } else {
+        coarse_probe_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, ctx->stream>>>(q, nq, coarse, nlist, nprobe, dmax2, probes,
+                                                                                       gdist, qE);
+    }
+    ctx->launches++;
+    return NAFP_OK;
+}
+
+// ------------------------------------------------------------------------------------------ search
 // CTA (probe p, query row i): LUT T[m][c] = |(q - c_l)_m - pq_m[c]|^2 in shared memory, ADC scan of list l
 __global__ void __launch_bounds__(256)
 ivfpq_scan_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse,
@@ -476,7 +495,7 @@ ivfpq_scan_kernel(const float* __restrict__ q, int64_t nq, const float* __restri
                     for (int b = 0; b < 4; ++b) d += lut[(kb * mlo + 4 * v + b) * PQ_KSUB + ((wds[b] >> sh) & 255u)];
                 }
             }
-            const uint64_t key = (static_cast<uint64_t>(__float_as_uint(d)) << 32) | static_cast<uint32_t>(lids[pos]);
+            const uint64_t key = dist_key(d, static_cast<uint32_t>(lids[pos]));
             if (key < thr_s) {
                 const int slot = atomicAdd(&cnt_s, 1);
                 buf[slot] = key;         // slot < CAP: the buffer is pruned whenever fewer than 256 slots remain
@@ -488,23 +507,14 @@ ivfpq_scan_kernel(const float* __restrict__ q, int64_t nq, const float* __restri
         const int filled = cnt_s;
         __syncthreads();
         if (filled > IVF_SCAN_CAP - 256) {
-            block_sort_asc_u64(buf, IVF_SCAN_CAP);
+            block_sort_u64<true>(buf, IVF_SCAN_CAP);
             for (int e = k + tid; e < IVF_SCAN_CAP; e += blockDim.x) buf[e] = ~0ull;
             if (tid == 0) { cnt_s = k; thr_s = buf[k - 1]; }
             __syncthreads();
         }
     }
-    block_sort_asc_u64(buf, IVF_SCAN_CAP);
-    for (int j = tid; j < k; j += blockDim.x) {
-        const uint64_t key = buf[j];
-        if (key != ~0ull) {
-            outD[j] = __uint_as_float(static_cast<uint32_t>(key >> 32));
-            outI[j] = static_cast<int64_t>(static_cast<uint32_t>(key)) + label_offset;
-        } else {
-            outD[j] = INFINITY;
-            outI[j] = -1;
-        }
-    }
+    block_sort_u64<true>(buf, IVF_SCAN_CAP);
+    store_topk(buf, k, label_offset, outD, outI);
 }
 
 // IVF-Flat: CTA (probe p, query row i) scans the stored rows of list l exactly (fp32), a warp per row
@@ -543,7 +553,7 @@ ivfflat_scan_kernel(const float* __restrict__ q, int64_t nq, const int32_t* __re
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
                 if (lane == 0) {
-                    const uint64_t key = (static_cast<uint64_t>(__float_as_uint(d)) << 32) | static_cast<uint32_t>(row);
+                    const uint64_t key = dist_key(d, static_cast<uint32_t>(row));
                     if (key < thr_s) buf[atomicAdd(&cnt_s, 1)] = key;      // slot < CAP: pruned below before it can fill
                 }
             }
@@ -552,23 +562,14 @@ ivfflat_scan_kernel(const float* __restrict__ q, int64_t nq, const int32_t* __re
         const int filled = cnt_s;           // block-uniform (see ivfpq_scan_kernel)
         __syncthreads();
         if (filled > IVF_SCAN_CAP - 8 * ROWS_PER_WARP) {
-            block_sort_asc_u64(buf, IVF_SCAN_CAP);
+            block_sort_u64<true>(buf, IVF_SCAN_CAP);
             for (int e = k + tid; e < IVF_SCAN_CAP; e += blockDim.x) buf[e] = ~0ull;
             if (tid == 0) { cnt_s = k; thr_s = buf[k - 1]; }
             __syncthreads();
         }
     }
-    block_sort_asc_u64(buf, IVF_SCAN_CAP);
-    for (int j = tid; j < k; j += blockDim.x) {
-        const uint64_t key = buf[j];
-        if (key != ~0ull) {
-            outD[j] = __uint_as_float(static_cast<uint32_t>(key >> 32));
-            outI[j] = static_cast<int64_t>(static_cast<uint32_t>(key)) + label_offset;
-        } else {
-            outD[j] = INFINITY;
-            outI[j] = -1;
-        }
-    }
+    block_sort_u64<true>(buf, IVF_SCAN_CAP);
+    store_topk(buf, k, label_offset, outD, outI);
 }
 
 // IVF-Flat, one warp per query row: keep the flat scan's candidates whose list is probed, in order.  k of them (or
@@ -610,12 +611,6 @@ __global__ void ivfpq_filter_kernel(const float* __restrict__ candD, const int64
     if (lane == 0) redo_rows[atomicAdd(redo_count, 1)] = static_cast<int32_t>(q);
 }
 
-__global__ void ivfpq_gather_q_kernel(const float* __restrict__ q, const int32_t* __restrict__ rows, int64_t n, float* __restrict__ out) {
-    const int lane = threadIdx.x & 31;
-    const int64_t w = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-    if (w >= n) return;
-    reinterpret_cast<float4*>(out + w * D128)[lane] = reinterpret_cast<const float4*>(q + static_cast<int64_t>(rows[w]) * D128)[lane];
-}
 __global__ void ivfpq_scatter_kernel(const float* __restrict__ Ds, const int64_t* __restrict__ Is, const int32_t* __restrict__ rows,
                                      int64_t n, int k, float* __restrict__ D, int64_t* __restrict__ I) {
     const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -728,22 +723,7 @@ ivfpqr_rerank_kernel(const float* __restrict__ q, const int64_t* __restrict__ ca
         if (lane == 0) { d_s[c] = d; i_s[c] = id; }
     }
     __syncthreads();
-    for (int kk = 2; kk <= 128; kk <<= 1) {
-        for (int j = kk >> 1; j > 0; j >>= 1) {
-            const int i = threadIdx.x, ixj = i ^ j;
-            if (ixj > i) {
-                const float da = d_s[i], db = d_s[ixj];
-                const int64_t ia = i_s[i], ib = i_s[ixj];
-                const bool a_after_b = (da > db) || (da == db && ia > ib);
-                const bool asc = (i & kk) == 0;
-                if (asc ? a_after_b : !a_after_b) {
-                    d_s[i] = db; d_s[ixj] = da;
-                    i_s[i] = ib; i_s[ixj] = ia;
-                }
-            }
-            __syncthreads();
-        }
-    }
+    block_sort_dist_label(d_s, i_s, 128);
     for (int j = threadIdx.x; j < k; j += blockDim.x) {
         const int64_t id = i_s[j];
         D[qi * k + j] = id == LLONG_MAX ? INFINITY : d_s[j];
@@ -896,30 +876,22 @@ int ivfpq_add_rows(nafp_index* idx, int64_t row0, int64_t n) {
         s->codes = c;
         s->cap = idx->cap;
     }
-    if (s->flat_lists) {               // list of every new row = its nearest coarse centroid (ties -> lower id)
-        kmeans_assign_kernel<<<static_cast<unsigned>((n + 7) / 8), 256, 8 * D128 * sizeof(float), ctx->stream>>>(
-            idx->x32 + row0 * D128, n, D128, D128, s->coarse, s->nlist, s->assign + row0, nullptr);
+    // list of every new row = its nearest coarse centroid, as a search probes it
+    NAFP_TRY(coarse_probe(ctx, idx->x32 + row0 * D128, n, s->coarse, s->nlist, 1, s->assign + row0));
+    if (!s->flat_lists) {
+        int64_t blocks = (n + 7) / 8;
+        if (s->m == 64 && s->dsub == 2) {
+            if (blocks > ctx->sm_count) blocks = ctx->sm_count;          // one block per SM: each loads its table once
+            NAFP_CUDA(cudaFuncSetAttribute(ivfpq_code_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ENC_CODE_SMEM));
+            ivfpq_code_smem_kernel<<<static_cast<unsigned>(blocks), 256, ENC_CODE_SMEM, ctx->stream>>>(idx->x32, row0, n, s->coarse,
+                                                                                                     s->pq, s->assign, s->codes);
+        } else {
+            if (blocks > ctx->sm_count * 8) blocks = ctx->sm_count * 8;
+            ivfpq_encode_kernel<<<static_cast<unsigned>(blocks), 256, 0, ctx->stream>>>(idx->x32, row0, n, s->coarse, s->assign, s->pq,
+                                                                                      s->m, s->dsub, s->codes);
+        }
         ctx->launches++;
-        NAFP_CUDA(cudaGetLastError());
-        s->dirty = true;
-        return NAFP_OK;
     }
-    int64_t blocks = (n + 7) / 8;
-    if (s->nlist <= ENC_NLIST && s->m == 64 && s->dsub == 2) {
-        if (blocks > ctx->sm_count) blocks = ctx->sm_count;          // one block per SM: each loads its table once
-        NAFP_CUDA(cudaFuncSetAttribute(ivfpq_assign_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ENC_ASSIGN_SMEM));
-        NAFP_CUDA(cudaFuncSetAttribute(ivfpq_code_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ENC_CODE_SMEM));
-        ivfpq_assign_smem_kernel<<<static_cast<unsigned>(blocks), 256, ENC_ASSIGN_SMEM, ctx->stream>>>(idx->x32, row0, n, s->coarse,
-                                                                                                     s->nlist, s->assign);
-        ivfpq_code_smem_kernel<<<static_cast<unsigned>(blocks), 256, ENC_CODE_SMEM, ctx->stream>>>(idx->x32, row0, n, s->coarse, s->pq,
-                                                                                                 s->assign, s->codes);
-        ctx->launches++;
-    } else {
-        if (blocks > ctx->sm_count * 8) blocks = ctx->sm_count * 8;
-        ivfpq_encode_kernel<<<static_cast<unsigned>(blocks), 256, 0, ctx->stream>>>(idx->x32, row0, n, s->coarse, s->nlist, s->pq,
-                                                                                  s->m, s->dsub, s->assign, s->codes);
-    }
-    ctx->launches++;
     if (s->refine) {
         ivfpqr_encode_kernel<<<static_cast<unsigned>((n * 32 + 255) / 256), 256, 0, ctx->stream>>>(
             idx->x32, s->assign, s->codes, row0, n, s->coarse, s->pq, s->m, s->dsub, s->rpq, s->rcodes);
@@ -995,11 +967,8 @@ int build_lists(nafp_index* idx) {
     return NAFP_OK;
 }
 
-__global__ void topk_merge_kernel(const float* __restrict__ D_all, const int64_t* __restrict__ I_all, int W, int64_t nq,
-                                  int k, float* __restrict__ D_out, int64_t* __restrict__ I_out);
-constexpr int TOPK_MERGE_KEYS = 4096;     // keys one topk_merge_kernel block sorts (seq_match.cu)
 // merge blocks per query row of the LUT scan: 1 when the nprobe * k partial keys fit one block, else the number of
-// groups of floor(4096 / k) probes merged in a first round
+// groups of floor(TOPK_MERGE_KEYS / k) probes merged in a first round
 static int lut_merge_groups(int nprobe, int k) {
     if (nprobe * k <= TOPK_MERGE_KEYS) return 1;
     const int G = TOPK_MERGE_KEYS / k;
@@ -1037,7 +1006,7 @@ int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, flo
     for (int64_t q0 = 0; q0 < nq; q0 += chunk) {
         const int64_t nc = nq - q0 < chunk ? nq - q0 : chunk;
         const float* qp = q_dev + q0 * D128;
-        ivfpq_probe_kernel<<<static_cast<unsigned>((nc + 7) / 8), 256, 0, ctx->stream>>>(qp, nc, s->coarse, s->nlist, nprobe, s->probes);
+        NAFP_TRY(coarse_probe(ctx, qp, nc, s->coarse, s->nlist, nprobe, s->probes));
         if (s->flat_lists)
             ivfflat_scan_kernel<<<dim3(nprobe, static_cast<unsigned>(nc)), 256, 0, ctx->stream>>>(
                 qp, nc, s->probes, nprobe, idx->x32, s->lids, s->loff, s->lend, k, idx->label_offset, n_search, s->partD, s->partI);
@@ -1060,7 +1029,7 @@ int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, flo
         }
         topk_merge_kernel<<<static_cast<unsigned>(nc), 128, 0, ctx->stream>>>(s->partD, s->partI, groups > 1 ? groups : nprobe, nc, k,
                                                                               D_dev + q0 * k, I_dev + q0 * k);
-        ctx->launches += 3;
+        ctx->launches += 2;
     }
     NAFP_CUDA(cudaGetLastError());
     s->lut_rows += static_cast<unsigned long long>(nq);
@@ -1097,12 +1066,11 @@ int ivfpq_redo_rows(nafp_index* idx, const float* q_dev, int32_t n_redo, int k, 
         NAFP_CUDA(cudaMalloc(&s->redo_D, static_cast<size_t>(s->redo_cap) * MAX_K * sizeof(float)));
         NAFP_CUDA(cudaMalloc(&s->redo_I, static_cast<size_t>(s->redo_cap) * MAX_K * sizeof(int64_t)));
     }
-    ivfpq_gather_q_kernel<<<static_cast<unsigned>((static_cast<int64_t>(n_redo) * 32 + 255) / 256), 256, 0, ctx->stream>>>(
-        q_dev, s->redo_rows, n_redo, s->redo_q);
+    NAFP_TRY(nafp_seq_gather_rows_dev(ctx, q_dev, s->redo_rows, n_redo, s->redo_q));
     NAFP_TRY(ivfpq_search_lut(idx, s->redo_q, n_redo, k, s->redo_D, s->redo_I));
     ivfpq_scatter_kernel<<<static_cast<unsigned>((static_cast<int64_t>(n_redo) * k + 255) / 256), 256, 0, ctx->stream>>>(
         s->redo_D, s->redo_I, s->redo_rows, n_redo, k, D_dev, I_dev);
-    ctx->launches += 2;
+    ctx->launches++;
     NAFP_CUDA(cudaGetLastError());
     return NAFP_OK;
 }
@@ -1192,11 +1160,11 @@ static int ivfpq_search_first_level(nafp_index* idx, const float* q_dev, int64_t
     idx->label_offset = off;
     NAFP_TRY(st);
     // 2. the nprobe nearest lists of every row, 3. keep the candidates that live in them
-    ivfpq_probe_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, ctx->stream>>>(q_dev, nq, s->coarse, s->nlist, nprobe, probes_all);
+    NAFP_TRY(coarse_probe(ctx, q_dev, nq, s->coarse, s->nlist, nprobe, probes_all));
     ivfpq_filter_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, ctx->stream>>>(s->candD, s->candI, nq, k, probes_all, nprobe,
                                                                                      s->assign, idx->label_offset, D_dev, I_dev,
                                                                                      s->redo_rows, redo_count);
-    ctx->launches += 2;
+    ctx->launches++;
     NAFP_CUDA(cudaGetLastError());
     int32_t n_redo = 0;
     NAFP_CUDA(cudaMemcpyAsync(&n_redo, redo_count, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));

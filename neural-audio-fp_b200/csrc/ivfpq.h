@@ -78,23 +78,11 @@ __host__ __device__ __forceinline__ int64_t lcode_off(int64_t pos, int sub, int 
     return (pos >> 7) * (LIST_TILE * m) + (sub / mlo) * (LIST_TILE * mlo) + (r >> 2) * (4 * mlo) + (sub % mlo) * 4 + (r & 3);
 }
 
-// bitonic sort of n (a power of two) keys in shared memory by the whole block
-__device__ __forceinline__ void block_sort_asc_u64(uint64_t* keys, int n) {
-    for (int k = 2; k <= n; k <<= 1)
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int i = threadIdx.x; i < n; i += blockDim.x) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const uint64_t a = keys[i], b = keys[ixj];
-                    const bool asc = (i & k) == 0;
-                    if (asc ? (a > b) : (a < b)) { keys[i] = b; keys[ixj] = a; }
-                }
-            }
-            __syncthreads();
-        }
-}
-
 // ivfpq.cu
+// the nprobe nearest coarse centroids of every row of q[nq][128] -> probes[nq][nprobe]; optionally their distances
+// gdist[nq][nprobe] and the list-major scan's rounding bound qE[nq] (from dmax2).  One launch on ctx->stream.
+int coarse_probe(nafp_ctx* ctx, const float* q, int64_t nq, const float* coarse, int nlist, int nprobe, int32_t* probes,
+                 float* gdist = nullptr, float* qE = nullptr, const int32_t* dmax2 = nullptr);
 int build_lists(nafp_index* idx);
 int ivfpq_search_lut(nafp_index* idx, const float* q_dev, int64_t nq, int k, float* D_dev, int64_t* I_dev);
 int ivfpq_redo_rows(nafp_index* idx, const float* q_dev, int32_t n_redo, int k, float* D_dev, int64_t* I_dev);

@@ -39,6 +39,7 @@
 
 #include "ivfpq.h"
 #include "ptx.cuh"
+#include "topk.cuh"
 
 namespace nafp {
 
@@ -192,128 +193,6 @@ static int lm_prepare(nafp_index* idx, int64_t n_search) {
 }
 
 // ------------------------------------------------------------------------------------------ per-search preparation
-// one warp per query row: the nprobe nearest coarse centroids, ascending (ties -> lower list id) and their distances
-// (ivfpq_probe_kernel's arithmetic), plus the rounding bound of the row's bf16 scores
-__global__ void lm_probe_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse, int nlist, int nprobe,
-                                const int32_t* __restrict__ dmax2, int32_t* __restrict__ probes, float* __restrict__ gdist,
-                                float* __restrict__ qE) {
-    __shared__ float qs[8][D128];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-    if (i >= nq) return;
-    const float4 qv = reinterpret_cast<const float4*>(q + i * D128)[lane];
-    reinterpret_cast<float4*>(qs[w])[lane] = qv;
-    float qq = qv.x * qv.x + qv.y * qv.y + qv.z * qv.z + qv.w * qv.w;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(0xffffffffu, qq, o);
-    // |sum bf(q_i) bf(d_i) - sum q_i d_i| <= |q| |d| (2^-8 + 2^-18) for round-to-nearest bf16 operands; 3 % on top
-    // for the norms' own rounding and the tensor core's fp32 accumulation (<= 128 * 2^-23 relative)
-    if (lane == 0) qE[i] = sqrtf(qq) * sqrtf(__int_as_float(*dmax2)) * (1.03f / 256.f) + 1e-7f;
-    __syncwarp();
-    float d[IVF_MAX_NLIST / 32];
-#pragma unroll
-    for (int t = 0; t < IVF_MAX_NLIST / 32; ++t) {
-        const int c = lane + 32 * t;
-        float acc = FLT_MAX;
-        if (c < nlist) {
-            acc = 0.f;
-            const float* cr = coarse + static_cast<int64_t>(c) * D128;
-            for (int j = 0; j < D128; ++j) {
-                const float v = qs[w][j] - __ldg(cr + j);
-                acc = fmaf(v, v, acc);
-            }
-        }
-        d[t] = acc;
-    }
-    for (int p = 0; p < nprobe; ++p) {
-        float best = FLT_MAX;
-        int bi = INT_MAX;
-#pragma unroll
-        for (int t = 0; t < IVF_MAX_NLIST / 32; ++t)
-            if (d[t] < best) { best = d[t]; bi = lane + 32 * t; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-        }
-        if (lane == 0) {
-            probes[i * nprobe + p] = bi == INT_MAX ? -1 : bi;
-            gdist[i * nprobe + p] = best;
-        }
-#pragma unroll
-        for (int t = 0; t < IVF_MAX_NLIST / 32; ++t)
-            if (lane + 32 * t == bi) d[t] = FLT_MAX;
-    }
-}
-
-// The same for nlist <= 256 with the centroids transposed in shared memory (128 KB, loaded once per block; the block
-// then walks over its share of the query rows): lane l owns centroids l, l + 32, ...; conflict-free reads.  12x the
-// kernel above at 22 k rows (2.7 ms -> 0.2 ms), identical arithmetic (fma(v, v, acc), dimensions ascending).
-constexpr int LM_PROBE_NLIST = 256;
-constexpr int LM_PROBE_SMEM = (D128 * LM_PROBE_NLIST + 8 * D128) * 4;
-__global__ void __launch_bounds__(256)
-lm_probe_smem_kernel(const float* __restrict__ q, int64_t nq, const float* __restrict__ coarse, int nlist, int nprobe,
-                     const int32_t* __restrict__ dmax2, int32_t* __restrict__ probes, float* __restrict__ gdist, float* __restrict__ qE) {
-    extern __shared__ float psm[];
-    float* cs = psm;                                   // [dim][256 centroids]
-    float* qs = psm + D128 * LM_PROBE_NLIST;           // [8 warps][128]
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    for (int e = threadIdx.x; e < D128 * LM_PROBE_NLIST; e += blockDim.x) {
-        const int j = e / LM_PROBE_NLIST, c = e % LM_PROBE_NLIST;
-        cs[e] = c < nlist ? __ldg(coarse + static_cast<int64_t>(c) * D128 + j) : 0.f;
-    }
-    __syncthreads();
-    const float dm = sqrtf(__int_as_float(*dmax2));
-    float* qr = qs + w * D128;
-    for (int64_t i = static_cast<int64_t>(blockIdx.x) * 8 + w; i < nq; i += static_cast<int64_t>(gridDim.x) * 8) {
-        const float4 qv = reinterpret_cast<const float4*>(q + i * D128)[lane];
-        __syncwarp();
-        reinterpret_cast<float4*>(qr)[lane] = qv;
-        float qq = qv.x * qv.x + qv.y * qv.y + qv.z * qv.z + qv.w * qv.w;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) qq += __shfl_xor_sync(0xffffffffu, qq, o);
-        if (lane == 0) qE[i] = sqrtf(qq) * dm * (1.03f / 256.f) + 1e-7f;
-        __syncwarp();
-        float d[LM_PROBE_NLIST / 32];
-#pragma unroll
-        for (int t = 0; t < LM_PROBE_NLIST / 32; ++t) d[t] = 0.f;
-#pragma unroll 4
-        for (int j = 0; j < D128; ++j) {
-            const float qj = qr[j];
-            const float* cr = cs + j * LM_PROBE_NLIST + lane;
-#pragma unroll
-            for (int t = 0; t < LM_PROBE_NLIST / 32; ++t) {
-                const float v = qj - cr[32 * t];
-                d[t] = fmaf(v, v, d[t]);
-            }
-        }
-#pragma unroll
-        for (int t = 0; t < LM_PROBE_NLIST / 32; ++t)
-            if (lane + 32 * t >= nlist) d[t] = FLT_MAX;
-        for (int p = 0; p < nprobe; ++p) {
-            float best = FLT_MAX;
-            int bi = INT_MAX;
-#pragma unroll
-            for (int t = 0; t < LM_PROBE_NLIST / 32; ++t)
-                if (d[t] < best) { best = d[t]; bi = lane + 32 * t; }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-                const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-                if (ob < best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-            }
-            if (lane == 0) {
-                probes[i * nprobe + p] = bi == INT_MAX ? -1 : bi;
-                gdist[i * nprobe + p] = best;
-            }
-#pragma unroll
-            for (int t = 0; t < LM_PROBE_NLIST / 32; ++t)
-                if (lane + 32 * t == bi) d[t] = FLT_MAX;
-        }
-    }
-}
-
 // (query, probe) pairs -> buckets: wave of the probe rank (0: the query's nearest list) * nlist + list
 __global__ void lm_hist_kernel(const int32_t* __restrict__ probes, int64_t n_pairs, int nprobe, int nlist, int32_t* __restrict__ hist) {
     __shared__ int h[LM_WAVES * IVF_MAX_NLIST];
@@ -361,9 +240,6 @@ __device__ __forceinline__ void lm_mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
-}
-__device__ __forceinline__ float lm_key_score(uint64_t key) {
-    return ord2f(static_cast<int32_t>(static_cast<uint32_t>(key >> 32) ^ 0x80000000u));
 }
 
 __global__ void __launch_bounds__(LM_THREADS, 1)
@@ -620,7 +496,7 @@ ivfpq_lm_scan_kernel(const float* __restrict__ q, int nprobe, int S, const LmIte
                                     const uint64_t ne = lane < p ? e : (lane == p ? key : up);
                                     lq[lane] = ne;
                                     const uint64_t last = __shfl_sync(0xffffffffu, ne, LM_KP - 1);
-                                    if (lane == qi && last != 0ull) thr = fmaxf(thr, lm_key_score(last));
+                                    if (lane == qi && last != 0ull) thr = fmaxf(thr, key_score(last));
                                     __syncwarp();
                                 }
                             }
@@ -705,7 +581,7 @@ __global__ void ivfpq_lm_bound_kernel(const float* __restrict__ q, int64_t nq, i
         const int l = probes[i * nprobe + p / per_probe];
         float d = INFINITY;
         // exact distance >= |q - c|^2 - 2 (bf16 score + E)
-        if (key != 0ull && l >= 0 && gdist[i * nprobe + p / per_probe] - 2.f * (lm_key_score(key) + E) <= dk_prev)
+        if (key != 0ull && l >= 0 && gdist[i * nprobe + p / per_probe] - 2.f * (key_score(key) + E) <= dk_prev)
             d = lm_exact_adc(qs, coarse + static_cast<int64_t>(l) * D128, pq, lcodes, static_cast<uint32_t>(key));
         ds[p * LM_KP + lane] = d;
     }
@@ -764,12 +640,12 @@ ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k
         if (key != 0ull) {
             const int p = e / per_probe;
             // (a survivor whose distance cannot be below the last bound -- an upper bound of the k-th -- is not re-scored)
-            if (gdist[i * nprobe + p] - 2.f * (lm_key_score(key) + E) <= dk) {
+            if (gdist[i * nprobe + p] - 2.f * (key_score(key) + E) <= dk) {
                 const int slot = atomicAdd(&cnt_s, 1);
                 if (slot < LM_MERGE_KEYS) keys[slot] = (static_cast<uint64_t>(p) << 32) | static_cast<uint32_t>(key);
             }
             if ((e & (LM_KP - 1)) == LM_KP - 1)
-                atomicMin(&bound_s, f2ord(gdist[i * nprobe + p] - 2.f * (lm_key_score(key) + E)));
+                atomicMin(&bound_s, f2ord(gdist[i * nprobe + p] - 2.f * (key_score(key) + E)));
         }
     }
     __syncthreads();
@@ -790,31 +666,22 @@ ivfpq_lm_merge_kernel(const float* __restrict__ q, int64_t q0, int nprobe, int k
             const uint32_t pos = static_cast<uint32_t>(pk);
             const int l = probes[i * nprobe + p];
             const float d = lm_exact_adc(qs, coarse + static_cast<int64_t>(l) * D128, pq, lcodes, pos);
-            out = (static_cast<uint64_t>(__float_as_uint(d)) << 32) | static_cast<uint32_t>(lids[pos]);
+            out = dist_key(d, static_cast<uint32_t>(lids[pos]));
         }
         __syncwarp();
         keys[c] = out;         // (slot c was read by this thread only)
     }
     __syncthreads();
-    block_sort_asc_u64(keys, P);
+    block_sort_u64<true>(keys, P);
     // 3. proof: nothing the full lists dropped can be closer than the k-th survivor
     const uint64_t kth = keys[k - 1];
-    const float Dk = kth != ~0ull ? __uint_as_float(static_cast<uint32_t>(kth >> 32)) : INFINITY;
+    const float Dk = kth != ~0ull ? key_dist(kth) : INFINITY;
     const bool proven = bound_s == INT_MAX || Dk < ord2f(bound_s);
     if (!proven) {
         if (tid == 0) redo_rows[atomicAdd(redo_count, 1)] = static_cast<int32_t>(q0 + i);
         return;
     }
-    for (int j = tid; j < k; j += blockDim.x) {
-        const uint64_t key = keys[j];
-        if (key != ~0ull) {
-            D[i * k + j] = __uint_as_float(static_cast<uint32_t>(key >> 32));
-            I[i * k + j] = static_cast<int64_t>(static_cast<uint32_t>(key)) + label_offset;
-        } else {
-            D[i * k + j] = INFINITY;
-            I[i * k + j] = -1;
-        }
-    }
+    store_topk(keys, k, label_offset, D + i * k, I + i * k);
 }
 
 // ------------------------------------------------------------------------------------------ host
@@ -864,7 +731,6 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
     int32_t* redo_count = s->redo_rows + s->redo_cap;
     NAFP_CUDA(cudaMemsetAsync(redo_count, 0, sizeof(int32_t), ctx->stream));
     NAFP_CUDA(cudaFuncSetAttribute(ivfpq_lm_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LM_SMEM));
-    NAFP_CUDA(cudaFuncSetAttribute(lm_probe_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LM_PROBE_SMEM));
     const LmBoundFn bound_kernel = lm_bound_fns[S - 1];
     const LmMergeFn merge_kernel = lm_merge_fns[S - 1];
     NAFP_CUDA(cudaFuncSetAttribute(bound_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lm_bound_smem(S)));
@@ -879,12 +745,7 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
         const int64_t np = nc * nprobe;
         const float* qp = q_dev + q0 * D128;
         NAFP_TRY(lm_reserve(idx, nc, nprobe, S));
-        if (nlist <= LM_PROBE_NLIST)
-            lm_probe_smem_kernel<<<static_cast<unsigned>(std::min<int64_t>((nc + 7) / 8, ctx->sm_count)), 256, LM_PROBE_SMEM, ctx->stream>>>(
-                qp, nc, s->coarse, nlist, nprobe, L->dmax2, L->probes, L->gdist, L->qE);
-        else
-            lm_probe_kernel<<<static_cast<unsigned>((nc + 7) / 8), 256, 0, ctx->stream>>>(qp, nc, s->coarse, nlist, nprobe, L->dmax2, L->probes,
-                                                                                          L->gdist, L->qE);
+        NAFP_TRY(coarse_probe(ctx, qp, nc, s->coarse, nlist, nprobe, L->probes, L->gdist, L->qE, L->dmax2));
         NAFP_CUDA(cudaMemsetAsync(hist, 0, nb * sizeof(int32_t), ctx->stream));
         lm_hist_kernel<<<static_cast<unsigned>(std::min<int64_t>((np + 255) / 256, 4 * ctx->sm_count)), 256, 0, ctx->stream>>>(
             L->probes, np, nprobe, nlist, hist);
@@ -927,7 +788,7 @@ int ivfpq_search_lm(nafp_index* idx, const float* q_dev, int64_t nq, int k, floa
         lm_scatter_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, ctx->stream>>>(L->probes, np, nprobe, nlist, cursor, L->pairs);
         NAFP_CUDA(cudaMemsetAsync(L->cand, 0, static_cast<size_t>(np) * S * LM_SLOT * sizeof(uint64_t), ctx->stream));
         NAFP_CUDA(cudaMemsetAsync(L->dkA, 0x7f, static_cast<size_t>(nc) * sizeof(float), ctx->stream));     // 0x7f7f7f7f = 3.4e38: "no bound"
-        ctx->launches += 3;
+        ctx->launches += 2;
         for (int wv = 0; wv < LM_WAVES; ++wv) {
             if (n_items[wv] > 0) {
                 const int grid = std::min(n_items[wv], ctx->sm_count);

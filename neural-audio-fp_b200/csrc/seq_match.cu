@@ -15,6 +15,7 @@
 
 #include "index.h"
 #include "ptx.cuh"
+#include "topk.cuh"
 
 namespace nafp {
 
@@ -91,25 +92,6 @@ __global__ void seq_gather_rows_kernel(const float* __restrict__ qall, const int
     reinterpret_cast<float4*>(out + w * D128)[lane] = reinterpret_cast<const float4*>(qall + static_cast<int64_t>(rows[w]) * D128)[lane];
 }
 
-__device__ void bitonic_sort_asc_1024(uint64_t* keys) {
-    for (int k = 2; k <= SEQ_MAXC; k <<= 1) {
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int i = threadIdx.x; i < SEQ_MAXC; i += blockDim.x) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const uint64_t a = keys[i], b = keys[ixj];
-                    const bool asc = (i & k) == 0;
-                    if (asc ? (a > b) : (a < b)) {
-                        keys[i] = b;
-                        keys[ixj] = a;
-                    }
-                }
-            }
-            __syncthreads();
-        }
-    }
-}
-
 __global__ void __launch_bounds__(256)
 seq_cand_kernel(const float* __restrict__ qall, int64_t n_query_rows, const int64_t* __restrict__ test_ids,
                 const int32_t* __restrict__ seq_lens, int n_len, int L, int k_probe,
@@ -142,7 +124,7 @@ seq_cand_kernel(const float* __restrict__ qall, int64_t n_query_rows, const int6
         keys[e] = key;
     }
     __syncthreads();
-    bitonic_sort_asc_1024(keys);
+    block_sort_u64<true>(keys, SEQ_MAXC);
 
     // compaction of first occurrences (sorted by candidate, then by j => first has the minimal j)
     int base = 0;
@@ -209,10 +191,9 @@ __global__ void __launch_bounds__(256)
 seq_top_kernel(int n_len, const int64_t* __restrict__ cand_ids, const float* __restrict__ cand_scores,
                const int32_t* __restrict__ n_cand, int64_t* __restrict__ pred_ids, float* __restrict__ pred_scores) {
     __shared__ uint64_t red[8];
-    __shared__ uint64_t win;
     const int64_t t = blockIdx.x / n_len;
     const int li = blockIdx.x % n_len;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int tid = threadIdx.x;
     const int nu = n_cand[t];
     const float* sc = cand_scores + (t * n_len + li) * SEQ_MAXC;
     uint64_t mine[SEQ_MAXC / 256];
@@ -222,9 +203,7 @@ seq_top_kernel(int n_len, const int64_t* __restrict__ cand_ids, const float* __r
         uint64_t key = 0;
         if (u < nu) {
             const float s = sc[u];
-            if (s > -INFINITY)
-                key = (static_cast<uint64_t>(static_cast<uint32_t>(f2ord(s)) ^ 0x80000000u) << 32) |
-                      static_cast<uint64_t>(0xFFFFFFFFu - static_cast<uint32_t>(u));
+            if (s > -INFINITY) key = score_key(s, static_cast<uint32_t>(u));
         }
         mine[r] = key;
     }
@@ -232,29 +211,17 @@ seq_top_kernel(int n_len, const int64_t* __restrict__ cand_ids, const float* __r
         uint64_t best = 0;
 #pragma unroll
         for (int r = 0; r < SEQ_MAXC / 256; ++r) best = mine[r] > best ? mine[r] : best;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const uint64_t other = __shfl_xor_sync(0xffffffffu, best, o);
-            best = other > best ? other : best;
-        }
-        if (lane == 0) red[warp] = best;
-        __syncthreads();
+        const uint64_t w = block_max_u64(best, red);
         if (tid == 0) {
-            uint64_t b = 0;
-            for (int w = 0; w < 8; ++w) b = red[w] > b ? red[w] : b;
-            win = b;
             const int64_t o = (t * n_len + li) * SEQ_NPRED + p;
-            if (b != 0) {
-                const uint32_t u = 0xFFFFFFFFu - static_cast<uint32_t>(b);
-                pred_ids[o] = cand_ids[t * SEQ_MAXC + u];
-                if (pred_scores) pred_scores[o] = ord2f(static_cast<int>(static_cast<uint32_t>(b >> 32) ^ 0x80000000u));
+            if (w != 0) {
+                pred_ids[o] = cand_ids[t * SEQ_MAXC + key_row(w)];
+                if (pred_scores) pred_scores[o] = key_score(w);
             } else {
                 pred_ids[o] = -1;
                 if (pred_scores) pred_scores[o] = -INFINITY;
             }
         }
-        __syncthreads();
-        const uint64_t w = win;
 #pragma unroll
         for (int r = 0; r < SEQ_MAXC / 256; ++r)
             if (mine[r] == w) mine[r] = 0;
@@ -264,11 +231,10 @@ seq_top_kernel(int n_len, const int64_t* __restrict__ cand_ids, const float* __r
 
 
 // merge W per-shard top-k lists (already holding global labels) into one: order by (distance, label)
-__global__ void __launch_bounds__(128)
-topk_merge_kernel(const float* __restrict__ D_all, const int64_t* __restrict__ I_all, int W, int64_t nq, int k,
-                  float* __restrict__ D_out, int64_t* __restrict__ I_out) {
-    __shared__ float d_s[4096];          // 16 + 32 KB: the static shared-memory limit
-    __shared__ int64_t i_s[4096];
+__global__ void topk_merge_kernel(const float* __restrict__ D_all, const int64_t* __restrict__ I_all, int W, int64_t nq, int k,
+                                  float* __restrict__ D_out, int64_t* __restrict__ I_out) {
+    __shared__ float d_s[TOPK_MERGE_KEYS];
+    __shared__ int64_t i_s[TOPK_MERGE_KEYS];
     const int64_t q = blockIdx.x;
     const int n = W * k;
     int npow = 1;
@@ -286,24 +252,7 @@ topk_merge_kernel(const float* __restrict__ D_all, const int64_t* __restrict__ I
         i_s[e] = id < 0 ? LLONG_MAX : id;
     }
     __syncthreads();
-    for (int kk = 2; kk <= npow; kk <<= 1) {
-        for (int j = kk >> 1; j > 0; j >>= 1) {
-            for (int i = threadIdx.x; i < npow; i += blockDim.x) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const float da = d_s[i], db = d_s[ixj];
-                    const int64_t ia = i_s[i], ib = i_s[ixj];
-                    const bool a_after_b = (da > db) || (da == db && ia > ib);
-                    const bool asc = (i & kk) == 0;
-                    if (asc ? a_after_b : !a_after_b) {
-                        d_s[i] = db; d_s[ixj] = da;
-                        i_s[i] = ib; i_s[ixj] = ia;
-                    }
-                }
-            }
-            __syncthreads();
-        }
-    }
+    block_sort_dist_label(d_s, i_s, npow);
     for (int j = threadIdx.x; j < k; j += blockDim.x) {
         const int64_t id = i_s[j];
         D_out[q * k + j] = d_s[j];
@@ -397,7 +346,8 @@ int nafp_topk_merge_dev(nafp_ctx* ctx, const float* D_all_dev, const int64_t* I_
                         int64_t nq, int32_t k, float* D_out_dev, int64_t* I_out_dev) {
     NAFP_RANGE("nafp_topk_merge_dev");
     NAFP_REQUIRE(ctx && D_all_dev && I_all_dev && D_out_dev && I_out_dev && n_shards >= 1 && k >= 1 &&
-                     n_shards * k <= 4096, NAFP_ERR_INVALID, "nafp_topk_merge_dev: need n_shards*k <= 4096");
+                     n_shards * k <= TOPK_MERGE_KEYS, NAFP_ERR_INVALID, "nafp_topk_merge_dev: need n_shards*k <= %d",
+                 TOPK_MERGE_KEYS);
     if (nq == 0) return NAFP_OK;
     topk_merge_kernel<<<static_cast<unsigned>(nq), 128, 0, ctx->stream>>>(D_all_dev, I_all_dev, n_shards, nq, k,
                                                                           D_out_dev, I_out_dev);
