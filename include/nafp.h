@@ -259,6 +259,29 @@ int nafp_seq_cand_dev(nafp_index* idx, const float* q_dev, int64_t n_query_rows,
 int nafp_seq_top_dev(nafp_ctx* ctx, int64_t n_test, int32_t n_len, const int64_t* cand_ids_dev,
                      const float* cand_scores_dev, const int32_t* n_cand_dev,
                      int64_t* pred_ids_dev, float* pred_scores_dev);
+/* ------------------------------------------------------------------ clip matcher
+ * Identifies recordings: the matcher of nafp_seq_match for one sequence per clip, of any length up to 4096 rows
+ * (34 min at the 0.5 s hop) and with any number of candidates.
+ *   q_host           (n_rows, d) float32 query fingerprints, the clips back to back
+ *   clip_off_host    n_clips+1 int64 row offsets: clip i is rows clip_off[i] .. clip_off[i+1]-1; clip_off[0] = 0,
+ *                    clip_off[n_clips] = n_rows, every clip 1..4096 rows
+ * One top-k_probe segment search of all n_rows rows (k_probe <= 128); per clip the offset-compensated candidates
+ * c = label - j >= 0, sorted and unique; score(c) = mean_j q[j].x[c+j] over the m = min(L, rows from c on) rows that
+ * exist (the arithmetic of nafp_seq_match, so a clip of L <= 32 rows scores bit for bit like seq_lens = [L]); the
+ * n_top (<= 100) best by score, ties to the lower id.
+ * Outputs: pred_ids_host (n_clips, n_top) int64 (-1 padded), pred_scores_host same shape float32 (-inf padded; may
+ * be NULL).  Bad arguments return NAFP_ERR_INVALID before any device work.  n_rows * k_probe < 2^31 per call. */
+int nafp_clip_match(nafp_index* idx, const float* q_host, int64_t n_rows, const int64_t* clip_off_host,
+                    int64_t n_clips, int32_t k_probe, int32_t n_top, int64_t* pred_ids_host,
+                    float* pred_scores_host);
+/* The same on device buffers, asynchronous on the context stream.  The offsets are checked on the device: unless
+ * 0 <= clip_off[0], every clip holds 1..4096 rows and clip_off[n_clips] <= n_rows, no clip gets a candidate and every
+ * output is -1 / -inf (no query row outside [0, n_rows) is read).  Rows outside [clip_off[0], clip_off[n_clips]) are
+ * searched and ignored. */
+int nafp_clip_match_dev(nafp_index* idx, const float* q_dev, int64_t n_rows, const int64_t* clip_off_dev,
+                        int64_t n_clips, int32_t k_probe, int32_t n_top, int64_t* pred_ids_dev,
+                        float* pred_scores_dev);
+
 /* merge n_shards top-k lists: D_all/I_all (n_shards, nq, k) -> (nq, k), ordered by (distance, label) */
 int nafp_topk_merge_dev(nafp_ctx* ctx, const float* D_all_dev, const int64_t* I_all_dev,
                         int32_t n_shards, int64_t nq, int32_t k, float* D_out_dev, int64_t* I_out_dev);

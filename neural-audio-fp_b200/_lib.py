@@ -96,6 +96,8 @@ _SIGS = {
     "nafp_seq_cand_dev": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32,
                                   c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "nafp_seq_top_dev": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "nafp_clip_match": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p]),
+    "nafp_clip_match_dev": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p]),
     "nafp_topk_merge_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_int32, c_void_p, c_void_p]),
     "nafp_pairwise_dists_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int32, c_int32, c_void_p]),
     "nafp_conv_eye_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int32, c_void_p]),

@@ -103,6 +103,7 @@ int nafp_ctx_destroy(nafp_ctx* ctx) {
     encoder_destroy(ctx);
     if (ctx->stage_dev) cudaFree(ctx->stage_dev);
     if (ctx->stage_pinned) cudaFreeHost(ctx->stage_pinned);
+    if (ctx->clip_ws) cudaFree(ctx->clip_ws);
     cudaEventDestroy(ctx->ev0);
     cudaEventDestroy(ctx->ev1);
     cudaStreamDestroy(ctx->own_stream);

@@ -72,6 +72,9 @@ struct nafp_ctx {
     int64_t stage_dev_bytes = 0;
     void* stage_pinned = nullptr;
     int64_t stage_pinned_bytes = 0;
+    // workspace of the clip matcher (search results, candidate sorts, scores)
+    void* clip_ws = nullptr;
+    int64_t clip_ws_bytes = 0;
 };
 
 namespace nafp {

@@ -328,5 +328,12 @@ __device__ __forceinline__ float warp_dot128(const float4 a, const float* __rest
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
     return s;
 }
+// the same arithmetic on a row already loaded (the clip matcher keeps several rows in flight)
+__device__ __forceinline__ float warp_dot128_f4(const float4 a, const float4 b) {
+    float s = a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    return s;
+}
 
 }  // namespace nafp

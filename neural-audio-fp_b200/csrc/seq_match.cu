@@ -11,6 +11,7 @@
 //   seq_top_kernel      the 10 best candidates per (test id, length), ties to the lower id (:232)
 // Candidates this shard does not own score -inf, so that a row-sharded database can combine the
 // per-rank score tables with a max-reduce between the two kernels.
+#include <algorithm>
 #include <climits>
 
 #include "index.h"
@@ -260,6 +261,198 @@ __global__ void topk_merge_kernel(const float* __restrict__ D_all, const int64_t
     }
 }
 
+// ---- clip matcher: one sequence of L (<= CLIP_MAXL) consecutive query rows per clip, any number of candidates.
+//   clip_offsets_kernel  the device-side check of the clip offsets: any clip out of order or out of range -> flag
+//   clip_cand_kernel     offset compensation c = label - j of every (row, neighbour) -> entry (clip << 32 | c)
+//   clip_sort_*          device-wide ascending bitonic sort of those entries: candidates grouped by clip, ascending
+//   clip_score_kernel    one warp per first occurrence: the running mean of q[j] . x32[c + j] (seq_cand_kernel's
+//                        arithmetic), re-keyed as (clip, score descending, position) -- the position orders equal
+//                        scores by candidate id
+//   clip_sort_*          the same sort of the scored entries
+//   clip_top_kernel      the first n_top entries of every clip
+constexpr int CLIP_MAXL = 4096;
+constexpr int CLIP_NTOP = 100;
+constexpr int CLIP_SORT_TILE = 2048;      // entries one block sorts in shared memory (32 KB)
+constexpr uint64_t CLIP_NONE = ~0ull;
+
+// bad != 0 afterwards (it is zeroed before) unless 0 <= clip_off[0], every clip holds 1..CLIP_MAXL rows and
+// clip_off[n_clips] <= n_rows
+__global__ void __launch_bounds__(256)
+clip_offsets_kernel(const int64_t* __restrict__ clip_off, int64_t n_clips, int64_t n_rows, int32_t* __restrict__ bad) {
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_clips;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int64_t off = clip_off[i], L = clip_off[i + 1] - off;
+        if (off < 0 || L < 1 || L > CLIP_MAXL || clip_off[i + 1] > n_rows) *bad = 1;
+    }
+}
+
+// with bad offsets no (row, neighbour) becomes a candidate: every clip then reports -1 / -inf, and no query row
+// outside [0, n_rows) is ever read
+__global__ void __launch_bounds__(256)
+clip_cand_kernel(const int64_t* __restrict__ I, int64_t n_keys, int k_probe, const int64_t* __restrict__ clip_off,
+                 int64_t n_clips, const int32_t* __restrict__ bad, int64_t owned_lo, int64_t owned_hi, int64_t n_pad,
+                 SortKV* __restrict__ out) {
+    const bool ok = *bad == 0;
+    for (int64_t t = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; t < n_pad;
+         t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        SortKV v{CLIP_NONE, CLIP_NONE};
+        if (ok && t < n_keys) {
+            const int64_t g = t / k_probe;        // query row
+            int64_t lo = 0, hi = n_clips;         // the last clip starting at or before g
+            while (hi - lo > 1) {
+                const int64_t mid = (lo + hi) >> 1;
+                if (clip_off[mid] <= g) lo = mid;
+                else hi = mid;
+            }
+            const int64_t off = clip_off[lo], L = clip_off[lo + 1] - off, j = g - off;
+            const int64_t lab = I[t];
+            const int64_t c = lab - j;
+            if (L >= 1 && L <= CLIP_MAXL && j >= 0 && j < L && lab >= 0 && c >= 0 && c >= owned_lo && c < owned_hi)
+                v = SortKV{(static_cast<uint64_t>(lo) << 32) | static_cast<uint64_t>(c), 0};
+        }
+        out[t] = v;
+    }
+}
+
+__global__ void __launch_bounds__(1024) clip_sort_tiles_kernel(SortKV* __restrict__ a) {
+    __shared__ SortKV s[CLIP_SORT_TILE];
+    SortKV* g = a + static_cast<int64_t>(blockIdx.x) * CLIP_SORT_TILE;
+    for (int i = threadIdx.x; i < CLIP_SORT_TILE; i += blockDim.x) s[i] = g[i];
+    __syncthreads();
+    block_sort_kv(s, CLIP_SORT_TILE);
+    for (int i = threadIdx.x; i < CLIP_SORT_TILE; i += blockDim.x) g[i] = s[i];
+}
+__global__ void __launch_bounds__(1024) clip_merge_tiles_kernel(SortKV* __restrict__ a) {
+    __shared__ SortKV s[CLIP_SORT_TILE];
+    SortKV* g = a + static_cast<int64_t>(blockIdx.x) * CLIP_SORT_TILE;
+    for (int i = threadIdx.x; i < CLIP_SORT_TILE; i += blockDim.x) s[i] = g[i];
+    __syncthreads();
+    block_merge_kv(s, CLIP_SORT_TILE);
+    for (int i = threadIdx.x; i < CLIP_SORT_TILE; i += blockDim.x) g[i] = s[i];
+}
+// one global step of the merge at stride j >= CLIP_SORT_TILE; the first step of a merge of two sorted runs of j
+// entries compares mirrored positions (i, 2j-1-i), which makes the pair one bitonic sequence
+template <bool First>
+__global__ void __launch_bounds__(256) clip_merge_step_kernel(SortKV* __restrict__ a, int64_t n_pairs, int64_t j) {
+    for (int64_t p = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; p < n_pairs;
+         p += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int64_t i = pair_lo(p, j);
+        kv_order(a, i, First ? (i | (j - 1)) + j - (i & (j - 1)) : i + j);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+clip_score_kernel(const float* __restrict__ q, const int64_t* __restrict__ clip_off, const SortKV* __restrict__ cand,
+                  int64_t n_pad, const float* __restrict__ x32, int64_t n_rows_local, int64_t label_offset,
+                  SortKV* __restrict__ ranked, float* __restrict__ scores) {
+    const int lane = threadIdx.x & 31;
+    const int64_t n_warps = static_cast<int64_t>(gridDim.x) * (blockDim.x >> 5);
+    for (int64_t e = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; e < n_pad; e += n_warps) {
+        const uint64_t key = cand[e].hi;
+        SortKV o{CLIP_NONE, CLIP_NONE};
+        if (key != CLIP_NONE && (e == 0 || cand[e - 1].hi != key)) {      // first occurrence of (clip, c)
+            const int64_t clip = static_cast<int64_t>(key >> 32), c = static_cast<int64_t>(key & 0xFFFFFFFFull);
+            const int64_t off = clip_off[clip], L = clip_off[clip + 1] - off;
+            const int64_t row = c - label_offset;
+            const int64_t left = n_rows_local - row;             // rows of x32 that exist at c, c+1, ... (clamp)
+            const int m = static_cast<int>(left < L ? left : L);
+            const float* qc = q + off * D128;
+            const float* xc = x32 + row * D128;
+            float sum = 0.f;
+            int j = 0;
+            // four rows in flight per step; the running sum still adds them one by one in ascending j
+            for (; j + 4 <= m; j += 4) {
+                float4 qv[4], xv[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    qv[u] = reinterpret_cast<const float4*>(qc + (j + u) * D128)[lane];
+                    xv[u] = reinterpret_cast<const float4*>(xc + (j + u) * D128)[lane];
+                }
+#pragma unroll
+                for (int u = 0; u < 4; ++u) sum += warp_dot128_f4(qv[u], xv[u]);
+            }
+            for (; j < m; ++j) sum += warp_dot128(reinterpret_cast<const float4*>(qc + j * D128)[lane], xc + j * D128, lane);
+            const float sc = sum / static_cast<float>(m);
+            if (sc > -INFINITY) {
+                const uint64_t desc = 0xFFFFFFFFull - (score_key(sc, 0) >> 32);
+                o = SortKV{(static_cast<uint64_t>(clip) << 32) | desc, static_cast<uint64_t>(e)};
+            }
+            if (lane == 0) scores[e] = sc;
+        }
+        if (lane == 0) ranked[e] = o;
+    }
+}
+
+// first entry of ranked[0, n) whose hi is >= v
+__device__ __forceinline__ int64_t kv_lower_bound(const SortKV* __restrict__ a, int64_t n, uint64_t v) {
+    int64_t lo = 0, hi = n;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (a[mid].hi < v) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+__global__ void __launch_bounds__(128)
+clip_top_kernel(const SortKV* __restrict__ ranked, int64_t n_pad, const SortKV* __restrict__ cand,
+                const float* __restrict__ scores, int64_t n_clips, int n_top, int64_t* __restrict__ pred_ids,
+                float* __restrict__ pred_scores) {
+    const int64_t t = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= n_clips * n_top) return;
+    const uint64_t clip = static_cast<uint64_t>(t / n_top);
+    const int64_t r = t % n_top;
+    const int64_t first = kv_lower_bound(ranked, n_pad, clip << 32);
+    const int64_t end = kv_lower_bound(ranked, n_pad, (clip + 1) << 32);
+    int64_t id = -1;
+    float sc = -INFINITY;
+    if (first + r < end) {
+        const int64_t e = static_cast<int64_t>(ranked[first + r].lo);
+        id = static_cast<int64_t>(cand[e].hi & 0xFFFFFFFFull);
+        sc = scores[e];
+    }
+    pred_ids[t] = id;
+    if (pred_scores) pred_scores[t] = sc;
+}
+
+// ascending sort of n_pad (a power of two >= CLIP_SORT_TILE) entries
+static int clip_sort(nafp_ctx* ctx, SortKV* a, int64_t n_pad) {
+    const unsigned tiles = static_cast<unsigned>(n_pad / CLIP_SORT_TILE);
+    const int64_t n_pairs = n_pad / 2;
+    const unsigned grid = static_cast<unsigned>(std::min<int64_t>((n_pairs + 255) / 256, int64_t(ctx->sm_count) * 16));
+    clip_sort_tiles_kernel<<<tiles, 1024, 0, ctx->stream>>>(a);
+    ctx->launches++;
+    for (int64_t s = 2 * CLIP_SORT_TILE; s <= n_pad; s <<= 1) {
+        clip_merge_step_kernel<true><<<grid, 256, 0, ctx->stream>>>(a, n_pairs, s >> 1);
+        ctx->launches++;
+        for (int64_t j = s >> 2; j >= CLIP_SORT_TILE; j >>= 1) {
+            clip_merge_step_kernel<false><<<grid, 256, 0, ctx->stream>>>(a, n_pairs, j);
+            ctx->launches++;
+        }
+        clip_merge_tiles_kernel<<<tiles, 1024, 0, ctx->stream>>>(a);
+        ctx->launches++;
+    }
+    NAFP_CUDA(cudaGetLastError());
+    return NAFP_OK;
+}
+
+static int64_t clip_pad(int64_t n_keys) {
+    int64_t p = CLIP_SORT_TILE;
+    while (p < n_keys) p <<= 1;
+    return p;
+}
+
+// every checked argument of the clip matcher except the offsets, which only the host entry point can read
+static int clip_check(nafp_index* idx, int64_t n_rows, int64_t n_clips, int32_t k_probe, int32_t n_top, const char* fn) {
+    NAFP_REQUIRE(idx && n_rows >= 0 && n_clips >= 0, NAFP_ERR_INVALID, "%s: bad arguments", fn);
+    NAFP_REQUIRE(k_probe >= 1 && k_probe <= MAX_K, NAFP_ERR_INVALID, "%s: k_probe %d outside [1,%d]", fn, k_probe, MAX_K);
+    NAFP_REQUIRE(n_top >= 1 && n_top <= CLIP_NTOP, NAFP_ERR_INVALID, "%s: n_top %d outside [1,%d]", fn, n_top, CLIP_NTOP);
+    NAFP_REQUIRE(n_rows * k_probe < (1ll << 31) && n_clips < (1ll << 31), NAFP_ERR_INVALID,
+                 "%s: n_rows * k_probe must stay below 2^31 (split the clips over several calls)", fn);
+    NAFP_REQUIRE(idx->label_offset + idx->n < (1ll << 32), NAFP_ERR_INVALID, "%s: labels must stay below 2^32", fn);
+    NAFP_REQUIRE(idx->x32 != nullptr || idx->n == 0, NAFP_ERR_STATE, "%s: index holds no rows", fn);
+    return NAFP_OK;
+}
+
 }  // namespace nafp
 
 using namespace nafp;
@@ -423,6 +616,102 @@ int nafp_seq_match(nafp_index* idx, const float* q_host, int64_t n_query_rows, c
     NAFP_CUDA(cudaMemcpyAsync(pred_ids_host, pid, static_cast<size_t>(n_test) * n_len * SEQ_NPRED * 8, cudaMemcpyDeviceToHost, ctx->stream));
     if (pred_scores_host)
         NAFP_CUDA(cudaMemcpyAsync(pred_scores_host, psc, static_cast<size_t>(n_test) * n_len * SEQ_NPRED * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
+    return NAFP_OK;
+}
+
+int nafp_clip_match_dev(nafp_index* idx, const float* q_dev, int64_t n_rows, const int64_t* clip_off_dev,
+                        int64_t n_clips, int32_t k_probe, int32_t n_top, int64_t* pred_ids_dev, float* pred_scores_dev) {
+    NAFP_RANGE("nafp_clip_match_dev");
+    NAFP_TRY(clip_check(idx, n_rows, n_clips, k_probe, n_top, "nafp_clip_match_dev"));
+    NAFP_REQUIRE(n_clips == 0 || (q_dev && clip_off_dev && pred_ids_dev), NAFP_ERR_INVALID,
+                 "nafp_clip_match_dev: NULL argument");
+    if (n_clips == 0) return NAFP_OK;
+    nafp_ctx* ctx = idx->ctx;
+    NAFP_CUDA(cudaSetDevice(ctx->device));
+    const int64_t n_keys = n_rows * k_probe;
+    const int64_t n_pad = clip_pad(n_keys);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t o_D = take(static_cast<size_t>(n_keys) * 4);
+    const size_t o_I = take(static_cast<size_t>(n_keys) * 8);
+    const size_t o_cand = take(static_cast<size_t>(n_pad) * sizeof(SortKV));
+    const size_t o_rank = take(static_cast<size_t>(n_pad) * sizeof(SortKV));
+    const size_t o_sc = take(static_cast<size_t>(n_pad) * 4);
+    const size_t o_bad = take(4);
+    NAFP_TRY(ensure_dev(ctx, &ctx->clip_ws, &ctx->clip_ws_bytes, static_cast<int64_t>(off)));
+    uint8_t* base = static_cast<uint8_t*>(ctx->clip_ws);
+    float* Dd = reinterpret_cast<float*>(base + o_D);
+    int64_t* Id = reinterpret_cast<int64_t*>(base + o_I);
+    SortKV* cand = reinterpret_cast<SortKV*>(base + o_cand);
+    SortKV* ranked = reinterpret_cast<SortKV*>(base + o_rank);
+    float* scores = reinterpret_cast<float*>(base + o_sc);
+    int32_t* bad = reinterpret_cast<int32_t*>(base + o_bad);
+
+    if (n_rows > 0) NAFP_TRY(nafp_index_search_dev(idx, q_dev, n_rows, k_probe, Dd, Id));
+    const int64_t n_search = idx->search_rows >= 0 && idx->search_rows < idx->n ? idx->search_rows : idx->n;
+    const unsigned grid = static_cast<unsigned>(std::min<int64_t>((n_pad + 255) / 256, int64_t(ctx->sm_count) * 16));
+    NAFP_CUDA(cudaMemsetAsync(bad, 0, 4, ctx->stream));
+    const unsigned grid_c = static_cast<unsigned>(std::min<int64_t>((n_clips + 255) / 256, int64_t(ctx->sm_count) * 4));
+    clip_offsets_kernel<<<grid_c, 256, 0, ctx->stream>>>(clip_off_dev, n_clips, n_rows, bad);
+    clip_cand_kernel<<<grid, 256, 0, ctx->stream>>>(Id, n_keys, k_probe, clip_off_dev, n_clips, bad, idx->label_offset,
+                                                   idx->label_offset + n_search, n_pad, cand);
+    ctx->launches += 2;
+    NAFP_CUDA(cudaGetLastError());
+    NAFP_TRY(clip_sort(ctx, cand, n_pad));
+    // one warp per entry: 8 per block, enough blocks to fill every SM many times over
+    const unsigned grid_w = static_cast<unsigned>(std::min<int64_t>((n_pad + 7) / 8, int64_t(ctx->sm_count) * 64));
+    clip_score_kernel<<<grid_w, 256, 0, ctx->stream>>>(q_dev, clip_off_dev, cand, n_pad, idx->x32, idx->n,
+                                                      idx->label_offset, ranked, scores);
+    ctx->launches++;
+    NAFP_CUDA(cudaGetLastError());
+    NAFP_TRY(clip_sort(ctx, ranked, n_pad));
+    const int64_t n_out = n_clips * n_top;
+    clip_top_kernel<<<static_cast<unsigned>((n_out + 127) / 128), 128, 0, ctx->stream>>>(
+        ranked, n_pad, cand, scores, n_clips, n_top, pred_ids_dev, pred_scores_dev);
+    ctx->launches++;
+    NAFP_CUDA(cudaGetLastError());
+    return NAFP_OK;
+}
+
+int nafp_clip_match(nafp_index* idx, const float* q_host, int64_t n_rows, const int64_t* clip_off_host,
+                    int64_t n_clips, int32_t k_probe, int32_t n_top, int64_t* pred_ids_host, float* pred_scores_host) {
+    NAFP_RANGE("nafp_clip_match");
+    NAFP_TRY(clip_check(idx, n_rows, n_clips, k_probe, n_top, "nafp_clip_match"));
+    NAFP_REQUIRE(clip_off_host && (n_clips == 0 || (q_host && pred_ids_host)), NAFP_ERR_INVALID,
+                 "nafp_clip_match: NULL argument");
+    NAFP_REQUIRE(clip_off_host[0] == 0 && clip_off_host[n_clips] == n_rows, NAFP_ERR_INVALID,
+                 "nafp_clip_match: clip offsets must run from 0 to n_rows (%lld)", static_cast<long long>(n_rows));
+    for (int64_t i = 0; i < n_clips; ++i) {
+        const int64_t L = clip_off_host[i + 1] - clip_off_host[i];
+        NAFP_REQUIRE(L >= 1 && L <= CLIP_MAXL, NAFP_ERR_INVALID,
+                     "nafp_clip_match: clip %lld has %lld rows; clip offsets must ascend by 1..%d rows",
+                     static_cast<long long>(i), static_cast<long long>(L), CLIP_MAXL);
+    }
+    if (n_clips == 0) return NAFP_OK;
+    nafp_ctx* ctx = idx->ctx;
+    NAFP_CUDA(cudaSetDevice(ctx->device));
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t o_q = take(static_cast<size_t>(n_rows) * D128 * 4);
+    const size_t o_off = take(static_cast<size_t>(n_clips + 1) * 8);
+    const size_t o_pid = take(static_cast<size_t>(n_clips) * n_top * 8);
+    const size_t o_psc = take(static_cast<size_t>(n_clips) * n_top * 4);
+    NAFP_TRY(ensure_dev(ctx, &ctx->stage_dev, &ctx->stage_dev_bytes, static_cast<int64_t>(off)));
+    uint8_t* base = static_cast<uint8_t*>(ctx->stage_dev);
+    float* q_dev = reinterpret_cast<float*>(base + o_q);
+    int64_t* off_dev = reinterpret_cast<int64_t*>(base + o_off);
+    int64_t* pid = reinterpret_cast<int64_t*>(base + o_pid);
+    float* psc = reinterpret_cast<float*>(base + o_psc);
+    NAFP_CUDA(cudaMemcpyAsync(q_dev, q_host, static_cast<size_t>(n_rows) * D128 * 4, cudaMemcpyHostToDevice, ctx->stream));
+    NAFP_CUDA(cudaMemcpyAsync(off_dev, clip_off_host, static_cast<size_t>(n_clips + 1) * 8, cudaMemcpyHostToDevice,
+                              ctx->stream));
+    NAFP_TRY(nafp_clip_match_dev(idx, q_dev, n_rows, off_dev, n_clips, k_probe, n_top, pid, psc));
+    NAFP_CUDA(cudaMemcpyAsync(pred_ids_host, pid, static_cast<size_t>(n_clips) * n_top * 8, cudaMemcpyDeviceToHost,
+                              ctx->stream));
+    if (pred_scores_host)
+        NAFP_CUDA(cudaMemcpyAsync(pred_scores_host, psc, static_cast<size_t>(n_clips) * n_top * 4,
+                                  cudaMemcpyDeviceToHost, ctx->stream));
     NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
     return NAFP_OK;
 }

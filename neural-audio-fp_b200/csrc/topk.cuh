@@ -71,6 +71,44 @@ __device__ __forceinline__ void block_sort_dist_label(float* d, int64_t* id, int
         }
 }
 
+// ---- 128-bit entries of the device-wide sorts of the clip matcher (seq_match.cu): ascending by (hi, lo); all ones is
+// past every real entry
+struct SortKV {
+    uint64_t hi, lo;
+};
+__device__ __forceinline__ bool kv_greater(const SortKV& a, const SortKV& b) {
+    return a.hi > b.hi || (a.hi == b.hi && a.lo > b.lo);
+}
+// s[i] <= s[j] afterwards
+__device__ __forceinline__ void kv_order(SortKV* s, int64_t i, int64_t j) {
+    const SortKV a = s[i], b = s[j];
+    if (kv_greater(a, b)) { s[i] = b; s[j] = a; }
+}
+// the lower index of compare pair p at stride j (a power of two): pairs (i, i + j) with bit j of i clear
+__device__ __forceinline__ int64_t pair_lo(int64_t p, int64_t j) { return ((p & ~(j - 1)) << 1) | (p & (j - 1)); }
+// ascending bitonic sort of n (a power of two) entries in shared memory by the whole block
+__device__ __forceinline__ void block_sort_kv(SortKV* s, int n) {
+    for (int k = 2; k <= n; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int p = threadIdx.x; p < (n >> 1); p += blockDim.x) {
+                const int i = static_cast<int>(pair_lo(p, j));
+                if ((i & k) == 0) kv_order(s, i, i + j);
+                else kv_order(s, i + j, i);
+            }
+            __syncthreads();
+        }
+}
+// the closing steps (strides n/2 .. 1) of an ascending bitonic merge whose larger strides are done
+__device__ __forceinline__ void block_merge_kv(SortKV* s, int n) {
+    for (int j = n >> 1; j > 0; j >>= 1) {
+        for (int p = threadIdx.x; p < (n >> 1); p += blockDim.x) {
+            const int i = static_cast<int>(pair_lo(p, j));
+            kv_order(s, i, i + j);
+        }
+        __syncthreads();
+    }
+}
+
 // ---- reductions
 // arg-min over the warp, ties to the lower index; every lane returns the winner
 __device__ __forceinline__ void warp_argmin(float& best, int& idx) {

@@ -19,6 +19,9 @@ from ..._lib import Context, NafpError, check, lib, ptr
 
 FLAT_L2, IVFPQ, IVF_FLAT, IVFPQR = 0, 1, 2, 3
 _ADD_CHUNK = 1 << 20      # rows per host->device copy (memmaps are read chunk by chunk)
+CLIP_MAXL = 4096          # rows of one clip (34 min at the 0.5 s hop), include/nafp.h
+CLIP_NTOP = 100           # best matches per clip, at most
+CLIP_CALL_ROWS = 1 << 16  # query rows per nafp_clip_match call: bounds its device workspace (~0.4 GB at k_probe 128)
 
 
 def _f32c(x):
@@ -168,6 +171,35 @@ class Index:
         scores = np.full((n_test, n_len, 10), -np.inf, dtype=np.float32)
         check(lib.nafp_seq_match(self.h, ptr(query), query.shape[0], ptr(test_ids), n_test, ptr(seq_lens), n_len,
                                  int(k_probe), ptr(pred), ptr(scores)))
+        return pred, scores
+
+    def clip_match(self, rows, clip_off, k_probe=20, n_top=10):
+        """Identify clips: clip i is ``rows[clip_off[i]:clip_off[i+1]]`` (1..CLIP_MAXL consecutive segment
+        fingerprints); every clip is matched as one sequence of its own length (``nafp_clip_match``).
+        Returns pred_ids (n_clips, n_top) int64 -- start rows of the best-matching sequences, -1 padded -- and their
+        scores (float32, -inf padded).  Clips are sent in calls of at most CLIP_CALL_ROWS rows."""
+        rows = _f32c(rows)
+        clip_off = np.ascontiguousarray(clip_off, dtype=np.int64)
+        if rows.ndim != 2 or rows.shape[1] != self.d:
+            raise ValueError(f"clip_match: expected (n, {self.d}) rows")
+        if clip_off.ndim != 1 or len(clip_off) < 1 or clip_off[0] != 0 or clip_off[-1] != len(rows):
+            raise ValueError("clip_match: clip_off must run from 0 to len(rows)")
+        n_clips = len(clip_off) - 1
+        pred = np.full((n_clips, n_top), -1, dtype=np.int64)
+        scores = np.full((n_clips, n_top), -np.inf, dtype=np.float32)
+        c0 = 0
+        while c0 < n_clips:
+            c1 = c0 + 1               # as many whole clips as fit in one call (one clip always goes)
+            while c1 < n_clips and clip_off[c1 + 1] - clip_off[c0] <= CLIP_CALL_ROWS:
+                c1 += 1
+            off = clip_off[c0:c1 + 1] - clip_off[c0]
+            q = rows[clip_off[c0]:clip_off[c1]]
+            p = np.empty((c1 - c0, n_top), dtype=np.int64)
+            s = np.empty((c1 - c0, n_top), dtype=np.float32)
+            check(lib.nafp_clip_match(self.h, ptr(q), len(q), ptr(off), c1 - c0, int(k_probe), int(n_top), ptr(p),
+                                      ptr(s)))
+            pred[c0:c1], scores[c0:c1] = p, s
+            c0 = c1
         return pred, scores
 
 

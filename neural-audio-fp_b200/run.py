@@ -1,5 +1,6 @@
-"""Command line: ``generate`` and ``evaluate`` of the reference's ``run.py`` (``run.py:77-162``).
-``train`` is outside the inference hot path and is not provided."""
+"""Command line: ``generate`` and ``evaluate`` of the reference's ``run.py`` (``run.py:77-162``), and ``identify``
+(recordings against the database ``generate`` wrote).  ``train`` is outside the inference hot path and is not
+provided."""
 from __future__ import annotations
 
 import os
@@ -70,6 +71,34 @@ def evaluate(checkpoint_name, checkpoint_index, config, index_type, test_seq_len
     if nogpu:
         argv.append('--nogpu')
     eval_faiss(argv)
+
+
+@cli.command()
+@click.argument('checkpoint_name', required=True)
+@click.argument('checkpoint_index', required=False)
+@click.option('--config', '-c', default='default', required=False, type=click.STRING)
+@click.option('--query', '-q', required=True, type=click.STRING,
+              help="A 16-bit 8 kHz mono WAV, or a directory of them, to identify.")
+@click.option('--emb_dir', default=None, type=click.STRING,
+              help="Directory of the database memmaps. Default is OUTPUT_ROOT_DIR/CHECKPOINT_NAME/CHECKPOINT_INDEX/.")
+@click.option('--source', '-s', default=None, type=click.STRING,
+              help="The --source the database was generated from (its rows are then custom_source).")
+@click.option('--skip_dummy', default=False, is_flag=True, help="The database was generated with --skip_dummy.")
+@click.option('--index_type', '-i', default='l2', type=click.STRING, help="One of {'l2', 'ivfpq', 'ivf', 'ivfpq-rr'}.")
+@click.option('--k_probe', '-k', default=20, type=click.INT, help="Top k search for each segment (<= 128). Default is 20.")
+@click.option('--top', default=10, type=click.INT, help="Matches reported per clip (<= 100). Default is 10.")
+@click.option('--window', default=None, type=click.FLOAT,
+              help="Identify consecutive windows of this many seconds separately (recordings of several tracks).")
+@click.option('--output', '-o', default=None, type=click.STRING, help="Write the matches to this JSON file.")
+def identify(checkpoint_name, checkpoint_index, config, query, emb_dir, source, skip_dummy, index_type, k_probe, top,
+             window, output):
+    """Identify recordings: for each query file (or --window of it), the database tracks and offsets it matches.
+
+    ex) python -m nafp_b200.run identify CKPT 100 -c default --query rec.wav -i l2"""
+    from .eval.identify import run_identify
+    cfg = load_config(config)
+    run_identify(cfg, checkpoint_name, checkpoint_index, query, emb_dir=emb_dir, source=source, skip_dummy=skip_dummy,
+                 index_type=index_type, k_probe=k_probe, top=top, window=window, output=output)
 
 
 if __name__ == '__main__':
