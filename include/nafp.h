@@ -148,6 +148,34 @@ int nafp_fingerprint_pcm16_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t 
 int nafp_fingerprint_pcm16_tracks_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t n_samples,
                                        const int64_t* seg_off_host, const int32_t* seg_valid_host,
                                        int64_t n_seg, int64_t group_size, float* emb_host);
+/* ------------------------------------------------------------------ resampling to the model rate
+ * The reference's reader (model/utils/audio_utils.py:140-264) refuses any WAV that is not 8 kHz mono; these entry points
+ * bring 16-bit PCM at any rate and channel count to an 8 kHz int16 track on the device.
+ * For a track of N frames of C interleaved channels at fs_in, to fs_out: g = gcd(fs_in, fs_out), up = fs_out / g,
+ * down = fs_in / g, hl = 10 max(up, down) (0 when up == down), h = scipy.signal.firwin(2 hl + 1, 1 / max(up, down),
+ * window=('kaiser', 5.0)) * up (resample_poly's default filter, built by the library in fp64), x[n] = mean of the C
+ * channels of frame n (0 outside [0, N)), and
+ *     y[m] = round_half_even_saturated( sum_n x[n] h[hl + m down - n up] ),   m < ceil(N up / down),
+ * summed in fp64 over ascending n (h = 0 outside [0, 2 hl]).  Equal rates are a copy (C == 1) or round(mean).
+ * Limits: max(up, down) <= NAFP_RESAMPLE_MAX_RATIO (NAFP_ERR_UNSUPPORTED otherwise), 1 <= C <= NAFP_RESAMPLE_MAX_CHANNELS. */
+enum { NAFP_RESAMPLE_MAX_RATIO = 1024, NAFP_RESAMPLE_MAX_CHANNELS = 8 };
+
+/* Outputs m0 .. m0 + n_out - 1 of a track -> out_dev (n_out int16).  in_dev holds the frames frame0 .. frame0 + n_frames - 1
+ * (interleaved int16); frames outside that window are read as zero.  The result is exact when the window covers frames
+ * ceil((m0 down - hl) / up) .. floor(((m0 + n_out - 1) down + hl) / up), clamped to [0, N).  Asynchronous on the ctx
+ * stream; the filter of an (fs_in, fs_out) pair is built once per ctx. */
+int nafp_resample_pcm16_dev(nafp_ctx* ctx, const int16_t* in_dev, int64_t frame0, int64_t n_frames, int32_t channels,
+                            int32_t fs_in, int32_t fs_out, int64_t m0, int64_t n_out, int16_t* out_dev);
+
+/* nafp_fingerprint_pcm16_tracks_host for source files at any rate (the 8 kHz tracks of generate --source / identify,
+ * model/utils/audio_utils.py:140-264): runs_host (n_runs, 7) int64 rows (pcm offset in int16 elements, frame0, n_frames,
+ * channels, fs_in, m0, n_out), each a window of one source track at pcm_host + offset as nafp_resample_pcm16_dev takes it.
+ * Run r is resampled to 8 kHz into positions [sum_{r' < r} n_out, + n_out) of one int16 track buffer on the device, one
+ * launch for all runs; seg_off / seg_valid index that buffer as they index pcm_host in nafp_fingerprint_pcm16_tracks_host.
+ * Every run, pcm range and segment window is checked before any device work. */
+int nafp_fingerprint_pcm16_sources_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t n_pcm, const int64_t* runs_host,
+                                        int64_t n_runs, const int64_t* seg_off_host, const int32_t* seg_valid_host,
+                                        int64_t n_seg, int64_t group_size, float* emb_host);
 /* Debug/parity taps: activation of conv `layer` (0..15) after its normalisation (any MODEL.BN) for the LAST
  * nafp_encoder_forward call, as float32 (n_seg, F, T, C) into out_host. */
 int nafp_encoder_activation_host(nafp_ctx* ctx, int layer, int64_t n_seg, float* out_host);

@@ -65,6 +65,10 @@ _SIGS = {
     "nafp_fingerprint_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "nafp_fingerprint_pcm16_host": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "nafp_fingerprint_pcm16_tracks_host": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
+    "nafp_resample_pcm16_dev": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int32, c_int32, c_int32, c_int64, c_int64,
+                                        c_void_p]),
+    "nafp_fingerprint_pcm16_sources_host": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64,
+                                                    c_int64, c_void_p]),
     "nafp_encoder_activation_host": (c_int, [c_void_p, c_int, c_int64, c_void_p]),
     "nafp_index_create": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, _vpp]),
     "nafp_index_destroy": (c_int, [c_void_p]),

@@ -12,7 +12,8 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["capi.cu", "flat_search.cu", "seq_match.cu", "ivfpq.cu", "ivfpq_lm.cu", "logmel.cu", "encoder.cu", "synth.cu", "mini_search.cu"]
+SOURCES = ["capi.cu", "flat_search.cu", "seq_match.cu", "ivfpq.cu", "ivfpq_lm.cu", "logmel.cu", "encoder.cu", "synth.cu", "mini_search.cu",
+           "resample.cu"]
 OUT = os.path.join(HERE, "libnafp.so")
 HASH = OUT + ".srchash"
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

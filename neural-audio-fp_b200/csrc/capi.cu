@@ -101,6 +101,7 @@ int nafp_ctx_destroy(nafp_ctx* ctx) {
     cudaStreamSynchronize(ctx->stream);
     logmel_destroy(ctx);
     encoder_destroy(ctx);
+    resample_destroy(ctx);
     if (ctx->stage_dev) cudaFree(ctx->stage_dev);
     if (ctx->stage_pinned) cudaFreeHost(ctx->stage_pinned);
     if (ctx->clip_ws) cudaFree(ctx->clip_ws);

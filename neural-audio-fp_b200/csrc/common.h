@@ -55,6 +55,7 @@ struct NvtxRange {
 
 struct LogmelState;
 struct EncoderState;
+struct ResampleState;
 
 }  // namespace nafp
 
@@ -67,6 +68,7 @@ struct nafp_ctx {
     int64_t launches = 0;
     nafp::LogmelState* logmel = nullptr;
     nafp::EncoderState* encoder = nullptr;
+    nafp::ResampleState* resample = nullptr;
     // reusable staging buffers for the *_host entry points
     void* stage_dev = nullptr;
     int64_t stage_dev_bytes = 0;
@@ -106,5 +108,18 @@ int make_tensor_map(CUtensorMap* out, CUtensorMapDataType dtype, int rank, void*
 // module destructors (called from nafp_ctx_destroy)
 void logmel_destroy(nafp_ctx* ctx);
 void encoder_destroy(nafp_ctx* ctx);
+void resample_destroy(nafp_ctx* ctx);
+
+// resampler (resample.cu): one run is a window of one track's source frames and the outputs m0 .. m0 + n_out - 1 it
+// yields, written at out_off of the output buffer
+struct SourceRun {
+    int64_t pcm_off, frame0, n_frames, m0, n_out, out_off;
+    int32_t channels, fs_in;
+};
+int resample_ratio(int32_t fs_in, int32_t fs_out, int32_t* up, int32_t* down, int32_t* hl);
+int resample_check_run(const char* fn, int64_t frame0, int64_t n_frames, int32_t channels, int32_t fs_in,
+                       int32_t fs_out, int64_t m0, int64_t n_out);
+int resample_launch(nafp_ctx* ctx, const int16_t* pcm_dev, const SourceRun* runs, int64_t n_runs, int32_t fs_out,
+                    int16_t* out_dev);
 
 }  // namespace nafp

@@ -1430,6 +1430,61 @@ int nafp_fingerprint_pcm16_tracks_host(nafp_ctx* ctx, const int16_t* pcm_host, i
     return NAFP_OK;
 }
 
+// The same for source files at any rate: the runs are resampled to one 8 kHz track buffer by one launch, which the
+// segments then index as above.
+int nafp_fingerprint_pcm16_sources_host(nafp_ctx* ctx, const int16_t* pcm_host, int64_t n_pcm, const int64_t* runs_host,
+                                        int64_t n_runs, const int64_t* seg_off_host, const int32_t* seg_valid_host,
+                                        int64_t n_seg, int64_t group_size, float* emb_host) {
+    NAFP_RANGE("nafp_fingerprint_pcm16_sources_host");
+    const char* fn = "nafp_fingerprint_pcm16_sources_host";
+    NAFP_REQUIRE(ctx && n_seg >= 0 && n_pcm >= 0 && n_runs >= 0 && group_size >= 1 &&
+                     (n_seg == 0 || (seg_off_host && seg_valid_host && emb_host)) && (n_runs == 0 || runs_host) &&
+                     (n_pcm == 0 || pcm_host),
+                 NAFP_ERR_INVALID, "%s: bad arguments", fn);
+    NAFP_REQUIRE(ctx->encoder && ctx->encoder->weights, NAFP_ERR_STATE, "%s: call nafp_weights_load first", fn);
+    std::vector<SourceRun> runs(static_cast<size_t>(n_runs));
+    int64_t n_samples = 0;
+    for (int64_t r = 0; r < n_runs; ++r) {
+        const int64_t* u = runs_host + r * 7;
+        NAFP_REQUIRE(u[3] >= 1 && u[3] <= 0x7fffffff && u[4] >= 1 && u[4] <= 0x7fffffff, u[3] < 1 || u[4] < 1 ? NAFP_ERR_INVALID : NAFP_ERR_UNSUPPORTED,
+                     "%s: run %lld has %lld channels at %lld Hz", fn, (long long)r, (long long)u[3], (long long)u[4]);
+        NAFP_TRY(resample_check_run(fn, u[1], u[2], static_cast<int32_t>(u[3]), static_cast<int32_t>(u[4]), 8000, u[5], u[6]));
+        NAFP_REQUIRE(u[0] >= 0 && u[0] <= n_pcm && u[2] * u[3] <= n_pcm - u[0], NAFP_ERR_INVALID,
+                     "%s: run %lld reads [%lld, +%lld) of %lld samples", fn, (long long)r, (long long)u[0],
+                     (long long)(u[2] * u[3]), (long long)n_pcm);
+        runs[r] = SourceRun{u[0], u[1], u[2], u[5], u[6], n_samples, static_cast<int32_t>(u[3]), static_cast<int32_t>(u[4])};
+        n_samples += u[6];
+    }
+    for (int64_t i = 0; i < n_seg; ++i)
+        NAFP_REQUIRE(seg_off_host[i] >= 0 && seg_valid_host[i] >= 0 && seg_valid_host[i] <= 8000 &&
+                         seg_off_host[i] + seg_valid_host[i] <= n_samples,
+                     NAFP_ERR_INVALID, "%s: segment %lld reads [%lld, +%d) of %lld resampled samples", fn, (long long)i,
+                     (long long)seg_off_host[i], (int)seg_valid_host[i], (long long)n_samples);
+    if (n_seg == 0) return NAFP_OK;
+    NAFP_CUDA(cudaSetDevice(ctx->device));
+    NAFP_CUDA(cudaStreamSynchronize(ctx->stream));      // the staging buffer may be re-allocated below
+    // one staging buffer, every part 256-byte aligned: source samples, 8 kHz samples (+1 so that neither is empty),
+    // offsets, valid lengths, fingerprints
+    const int64_t src_pad = ((n_pcm + 1) * 2 + 255) / 256 * 256, pcm_pad = ((n_samples + 1) * 2 + 255) / 256 * 256;
+    const int64_t off_bytes = (n_seg * 8 + 255) / 256 * 256, val_bytes = (n_seg * 4 + 255) / 256 * 256;
+    const int64_t emb_bytes = n_seg * EMB * static_cast<int64_t>(sizeof(float));
+    NAFP_TRY(ensure_dev(ctx, &ctx->stage_dev, &ctx->stage_dev_bytes, src_pad + pcm_pad + off_bytes + val_bytes + emb_bytes));
+    uint8_t* base = static_cast<uint8_t*>(ctx->stage_dev);
+    int16_t* src_dev = reinterpret_cast<int16_t*>(base);
+    int16_t* pcm_dev = reinterpret_cast<int16_t*>(base + src_pad);
+    int64_t* off_dev = reinterpret_cast<int64_t*>(base + src_pad + pcm_pad);
+    int32_t* val_dev = reinterpret_cast<int32_t*>(base + src_pad + pcm_pad + off_bytes);
+    float* emb_dev = reinterpret_cast<float*>(base + src_pad + pcm_pad + off_bytes + val_bytes);
+    NAFP_CUDA(cudaMemcpyAsync(src_dev, pcm_host, static_cast<size_t>(n_pcm) * 2, cudaMemcpyHostToDevice, ctx->stream));
+    NAFP_CUDA(cudaMemcpyAsync(off_dev, seg_off_host, static_cast<size_t>(n_seg) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    NAFP_CUDA(cudaMemcpyAsync(val_dev, seg_valid_host, static_cast<size_t>(n_seg) * 4, cudaMemcpyHostToDevice, ctx->stream));
+    NAFP_TRY(resample_launch(ctx, src_dev, runs.data(), n_runs, 8000, pcm_dev));
+    NAFP_TRY(fingerprint_dev(ctx, pcm_dev, true, n_seg, group_size, emb_dev, off_dev, val_dev));
+    NAFP_CUDA(cudaMemcpyAsync(emb_host, emb_dev, static_cast<size_t>(emb_bytes), cudaMemcpyDeviceToHost, ctx->stream));
+    NAFP_CUDA(cudaStreamSynchronize(ctx->stream));
+    return NAFP_OK;
+}
+
 int nafp_encoder_activation_host(nafp_ctx* ctx, int layer, int64_t n_seg, float* out_host) {
     NAFP_RANGE("nafp_encoder_activation_host");
     NAFP_REQUIRE(ctx && ctx->encoder && out_host && layer >= 0 && layer < ENC_LAYERS, NAFP_ERR_INVALID,

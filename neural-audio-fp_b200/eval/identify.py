@@ -123,8 +123,7 @@ def fingerprint_sequence(m_fp, seq, batches_per_call=64):
     out = np.empty((seq.n_samples, 128), np.float32)
     for i in range(0, len(seq), batches_per_call):
         j = min(i + batches_per_call, len(seq))
-        pcm, seg_off, seg_valid = seq.get_track_block(i, j)
-        emb = m_fp.fingerprint_tracks(pcm, seg_off, seg_valid, group_size=seq.bsz)
+        emb = m_fp.fingerprint_block(seq.get_source_block(i, j), group_size=seq.bsz)
         out[i * seq.bsz:i * seq.bsz + len(emb)] = emb
     return out
 
@@ -147,6 +146,8 @@ def run_identify(cfg, checkpoint_name, checkpoint_index, query, emb_dir=None, so
     hop = float(cfg['MODEL']['HOP'])
     check_limits(k_probe, top, window, hop, index_type)
     seq = query_sequence(cfg, query)               # WAV headers only
+    if seq.conversions():
+        print(seq.conversions())
     window_seg = None if window is None else window_segments(window, hop)
     clip_off, clip_file, clip_first = split_clips(seq.file_first, window_seg)
     longest = int(np.diff(clip_off).max())

@@ -164,6 +164,30 @@ class FingerPrinter:
                                                      int(group_size), ptr(emb)))
         return emb
 
+    def fingerprint_sources(self, pcm, seg_off, seg_valid, runs, group_size):
+        """``fingerprint_tracks`` for source files at any rate and channel count (``SegmentSequence.get_source_block``):
+        one launch resamples the runs to 8 kHz int16 on the GPU, which the segments then index."""
+        pcm = np.ascontiguousarray(pcm, dtype=np.int16)
+        runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 7)
+        seg_off = np.ascontiguousarray(seg_off, dtype=np.int64)
+        seg_valid = np.ascontiguousarray(seg_valid, dtype=np.int32)
+        n = len(seg_off)
+        if len(seg_valid) != n:
+            raise ValueError("seg_off and seg_valid differ in length")
+        emb = np.empty((n, 128), dtype=np.float32)
+        check(lib.nafp_logmel_set_segment_norm(self.ctx.h, int(self.segment_norm)))
+        check(lib.nafp_fingerprint_pcm16_sources_host(self.ctx.h, ptr(pcm), len(pcm), ptr(runs), len(runs), ptr(seg_off),
+                                                      ptr(seg_valid), n, int(group_size), ptr(emb)))
+        return emb
+
+    def fingerprint_block(self, block, group_size):
+        """Fingerprints of a ``SegmentSequence.get_source_block`` block: blocks of 8 kHz mono files take the
+        ``fingerprint_tracks`` path, any other through ``fingerprint_sources``."""
+        pcm, seg_off, seg_valid, runs = block
+        if runs is None:
+            return self.fingerprint_tracks(pcm, seg_off, seg_valid, group_size)
+        return self.fingerprint_sources(pcm, seg_off, seg_valid, runs, group_size)
+
     def activation(self, layer, n_seg):
         """Activation (n_seg, F, T, C) of conv ``layer`` after its normalisation, from the last encoder pass."""
         s = arch.conv_specs()[layer]

@@ -162,18 +162,21 @@ def generate_fingerprint(cfg, checkpoint_name, checkpoint_index, source_root_dir
             arr = np.memmap(path, dtype='float32', mode='r+', shape=arr_shape)
 
         print(f"=== Generating fingerprint from \x1b[1;32m'{key}'\x1b[0m bsz={bsz}, {n_items} items, d={dim} ===")
+        if rank == 0 and ds[key].conversions():
+            print(ds[key].conversions())
         b_lo, b_hi = _shard(len(ds[key]), rank, world_size)
         # several whole batches per call (the library keeps TS_BATCH_SZ groups separate); the next block is cut
         # from the WAV files by a worker thread while the GPU works on this one (ctypes releases the GIL)
         from concurrent.futures import ThreadPoolExecutor
         blocks = [(i, min(i + batches_per_call, b_hi)) for i in range(b_lo, b_hi, batches_per_call)]
         with ThreadPoolExecutor(max_workers=1) as pool:
-            nxt = pool.submit(ds[key].get_track_block, *blocks[0]) if blocks else None
+            nxt = pool.submit(ds[key].get_source_block, *blocks[0]) if blocks else None
             for n_blk, (i, j) in enumerate(blocks):
-                pcm, seg_off, seg_valid = nxt.result()
-                nxt = pool.submit(ds[key].get_track_block, *blocks[n_blk + 1]) if n_blk + 1 < len(blocks) else None
-                # whole-track sample runs + one window per segment: the GPU cuts the overlapping segments
-                emb = m_fp.fingerprint_tracks(pcm, seg_off, seg_valid, group_size=bsz)
+                block = nxt.result()
+                nxt = pool.submit(ds[key].get_source_block, *blocks[n_blk + 1]) if n_blk + 1 < len(blocks) else None
+                # whole-track sample runs + one window per segment: the GPU resamples the runs that are not 8 kHz mono
+                # and cuts the overlapping segments
+                emb = m_fp.fingerprint_block(block, group_size=bsz)
                 arr[i * bsz:i * bsz + len(emb), :] = emb
                 if rank == 0:
                     print(f'\r{j - b_lo}/{b_hi - b_lo}', end='', flush=True)

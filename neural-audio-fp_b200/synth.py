@@ -42,8 +42,10 @@ def add_noise_snr(x_int16, snr_db, seed):
 
 
 def write_wav(path, x_int16, fs=8000):
+    """16-bit PCM WAV of x: (n,) mono or (n, channels) frames."""
+    x_int16 = np.asarray(x_int16)
     with wave.open(path, "w") as w:
-        w.setnchannels(1)
+        w.setnchannels(1 if x_int16.ndim == 1 else x_int16.shape[1])
         w.setsampwidth(2)
         w.setframerate(fs)
         w.writeframes(np.asarray(x_int16, dtype="<i2").tobytes())
